@@ -4,6 +4,13 @@
     python bench.py [--gpus N] [--steps K] [--warmup W]            # our CUDA path
     python bench.py --impl reference [...]                          # the reference's CPU arithmetic (oracle port)
     torchrun --nproc-per-node N ... bench.py --gpus N ...           # one rank per GPU, utterance-sharded
+    python bench.py --dump-outputs DIR [...]                        # + the outputs of every entry's last timed step as .npy
+
+Outputs written by ``--dump-outputs`` (float32; ``_rank<r>`` appended to each name under N > 1 ranks): ``headline_codes``
+and ``<key>_codes`` of the decode entries, the ids the last timed step left in the batch, [utterances, rows, frames];
+``mimi_bs*_pcm``, every frame of the last timed end-to-end step, [streams, frames, samples]; ``tts_stream_bs1_pcm``, the
+chunks of the last timed stream, concatenated.  The inputs are seeded, so two builds run with the same arguments can be
+compared file by file.
 
 A *step* is one pass of the hot path over one batch of synthetic input: ``frames`` Mimi frames decoded for
 ``batch`` utterances per GPU, starting from a prefilled synthetic prompt.  The headline (top-level keys) is
@@ -42,6 +49,7 @@ if ROOT not in sys.path:
 
 FALLBACK_HBM_GBS = 6650.0  # /opt/skills/guides/B200_PROFILING.md fallback when MEASURED_PEAKS.json is absent
 CPU_SAMPLE_FRAMES = 128    # frames of one CPU-arm step (a bounded sample of the workload, centred on its mean context)
+DUMP_BYTES = 64 << 20      # --dump-outputs: all files together
 
 
 @dataclass
@@ -112,7 +120,30 @@ def parse_args():
     ap.add_argument("--no-stream-overlap", action="store_true", help="tts_stream_bs1: codec step after the decode step instead of beside the next one")
     ap.add_argument("--cpu-frames", type=int, default=0, help="frames of the CPU sample (0 = %d)" % CPU_SAMPLE_FRAMES)
     ap.add_argument("--opt", action="append", default=[], help="engine option name=value (smol_set_option), repeatable")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what each entry's last timed step computed as DIR/<name>.npy (float32, "
+                         "%d MB at most in all), to compare two builds output for output" % (DUMP_BYTES >> 20))
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
+    return args
+
+
+def dump_outputs(out_dir: str, arrays: dict, budget: int) -> None:
+    """Writes each array as out_dir/<name>.npy in float32 (the codes are small integers: exact).  When the arrays exceed
+    `budget` bytes together, each keeps the same share of its elements: a fixed sample (flat indices drawn with seed 0, in
+    increasing order) stored 1-D, so that two runs with the same arguments write the same elements."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(a.size * 4 for a in arrays.values())
+    keep = min(1.0, (budget - 1024 * len(arrays)) / total) if total else 1.0   # 1 KB per file for the .npy header
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float32)
+        if keep < 1.0:
+            idx = np.random.default_rng(0).choice(a.size, int(a.size * keep), replace=False)
+            a = a.reshape(-1)[np.sort(idx)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def load_peaks():
@@ -405,6 +436,8 @@ def measure(work: Work, args, steps: int, warmup: int, ctx) -> dict:
     total_ms = start.elapsed_time(stop)
     kernel_ms = statistics.mean(a.elapsed_time(b) for a, b in ev)
     codes_check = int(batch.out_codes.sum().item())  # the result is really produced
+    # what the last timed step handed back: [batch, rows, frames] ids, as generate_batch(audio_only=False) returns per utterance
+    outputs = {"codes": batch.out_codes.permute(0, 2, 1).cpu().numpy()} if args.dump_outputs else {}
     frame_lat = None
     if frame_clock is not None:  # stamps of the last timed step: p50 / p99 of the per-frame latency (BASELINE.json's second metric)
         ns = frame_clock.cpu().numpy().astype("float64")
@@ -462,7 +495,7 @@ def measure(work: Work, args, steps: int, warmup: int, ctx) -> dict:
         "launch_mode": ("data-flow persistent kernel (LL flag words, TMA producer warp, one team of CTAs per sequence), one launch per step" if dataflow
                         else "persistent cooperative kernel with grid barriers, one launch per step" if args.mode != 1
                         else "per-phase launches in a CUDA graph"),
-        "config": public_config(work, world),
+        "config": public_config(work, world), "outputs": outputs,
     }
     del model
     torch.cuda.empty_cache()
@@ -525,6 +558,8 @@ def measure_mimi(key: str, batch: int, frames: int, args, steps: int, warmup: in
         run(False)
     torch.cuda.synchronize()
     e2e_ms = (time.perf_counter() - t0) * 1e3
+    # the resident arm keeps only the last frame's PCM; the e2e arm's last step leaves every frame of the same codes in pcm_h
+    outputs = {"pcm": pcm_h.permute(1, 0, 2).numpy().copy()} if args.dump_outputs else {}     # [streams, frames, samples]
     t = torch.tensor([total_ms, e2e_ms], dtype=torch.float64, device=dev)
     if dist is not None:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -551,7 +586,7 @@ def measure_mimi(key: str, batch: int, frames: int, args, steps: int, warmup: in
         "e2e": {"value": steps * frames * batch * world / (e2e_ms * 1e-3), "unit": "frames/s", "h2d_bytes_per_step": frames * batch * 8 * 4,
                 "d2h_bytes_per_step": frames * batch * m.samples_per_frame * 4, "steps": steps},
         "clocks": clocks, "gpu_launches": steps * frames * m.launches_per_step, "launch_mode": "57 launches per decode_step, CUDA-graph replay",
-        "realtime_factor": steps * frames * batch * world / (total_ms * 1e-3) / 12.5, "check": check,
+        "realtime_factor": steps * frames * batch * world / (total_ms * 1e-3) / 12.5, "check": check, "outputs": outputs,
     }
     if rank == 0 and world == 1 and batch == 1 and not args.no_cpu_baseline:
         from oracle.mimi_oracle import MimiOracle, StreamState   # CPU leg only (the checker, never the product)
@@ -575,6 +610,7 @@ def measure_tts_stream(args, steps: int, warmup: int, ctx, frames: int = 128) ->
     """The reference's streaming loop end to end (smoltts_mlx/__init__.py:85-95) at one utterance: prompt -> one frame per
     SingleBatchGenerator.__next__ (one launch of the data-flow kernel, ids read back by the host) -> MimiModel.decode_step ->
     the 80 ms PCM chunk on the host.  There is no device-resident form of this loop: value == e2e."""
+    import numpy as np
     import torch
 
     from smoltts_b200 import GenerationSettings, MimiModel, PromptEncoder, RQTransformer, SmolTTS, byte_level_tokenizer, named_config
@@ -588,13 +624,15 @@ def measure_tts_stream(args, steps: int, warmup: int, ctx, frames: int = 128) ->
     enc = PromptEncoder.from_model(byte_level_tokenizer(cfg.codebook_size), lm)
     tts = SmolTTS(lm, enc, codec, settings=GenerationSettings(default_temp=0.0, default_fast_temp=0.0, max_new_tokens=frames - 1))
     text = "The quick brown fox jumps over the lazy dog. " * 4          # 180 bytes
+    chunks = []
 
     def run():
         # random-init weights emit non-audio ids now and then (they skip the codec, as in the reference) and may hit
         # <|im_end|> early: SmolTTS.stream reports what it generated
         st = {}
+        chunks.clear()
         for chunk in tts.stream(text, "nova", overlap=not args.no_stream_overlap, lm_ctas=args.stream_lm_ctas, stats=st):
-            pass
+            chunks.append(chunk)
         return st["frames"], st["audio_frames"]
 
     def barrier():
@@ -632,6 +670,7 @@ def measure_tts_stream(args, steps: int, warmup: int, ctx, frames: int = 128) ->
                        + ("" if args.no_stream_overlap else "; pipelined: the decode step of frame t + 1 is launched before the host reads frame t, whose ids, "
                                                               "codec step and PCM go through a side stream (decode kernel on %d of the SMs)" % args.stream_lm_ctas),
         "realtime_factor": value / 12.5,
+        "outputs": {"pcm": np.concatenate(chunks)} if args.dump_outputs and chunks else {},   # the chunks of the last timed run
     }
     del tts, lm, codec
     torch.cuda.empty_cache()
@@ -688,6 +727,11 @@ def run_ours(args):
                 entries.append(measure_mimi(key, b, f, args, max(1, min(args.steps, args.config_steps)), 3, ctx))
         if (wanted is None or "tts_stream_bs1" in wanted) and args.model == "smoltts_byte_150m":
             entries.append(measure_tts_stream(args, max(1, min(args.steps, 3)), 2, ctx))
+    if args.dump_outputs:
+        suffix = f"_rank{rank}" if world > 1 else ""
+        dump_outputs(args.dump_outputs, {f"{key}_{name}{suffix}": a for key, outs in [("headline", main["outputs"])]
+                                         + [(e["key"], e["outputs"]) for e in entries] for name, a in outs.items()},
+                     DUMP_BYTES // world)
 
     if rank == 0:
         cfg_pub = dict(main["config"])  # identical in both arms (ours / --impl reference): the configuration measured
