@@ -32,6 +32,7 @@ namespace ll2 { using SmemPlan = LL2SmemPlan; }
 bool ll2_plan(const DevModel& M, int holdoff, int flags, ll2::SmemPlan* sp, size_t* smem);
 cudaError_t ll2_configure(size_t smem);
 cudaError_t ll2_max_ctas(size_t smem, int* per_sm);
+int ll2_mlp_cluster(const DevModel& M, size_t smem, int n_slots, int* n_clusters);
 cudaError_t ll2_launch(const DevModel& M, const CallArgs& A, const ll2::SmemPlan& sp, size_t smem, int n_ctas, cudaStream_t stream);
 cudaError_t ll2_pack_launch(uint16_t* dst, const uint16_t* a, const uint16_t* b, int rows, int K, cudaStream_t stream);
 }  // namespace smol
@@ -65,6 +66,10 @@ struct SmolModel {
     int ll2_holdoff = 400;     // option "ll_holdoff": cycles between the end of a phase and the first poll of the next
     int ll2_max_batch = 8;     // option: sequences (teams of CTAs) the kernel carries per launch; larger batches go to the
                                // barrier kernel / its tcgen05 variant (measured at bs=8: 1.5 ms per frame step against 2.3 ms)
+    int ll2_fused_mlp = 1;     // option "ll_fused_mlp": batch 1 runs the gated MLP fused in thread-block clusters when they fit
+    int ll2_cluster = 0;       // CTAs per cluster of the fused MLP (0: no cluster size fits this model / GPU)
+    int ll2_clusters = 0;      // clusters of the fused grid
+    int ll2_last_fused = 0;    // the last data-flow launch ran the fused MLP
     smol::ll2::SmemPlan ll2_sp;
     size_t ll2_smem = 0;
     bool packed_ready = false; // tensor-core GEMV layout of the bound weights (rebuilt after a weight / workspace bind)
@@ -105,7 +110,7 @@ static int imax(int a, int b) { return a > b ? a : b; }
 
 struct WsLayout {
     size_t x, h, xf, q, attn, act, xn, silu_lut, tmaps, kpart, fkv, token_logits, depth_logits, frame_tokens, partial, split_count, barrier;
-    size_t ll, ll_epoch, ll2_score, ll2_tok, ll2_cand, packed, total;
+    size_t ll, ll_epoch, ll2_score, ll2_tok, ll2_cand, ll2_psum, packed, total;
 };
 
 static int ll_batch_of(const SmolConfig& c) { (void)c; return smol::kLL2MaxTeams; }  // word regions for up to 8 teams
@@ -178,6 +183,8 @@ static WsLayout ws_layout(const SmolConfig& c, int depth) {
     L.ll2_score = take((size_t)bl * 2 * c.n_head * ll2_score_len(c) * 8);
     L.ll2_tok = take((size_t)bl * (1 + depth) * smol::kLLMaxCtas * 8);
     L.ll2_cand = take((size_t)bl * (1 + depth) * smol::kLLRep * smol::kLLMaxCtas * 8);
+    // one sequence only: the fused MLP runs at batch 1
+    L.ll2_psum = take((size_t)(c.n_layer + depth * c.n_fast_layer) * smol::kLLRep * smol::kLL2Warps * c.dim * 8);
     L.packed = take(packed_bytes(c, depth));
     L.total = off;
     return L;
@@ -318,6 +325,7 @@ int smol_bind_workspace(SmolModel* m, void* d_workspace, size_t bytes) {
     d.ll = (unsigned long long*)(base + L.ll); d.ll_epoch = (uint32_t*)(base + L.ll_epoch);
     d.ll2_score = (unsigned long long*)(base + L.ll2_score); d.ll2_tok = (unsigned long long*)(base + L.ll2_tok);
     d.ll2_cand = (unsigned long long*)(base + L.ll2_cand); d.ll2_score_len = ll2_score_len(m->cfg);
+    d.ll2_psum = (unsigned long long*)(base + L.ll2_psum);
     m->packed_ready = false;
     // split counters, barrier words and every LL word (epoch 0 = never written) must start at zero
     // (setup-time, synchronous)
@@ -469,7 +477,21 @@ static int ensure_ll2(SmolModel* m) {
     int per_sm = 0;
     CU(smol::ll2_max_ctas(m->ll2_smem, &per_sm));
     m->ll2_state = per_sm >= 1 ? 1 : -1;
+    if (m->ll2_state == 1) m->ll2_cluster = smol::ll2_mlp_cluster(m->dm, m->ll2_smem, m->ll2_sp.n_slots, &m->ll2_clusters);
     return SMOL_OK;
+}
+
+// Grid of the fused gated MLP for a solo decode (ll2_kernel.cu: build_desc): clusters of ll2_cluster CTAs, one per K-slice
+// (+ one idle in the MLP when it fits).  An "n_ctas" override keeps it only when it is such a grid.  The fused and the
+// unfused program compute the same bits, so every other case simply runs unfused.  Returns the cluster size, 0 = unfused.
+static int ll2_fused_cluster(const SmolModel* m, int* n_ctas) {
+    const int S = m->ll2_cluster;
+    if (!m->ll2_fused_mlp || S <= 0) return 0;
+    if (m->n_ctas_override <= 0) { *n_ctas = m->ll2_clusters * S; return S; }
+    const int n = m->n_ctas;
+    if (n % S || n / S < smol::kLL2Warps || n / S > m->ll2_clusters) return 0;
+    *n_ctas = n;
+    return S;
 }
 
 // Grid of a SOLO decode on the data-flow kernel.  An exchange has as many participants as the grid has CTAs, a phase takes as
@@ -531,6 +553,8 @@ static int enqueue(SmolModel* m, CallArgs A, cudaStream_t stream, bool whole_ite
         if (m->ll2_state == 1) {
             if (A.n_iter == 0) return SMOL_OK;
             A.team_ctas = A.batch == 1 ? ll2_solo_ctas(m) : m->n_ctas / A.batch;
+            A.mlp_cluster = A.batch == 1 ? ll2_fused_cluster(m, &A.team_ctas) : 0;
+            m->ll2_last_fused = A.mlp_cluster > 0 ? 1 : 0;
             m->ll2_sp.holdoff = m->ll2_holdoff;
             m->ll2_sp.flags = m->ll_flags;
             CU(smol::ll2_launch(m->dm, A, m->ll2_sp, m->ll2_smem, A.team_ctas * A.batch, stream));
@@ -812,6 +836,10 @@ int smol_set_option(SmolModel* m, const char* name, int64_t value) {
         m->ll2_holdoff = value > 0 ? (int)value : 0;
         return SMOL_OK;
     }
+    if (!std::strcmp(name, "ll_fused_mlp")) {
+        m->ll2_fused_mlp = value != 0 ? 1 : 0;
+        return SMOL_OK;
+    }
     if (!std::strcmp(name, "ll_max_batch")) {
         if (value < 0 || value > smol::kLL2MaxTeams) return fail(SMOL_ERR_INVALID, "ll_max_batch must be in [0, 8]");
         m->ll2_max_batch = (int)value;
@@ -842,6 +870,10 @@ int64_t smol_get_option(const SmolModel* m, const char* name) {
     if (!std::strcmp(name, "ll_holdoff")) return (int64_t)m->ll2_holdoff;
     if (!std::strcmp(name, "ll_slots")) return (int64_t)m->ll2_sp.n_slots;
     if (!std::strcmp(name, "ll_solo_ctas")) return (int64_t)ll2_solo_ctas(m);
+    if (!std::strcmp(name, "ll_fused_mlp")) return (int64_t)m->ll2_fused_mlp;
+    if (!std::strcmp(name, "ll_mlp_cluster")) return (int64_t)m->ll2_cluster;
+    if (!std::strcmp(name, "ll_mlp_clusters")) return (int64_t)m->ll2_clusters;
+    if (!std::strcmp(name, "ll_last_fused")) return (int64_t)m->ll2_last_fused;
     return -1;
 }
 

@@ -40,7 +40,7 @@ constexpr int kLL2PvDims = 8;            // head dims per PV unit
 constexpr int kLL2Depth = 8;             // depth positions whose K/V the kernel keeps in shared memory
 
 struct LL2SmemPlan {   // second-generation data-flow kernel: byte offsets into dynamic shared memory + launch-time knobs
-    int xbuf, res_x, res_h, part, desc, fq, fkv, scratch, ring;
+    int xbuf, res_x, res_h, part, desc, fq, fkv, scratch, act, ring;   // act: the fused MLP's K-slice of act (DSMEM)
     int n_slots;
     int holdoff;       // cycles between the end of a phase and the first poll of the next
     int flags;         // experiment switches
@@ -131,6 +131,8 @@ struct DevModel {
     unsigned long long* ll2_tok;     // sampled ids [teams][n_rows][kLLMaxCtas] words
     unsigned long long* ll2_cand;    // greedy candidates [teams][n_rows][kLLRep][kLLMaxCtas] words
     int ll2_score_len;
+    unsigned long long* ll2_psum;    // fused MLP (batch 1): fp32 partial sums of the W2 phases {fp32 bits, epoch}
+                                     // [W2 phase][kLLRep][7 K-slices][dim] words (ll2_kernel.cu: psum_region)
 };
 
 // Words (8 bytes, two bf16 + epoch) one sequence publishes in a phase; multiples of 16 words (128 B).
@@ -141,7 +143,7 @@ __host__ __device__ inline int ll_phase_words(int kind, int fast, int dim, int n
         case 1: n = dim / 2; break;                      // PH_ATTN (attention output)
         case 2: n = dim / 2; break;                      // PH_WO
         case 3: n = inter / 2; break;                    // PH_W13
-        case 4: n = dim / 2; break;                      // PH_W2
+        case 4: n = dim / 2; break;                      // PH_W2 (the fused MLP's partial sums: ll2_psum)
         case 5: n = n_out / 2; break;                    // PH_HEAD
         default: n = 0; break;
     }
@@ -170,6 +172,7 @@ struct CallArgs {
                       // 3 = only its post-step (0 = the whole phase: cooperative launches)
     int tc_split;     // tensor-core variant: cached positions per attention split (0 = default)
     int team_ctas;    // second-generation data-flow kernel: CTAs per sequence (one team each); grid = batch * team_ctas
+    int mlp_cluster;  // data-flow kernel, batch 1: CTAs per thread-block cluster of the fused gated MLP (0 = unfused)
     const int32_t* prompt;      // prefill: [B][n_rows][s_max]
     const int32_t* prompt_len;  // prefill: [B]
     int s_max;

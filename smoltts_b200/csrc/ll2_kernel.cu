@@ -33,6 +33,8 @@
 // slow step P:223-260 / M:173-192; depth loop P:409-448, M:194-220, G:110-141; sampling G:88-99,118-132; frame
 // assembly + stop rule G:143-171.
 
+#include <algorithm>
+
 #include "common.cuh"
 #include "dev_model.h"
 
@@ -149,6 +151,9 @@ __device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
 __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
     asm volatile("mbarrier.arrive.relaxed.cta.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
+__device__ __forceinline__ void mbar_arrive_n(uint32_t bar, uint32_t n) {
+    asm volatile("mbarrier.arrive.relaxed.cta.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(n) : "memory");
+}
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
     uint32_t ok, spins = 0;
     for (;;) {
@@ -167,9 +172,25 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t
                  ::"r"(dst), "l"(src), "r"(bytes), "r"(bar), "l"(policy) : "memory");
 }
 
+// ---- thread-block cluster (the fused gated MLP) ---------------------------------------------------------------
+__device__ __forceinline__ uint32_t mapa(uint32_t a, uint32_t rank) {   // the same shared-memory offset in CTA `rank`
+    uint32_t r;
+    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(a), "r"(rank));
+    return r;
+}
+// 16 bytes into a cluster peer's shared memory; the peer's mbarrier `bar` counts them on arrival
+__device__ __forceinline__ void st_async_v4(uint32_t a, uint32_t x, uint32_t y, uint32_t z, uint32_t w, uint32_t bar) {
+    asm volatile("st.async.shared::cluster.mbarrier::complete_tx::bytes.v4.b32 [%0], {%1,%2,%3,%4}, [%5];"
+                 ::"r"(a), "r"(x), "r"(y), "r"(z), "r"(w), "r"(bar) : "memory");
+}
+__device__ __forceinline__ void cluster_sync_all() {
+    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+
 // ---- per-CTA shared state ------------------------------------------------------------------------
 __shared__ __align__(8) uint64_t s_full[kMaxSlots];
 __shared__ __align__(8) uint64_t s_empty[kMaxSlots];
+__shared__ __align__(8) uint64_t s_actbar;   // fused MLP: the slice's act values have arrived from the cluster
 __shared__ SampleScratch s_sc;
 __shared__ float s_ssq[kNW];            // per-warp partial sums of squares (RMSNorm)
 __shared__ uint32_t s_best;             // HEAD phases: the CTA's best (logit, index) candidate
@@ -197,8 +218,17 @@ struct Team {
 //        11    K | n_items << 16
 //        12    kind | fast << 4 | layer << 8 | depth_pos << 16
 //        13    first item of this CTA
-//        14    (unused)
+//        14    fused MLP (W13 and W2 phases): lo | hi << 8 | n_units << 16 -- the K-slice [lo, hi) (k-blocks of w2) of this
+//              CTA's cluster and the W2 row tiles this CTA carries (i0, i0 + S, ..); 0 = not fused / no work
 //        15    len_out (words per replica of the output region) | n_src_words << 16
+//
+// Fused gated MLP (batch 1, A.mlp_cluster = S > 0; grid = clusters of S CTAs).  The 7 consumer warps split a w2 tile's
+// K = inter into the ranges [kb w / 7, kb (w + 1) / 7), and a w2 row is the sum, in warp order, of one acc / acd MMA chain
+// per range.  Cluster c < 7 owns range c: its CTAs compute the act values of the range (the w13 tiles of it, unchanged),
+// hand them to each other through DSMEM, and then run warp c's chain of every w2 row tile, one warp per tile, publishing
+// the fp32 partial sums with the W2 phase's epoch.  The consumers of the W2 region add the 7 partials in range order and
+// the residual (the bf16 roundings of the unfused epilogue): bit for bit the unfused result, with one L2 exchange per
+// MLP instead of two.  The W2 phase itself has no tiles and no input.
 __device__ __forceinline__ int phase_rows(const DevModel& M, const Phase& ph) {
     const bool fast = ph.fast != 0;
     switch (ph.kind) {
@@ -236,7 +266,14 @@ __device__ __forceinline__ unsigned long long* ll_region(const DevModel& M, int 
     return M.ll + M.ll_off[p] + (size_t)(team * kLLRep + rep) * M.ll_len[p];
 }
 
-__device__ __forceinline__ void build_desc(const DevModel& M, const Team& tm, int p, uint32_t dsc) {
+// Fused MLP: the W2 phase p's partial-sum words, replica rep (batch 1 only: one sequence)
+__device__ __forceinline__ unsigned long long* psum_region(const DevModel& M, int p, int rep) {
+    const Phase ph = unpack_phase(M.prog[p]);
+    const int w2 = ph.fast ? M.n_layer + ph.depth_pos * M.n_flayer + ph.layer : ph.layer;
+    return M.ll2_psum + ((size_t)w2 * kLLRep + rep) * kNW * M.dim;
+}
+
+__device__ __forceinline__ void build_desc(const DevModel& M, const Team& tm, int S, int p, uint32_t dsc) {
     const int rep = tm.cta % kLLRep;
     const Phase ph = unpack_phase(M.prog[p]);
     const bool fast = ph.fast != 0;
@@ -245,13 +282,27 @@ __device__ __forceinline__ void build_desc(const DevModel& M, const Team& tm, in
     uint32_t w[kDescWords];
 #pragma unroll
     for (int i = 0; i < kDescWords; ++i) w[i] = 0u;
-    int src_kind = 3, nrep = kLLRep, n_items = 0, i0 = 0, K = 0, gather = 0, n_src = 0, e_back = 1;
+    int src_kind = 3, nrep = kLLRep, n_items = 0, i0 = 0, K = 0, gather = 0, n_src = 0, e_back = 1, psum = 0;
     if (kind != PH_ATTN && kind != PH_SAMPLE) {
         K = phase_k(M, ph);
         // work item = one MMA tile of 16 row slots: 16 rows of the matrix, or 8 rows of w1 over the same 8 rows of w3
         const int items = phase_rows(M, ph) / (kind == PH_W13 ? 8 : 16);
         i0 = (items * tm.cta) / tm.n;
         n_items = (items * (tm.cta + 1)) / tm.n - i0;
+        if (S > 0 && (kind == PH_W13 || kind == PH_W2)) {
+            const int slice = tm.cta / S, r = tm.cta - slice * S;
+            const int kb2 = (fast ? M.finter : M.inter) / 32, rt = (fast ? M.fdim : M.dim) / 16;
+            const int lo = slice < kNW ? (kb2 * slice) / kNW : 0, hi = slice < kNW ? (kb2 * (slice + 1)) / kNW : 0;
+            const int nu = slice < kNW ? (rt - r + S - 1) / S : 0;
+            if (kind == PH_W13) {   // the w13 tiles of the slice's act values (8 per tile)
+                i0 = 4 * lo + (4 * (hi - lo) * r) / S;
+                n_items = 4 * lo + (4 * (hi - lo) * (r + 1)) / S - i0;
+            } else {
+                i0 = r;
+                n_items = 0;
+            }
+            w[14] = nu > 0 ? (uint32_t)lo | ((uint32_t)hi << 8) | ((uint32_t)nu << 16) : 0u;
+        }
         int p_src = p - 1;
         unsigned long long src = 0ull;
         if (kind == PH_QKV && ph.layer == 0) {
@@ -266,11 +317,16 @@ __device__ __forceinline__ void build_desc(const DevModel& M, const Team& tm, in
         if (src_kind == 3) {
             src = (unsigned long long)ll_region(M, tm.team, p_src, rep);
             n_src = (kind == PH_WO && fast) ? (M.fn_head + 2 * M.fn_kv) * kHeadDim / 2 : K / 2;
+            if (S > 0 && unpack_phase(M.prog[p_src]).kind == PH_W2) {   // 7 fp32 partials per element
+                psum = 1;
+                n_src = kNW * K;
+                src = (unsigned long long)psum_region(M, p_src, rep);
+            }
         }
         e_back = p - p_src;
         const DevLayer& L = fast ? M.fast_layers[ph.layer] : M.layers[ph.layer];
         const uint16_t* nw = kind == PH_QKV ? L.attention_norm : kind == PH_W13 ? L.ffn_norm : kind == PH_HEAD ? (fast ? M.fast_norm : M.norm) : nullptr;
-        const unsigned long long out = (unsigned long long)ll_region(M, tm.team, p, 0);
+        const unsigned long long out = (unsigned long long)(S > 0 && kind == PH_W2 ? psum_region(M, p, 0) : ll_region(M, tm.team, p, 0));
         unsigned long long aux = 0ull;
         if (kind == PH_QKV) aux = (unsigned long long)(fast ? M.fast_rope + (size_t)ph.depth_pos * kHeadDim : M.rope);
         if (kind == PH_HEAD) {
@@ -288,11 +344,12 @@ __device__ __forceinline__ void build_desc(const DevModel& M, const Team& tm, in
         w[8] = (uint32_t)wp; w[9] = (uint32_t)(wp >> 32);
     }
     const int res_sel = (kind == PH_QKV || kind == PH_WO) ? 0 : 1;
-    w[10] = (uint32_t)e_back | ((uint32_t)src_kind << 8) | ((uint32_t)nrep << 12) | ((uint32_t)res_sel << 20) | ((uint32_t)gather << 21);
+    w[10] = (uint32_t)e_back | ((uint32_t)src_kind << 8) | ((uint32_t)nrep << 12) | ((uint32_t)res_sel << 20) | ((uint32_t)gather << 21) |
+            ((uint32_t)psum << 22);
     w[11] = (uint32_t)K | ((uint32_t)n_items << 16);
     w[12] = (uint32_t)kind | ((uint32_t)(fast ? 1 : 0) << 4) | ((uint32_t)ph.layer << 8) | ((uint32_t)ph.depth_pos << 16);
     w[13] = (uint32_t)i0;
-    w[15] = (uint32_t)M.ll_len[p] | ((uint32_t)n_src << 16);
+    w[15] = (uint32_t)(S > 0 && kind == PH_W2 ? kNW * M.dim : M.ll_len[p]) | ((uint32_t)n_src << 16);
 #pragma unroll
     for (int i = 0; i < kDescWords / 4; ++i) sts_v4(dsc + 16u * i, make_uint4(w[4 * i], w[4 * i + 1], w[4 * i + 2], w[4 * i + 3]));
 }
@@ -314,7 +371,8 @@ __device__ __noinline__ void producer(const CallArgs& A, const SmemPlan& SP, uin
             const uint4 d2 = lds_v4(dsc + 32u), d3 = lds_v4(dsc + 48u);
             const int kind = (int)(d3.x & 15u);
             const int n_items = (int)(d2.w >> 16), K = (int)(d2.w & 0xffffu);
-            if (kind == PH_ATTN || kind == PH_SAMPLE || n_items == 0) continue;
+            const bool units = kind == PH_W2 && d3.z != 0u;   // fused MLP: the K-slice of each of this CTA's w2 row tiles
+            if (kind == PH_ATTN || kind == PH_SAMPLE || (n_items == 0 && !units)) continue;
             const bool fast = (d3.x >> 4) & 1u;
             const unsigned char* wp = reinterpret_cast<const unsigned char*>((unsigned long long)d2.x | ((unsigned long long)d2.y << 32));
             // the slow transformer's weights are read once per frame: evict first; the depth transformer's are re-read
@@ -322,6 +380,19 @@ __device__ __noinline__ void producer(const CallArgs& A, const SmemPlan& SP, uin
             const uint64_t pol = (fast && kind != PH_HEAD) ? pol_keep : pol_stream;
             const int tiles = n_items, chunks = phase_chunks(K), kb = K / 32;
             const size_t tile_bytes = (size_t)K * 32;
+            if (units) {   // one stage per (row tile, slice): k-blocks lo .. hi - 1 of tiles i0, i0 + S, ..
+                const int lo = (int)(d3.z & 255u), hi = (int)((d3.z >> 8) & 255u), nu = (int)(d3.z >> 16);
+                const uint32_t bytes = (uint32_t)((hi - lo) * 1024);
+                for (int u = 0; u < nu; ++u) {
+                    if (stage >= ns) mbar_wait(empty0 + 8u * slot, par ^ 1u);
+                    const uint32_t bar = full0 + 8u * slot;
+                    mbar_expect_tx(bar, bytes);
+                    bulk_g2s(ring + slot * (uint32_t)kLL2SlotBytes, wp + (size_t)u * A.mlp_cluster * tile_bytes + (size_t)lo * 1024, bytes, bar, pol);
+                    ++stage;
+                    if (++slot == ns) { slot = 0u; par ^= 1u; }
+                }
+                continue;
+            }
             for (int t = 0; t < tiles; ++t) {
                 for (int kc = 0; kc < chunks; ++kc) {
                     const int kb0 = kc * kLL2ChunkKb, nkb = min(kLL2ChunkKb, kb - kb0);
@@ -469,6 +540,54 @@ __device__ __noinline__ float gather_words(const unsigned long long* src, int n_
             ss = fmaf(bf_hi(v[i].z), bf_hi(v[i].z), ss);
         }
     }
+    return ss;
+}
+
+// Staging of the output of a FUSED MLP: x = bf16(h + bf16(sum of the 7 fp32 partials, in slice order)) -- the reduction and
+// the residual epilogue of the unfused W2 phase, with h from res_h (staged by the W13 phase).  Region: word s * K + e = the
+// partial of slice s for element e.  The element -> thread map (and so the sum of squares) is that of gather_words: thread
+// t holds elements 4 t .. 4 t + 3 (K <= 768: one quad per thread).
+__device__ __noinline__ float gather_psum(const unsigned long long* src, int K, uint32_t e_src, uint32_t dst, uint32_t dst2, uint32_t resh) {
+    const int tid = threadIdx.x;
+    const bool need = 4 * tid < K;
+    uint4 v[kNW][2];
+#pragma unroll
+    for (int s = 0; s < kNW; ++s) {
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+            v[s][h] = make_uint4(0u, e_src, 0u, e_src);
+            if (need) v[s][h] = ld_relaxed_v4(src + s * K + 4 * tid + 2 * h);
+        }
+    }
+    uint32_t spins = 0;
+    for (;;) {
+        bool ready = true;
+#pragma unroll
+        for (int s = 0; s < kNW; ++s) {
+#pragma unroll
+            for (int h = 0; h < 2; ++h)
+                if (v[s][h].y != e_src || v[s][h].w != e_src) { ready = false; v[s][h] = ld_relaxed_v4(src + s * K + 4 * tid + 2 * h); }
+        }
+        if (ready) break;
+        LL2_SPIN_GUARD(spins);
+    }
+    if (!need) return 0.f;
+    const uint32_t hw0 = lds_u32(resh + (uint32_t)tid * 8u), hw1 = lds_u32(resh + (uint32_t)tid * 8u + 4u);
+    const float hv[4] = {bf_lo(hw0), bf_hi(hw0), bf_lo(hw1), bf_hi(hw1)};
+    float x[4];
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+        float a = 0.f;
+#pragma unroll
+        for (int s = 0; s < kNW; ++s) a = __fadd_rn(a, __uint_as_float((e & 1) ? v[s][e >> 1].z : v[s][e >> 1].x));
+        x[e] = bf16_round(__fadd_rn(hv[e], bf16_round(a)));
+    }
+    const uint32_t o0 = pack_bf16(x[0], x[1]), o1 = pack_bf16(x[2], x[3]);
+    sts_v2(dst + (uint32_t)tid * 8u, o0, o1);
+    if (dst2) sts_v2(dst2 + (uint32_t)tid * 8u, o0, o1);
+    float ss = 0.f;
+#pragma unroll
+    for (int e = 0; e < 4; ++e) ss = fmaf(x[e], x[e], ss);
     return ss;
 }
 
@@ -1097,12 +1216,14 @@ smol_ll2_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Call
 #define FKV (sm0 + (uint32_t)SP.fkv)
 #define SCR (sm0 + (uint32_t)SP.scratch)
 #define RING (sm0 + (uint32_t)SP.ring)
+#define ACT (sm0 + (uint32_t)SP.act)
 #define NSLOTS ((uint32_t)SP.n_slots)
 
     {
         const Seq sq = seq_of(M, A, tm.team);
         if (tid == 0) {
             for (int i = 0; i < SP.n_slots; ++i) { mbar_init(full0 + 8u * i, 1u); mbar_init(empty0 + 8u * i, (uint32_t)kNW); }
+            mbar_init(smem_u32(&s_actbar), 1u);
             asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
             s_pos = ldcg_i32(sq.seq_len);
             s_step = sq.step ? ldcg_i32(sq.step) : 0;
@@ -1110,11 +1231,12 @@ smol_ll2_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Call
             s_best = 0u;
         }
         if (tid < M.n_rows) { s_tok[tid] = ldcg_i32(sq.tokens + tid); s_nw[tid] = 0; }
-        for (int p = tid; p < per_iter; p += kLL2Threads) build_desc(M, tm, p, DSC0 + (uint32_t)p * (kDescWords * 4u));
+        for (int p = tid; p < per_iter; p += kLL2Threads) build_desc(M, tm, A.mlp_cluster, p, DSC0 + (uint32_t)p * (kDescWords * 4u));
         for (int i = tid; i < kBtabCache && i < A.b.max_pages; i += kLL2Threads) s_btab[i] = ldcg_i32(sq.btab + i);
     }
     __syncthreads();
     if (tid == 0) s_epoch0 = (uint32_t)ldcg_i32(M.ll_epoch);
+    if (A.mlp_cluster > 0) cluster_sync_all();   // every act barrier of the cluster is initialised before the first DSMEM store
     __syncthreads();
 
     if (warp == kNW) {  // the TMA producer warp
@@ -1137,6 +1259,7 @@ smol_ll2_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Call
     uint32_t tile_ctr = 0;   // tiles reduced so far: the reducing warp rotates with it
     uint32_t pass_ctr = 0;   // passes so far: parity of the partial-sum buffer
     uint32_t cslot = 0, cpar = 0;   // ring slot and parity of the next stage this CTA consumes
+    uint32_t mlp_par = 0;           // fused MLP: parity of the act barrier's next phase
     const int g = lane >> 2, c = lane & 3;
     uint32_t t_end = clock32_now();
     for (int it = 0; it < A.n_iter; ++it) {
@@ -1176,6 +1299,9 @@ smol_ll2_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Call
             const unsigned long long aux = (unsigned long long)d1.z | ((unsigned long long)d1.w << 32);
             const int len_out = (int)(d3.w & 0xffffu), n_src = (int)(d3.w >> 16);
             const int i0 = (int)d3.y;
+            const uint32_t mlp = kind == PH_W13 ? d3.z : 0u;   // fused MLP: lo | hi << 8 | n_units << 16 (0: unfused)
+            const int mlp_lo = (int)(mlp & 255u), mlp_hi = (int)((mlp >> 8) & 255u);
+            if (mlp != 0u && tid == 0) mbar_expect_tx(smem_u32(&s_actbar), (uint32_t)(mlp_hi - mlp_lo) * 64u);  // the slice's act, bf16
 
             const int Hq = fast ? M.fn_head : M.n_head, Hkv = fast ? M.fn_kv : M.n_kv;
             const int q_rows = Hq * kHeadDim, k_end = (Hq + Hkv) * kHeadDim;
@@ -1208,6 +1334,7 @@ smol_ll2_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Call
             } else if (do_gather) {
                 if (SP.holdoff > 0) { while (clock32_now() - t_end < (uint32_t)SP.holdoff) {} }
                 if (kind == PH_WO && fast) fast_attention(M, layer, depth_pos, src, e_src, FQ, FKV, XB);
+                else if ((d2.z >> 22) & 1u) ss = gather_psum(src, K, e_src, XB, (normed && kind != PH_HEAD) ? res : 0u, RESH);
                 else ss = gather_words(src, n_src, e_src, XB, (normed && kind != PH_HEAD) ? res : 0u);
             }
             LL2_TRACE(1);
@@ -1324,20 +1451,69 @@ smol_ll2_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Call
                     const float nxt = __shfl_down_sync(0xffffffffu, val, 1);
                     const uint32_t word = pack_bf16(val, nxt);
                     if (kind == PH_QKV && !fast && valid && !(lane & 1) && n >= q_rows) kv_append(M, A, tm.team, layer, n, word);
+                    if (mlp != 0u) {
+                        // fused MLP: the tile's 8 act values (16 bytes) into every CTA of the cluster, lane r -> rank r
+                        const uint32_t a0 = __shfl_sync(0xffffffffu, word, 0), a1 = __shfl_sync(0xffffffffu, word, 2);
+                        const uint32_t a2 = __shfl_sync(0xffffffffu, word, 4), a3 = __shfl_sync(0xffffffffu, word, 6);
+                        if (lane < A.mlp_cluster) {
+                            const uint32_t dst = ACT + (uint32_t)(((i0 + t) * 8 - mlp_lo * 32) * 2);
+                            st_async_v4(mapa(dst, (uint32_t)lane), a0, a1, a2, a3, mapa(smem_u32(&s_actbar), (uint32_t)lane));
+                        }
+                    } else {
 #pragma unroll
-                    for (int rnd = 0; rnd < 2; ++rnd) {
-                        const int idx = lane + 32 * rnd;
-                        const int wi = nrep == 1 ? idx : idx >> 3, rp = nrep == 1 ? 0 : idx & 7;
-                        const int sl = 2 * (wi & 7);
-                        const uint32_t wv = __shfl_sync(0xffffffffu, word, sl);
-                        const int wn = __shfl_sync(0xffffffffu, n, sl);
-                        const int wok = __shfl_sync(0xffffffffu, valid ? 1 : 0, sl);
-                        if (wi < 8 && wok && (nrep > 1 || rnd == 0)) st_relaxed_v2(out + (size_t)rp * len_out + (wn >> 1), wv, epoch);
+                        for (int rnd = 0; rnd < 2; ++rnd) {
+                            const int idx = lane + 32 * rnd;
+                            const int wi = nrep == 1 ? idx : idx >> 3, rp = nrep == 1 ? 0 : idx & 7;
+                            const int sl = 2 * (wi & 7);
+                            const uint32_t wv = __shfl_sync(0xffffffffu, word, sl);
+                            const int wn = __shfl_sync(0xffffffffu, n, sl);
+                            const int wok = __shfl_sync(0xffffffffu, valid ? 1 : 0, sl);
+                            if (wi < 8 && wok && (nrep > 1 || rnd == 0)) st_relaxed_v2(out + (size_t)rp * len_out + (wn >> 1), wv, epoch);
+                        }
                     }
                 }
                 tile_ctr += (uint32_t)nt;
                 pass_ctr += 1u;
                 t0 += nt;
+            }
+            if (mlp != 0u) {
+                // ---- fused MLP, w2 part: one warp per row tile replays warp `slice`'s MMA chain of the unfused K sweep ------
+                const int nu = (int)(mlp >> 16), nkb = mlp_hi - mlp_lo, S = A.mlp_cluster, slice = tm.cta / S;
+                const uint32_t dw = dsc + (uint32_t)(kDescWords * 4);   // the W2 phase's descriptor: region, row tile i0
+                const uint4 w1 = lds_v4(dw + 16u), w3 = lds_v4(dw + 48u);
+                unsigned long long* out2 = reinterpret_cast<unsigned long long*>((unsigned long long)w1.x | ((unsigned long long)w1.y << 32));
+                const int len2 = (int)(w3.w & 0xffffu), D = (fast ? M.fdim : M.dim);
+                mbar_wait(smem_u32(&s_actbar), mlp_par);   // the slice's act values from every CTA of the cluster
+                mlp_par ^= 1u;
+#pragma unroll 1
+                for (int u = warp; u < nu; u += kNW) {
+                    uint32_t sl = cslot + (uint32_t)u, pr = cpar;
+                    while (sl >= NSLOTS) { sl -= NSLOTS; pr ^= 1u; }
+                    mbar_wait(full0 + 8u * sl, pr);
+                    const uint32_t ab = RING + sl * (uint32_t)kLL2SlotBytes + (uint32_t)lane * 16u, xb = ACT + (uint32_t)c * 16u;
+                    float acc[4] = {0.f, 0.f, 0.f, 0.f}, acd[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll 1
+                    for (int j = 0; j < nkb; ++j) {
+                        const uint4 bx = lds_v4(xb + (uint32_t)j * 64u);
+                        const uint4 a0 = lds_v4(ab + (uint32_t)j * 1024u), a1 = lds_v4(ab + (uint32_t)j * 1024u + 512u);
+                        mma_bf16_16816(acc, a0.x, a0.y, a0.z, a0.w, bx.x, bx.y);
+                        mma_bf16_16816(acd, a1.x, a1.y, a1.z, a1.w, bx.z, bx.w);
+                    }
+                    __syncwarp();
+                    if (lane == 0) mbar_arrive_n(empty0 + 8u * sl, (uint32_t)kNW);   // the stage's only consumer
+                    // partials of row slots g (acc[0] + acd[0]) and g + 8 (acc[2] + acd[2]), held by the lanes with c == 0:
+                    // lane l publishes row slot l & 15 to replicas l >> 4, + 2, + 4, + 6
+                    const float q0 = __fadd_rn(acc[0], acd[0]), q1 = __fadd_rn(acc[2], acd[2]);
+                    const int rs = lane & 15;
+                    const float qa = __shfl_sync(0xffffffffu, q0, (rs & 7) * 4), qb = __shfl_sync(0xffffffffu, q1, (rs & 7) * 4);
+                    const uint32_t pv = __float_as_uint(rs < 8 ? qa : qb);
+                    unsigned long long* o = out2 + slice * D + ((int)w3.y + u * S) * 16 + rs;   // w3.y = first row tile
+#pragma unroll
+                    for (int i = 0; i < kLLRep / 2; ++i) st_relaxed_v2(o + (size_t)((lane >> 4) + 2 * i) * len2, pv, epoch + 1u);
+                }
+                uint32_t sl = cslot + (uint32_t)nu;
+                while (sl >= NSLOTS) { sl -= NSLOTS; cpar ^= 1u; }
+                cslot = sl;
             }
             if (kind == PH_HEAD && M.force == nullptr && (fast ? A.s.fast_temp : A.s.temp) == 0.0f) {
                 // greedy row: the CTA's best (logit, index) goes out as one word per replica
@@ -1419,6 +1595,7 @@ bool ll2_plan(const DevModel& M, int holdoff, int flags, ll2::SmemPlan* sp, size
     const size_t attn = (size_t)lmax * 4 + (size_t)(lmax / kLL2ScoreBlock) * 9 * 4;
     if (attn > sc) sc = attn;
     sp->scratch = take(sc);
+    sp->act = take((size_t)((kmax / 32 + ll2::kNW - 1) / ll2::kNW) * 32 * 2);   // the largest K-slice of act (fused MLP)
     off = (off + 1023) / 1024 * 1024;
     sp->ring = (int)off;
     const size_t budget = 227 * 1024 - 4096;   // static shared memory (barriers, sampler scratch, state) stays below 4 KB
@@ -1443,11 +1620,62 @@ cudaError_t ll2_configure(size_t smem) {
 cudaError_t ll2_max_ctas(size_t smem, int* per_sm) {
     return cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, ll2::smol_ll2_kernel<true>, kLL2Threads, smem);
 }
+// Cluster size of the fused gated MLP: the largest S <= 16 with at least 7 co-resident clusters of S CTAs (one per K-slice;
+// an 8th is taken when it fits: it idles in the MLP phases but gives the other phases a larger grid).  S is also bounded so
+// that every CTA of a slice cluster has a w13 tile and a w2 row tile in every layer: each CTA then both sends act values
+// and waits for them, which keeps consecutive layers' DSMEM hand-offs from overlapping (one act buffer, one barrier).
+// Returns 0 when no cluster size fits (the kernel then runs the unfused program).
+int ll2_mlp_cluster(const DevModel& M, size_t smem, int n_slots, int* n_clusters) {
+    *n_clusters = 0;
+    int smax = 16;
+    smax = std::min(smax, std::min(M.dim, M.fdim) / 16);
+    smax = std::min(smax, 4 * ((std::min(M.inter, M.finter) / 32) / ll2::kNW));
+    // a CTA's w2 row tiles: one warp and one ring stage each, all stages in the ring at once (a warp waits on stage
+    // cslot + u with its parity: safe only while no two of them share a slot)
+    const int rt = M.dim / 16, max_units = std::min(ll2::kNW, n_slots);
+    int smin = (rt + max_units - 1) / max_units;
+    const void* fns[2] = {(const void*)ll2::smol_ll2_kernel<false>, (const void*)ll2::smol_ll2_kernel<true>};
+    for (const void* fn : fns)
+        if (cudaFuncSetAttribute(fn, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) != cudaSuccess) { (void)cudaGetLastError(); return 0; }
+    for (int S = smax; S >= smin && S >= 1; --S) {
+        cudaLaunchConfig_t cfg = {};
+        cfg.gridDim = dim3(8 * S);
+        cfg.blockDim = dim3(kLL2Threads);
+        cfg.dynamicSmemBytes = smem;
+        cudaLaunchAttribute at[1];
+        at[0].id = cudaLaunchAttributeClusterDimension;
+        at[0].val.clusterDim.x = S; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+        cfg.attrs = at;
+        cfg.numAttrs = 1;
+        int n = 0;
+        if (cudaOccupancyMaxActiveClusters(&n, fns[1], &cfg) != cudaSuccess) { (void)cudaGetLastError(); continue; }
+        if (n >= ll2::kNW) {
+            *n_clusters = std::min(n, ll2::kNW + 1);
+            return S;
+        }
+    }
+    return 0;
+}
+
 cudaError_t ll2_launch(const DevModel& M, const CallArgs& A, const ll2::SmemPlan& sp, size_t smem, int n_ctas, cudaStream_t stream) {
     void* args[3] = {(void*)&M, (void*)&A, (void*)&sp};
-    // cooperative launch only for the co-residency guarantee: CTAs spin on each other's words
     const void* fn = M.prof != nullptr ? (const void*)ll2::smol_ll2_kernel<true> : (const void*)ll2::smol_ll2_kernel<false>;
-    return cudaLaunchCooperativeKernel(fn, dim3(n_ctas), dim3(kLL2Threads), args, smem, stream);
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(n_ctas);
+    cfg.blockDim = dim3(kLL2Threads);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = stream;
+    cudaLaunchAttribute at[2];
+    at[0].id = cudaLaunchAttributeCooperative;   // only for the co-residency guarantee: CTAs spin on each other's words
+    at[0].val.cooperative = 1;
+    cfg.numAttrs = 1;
+    if (A.mlp_cluster > 0) {
+        at[1].id = cudaLaunchAttributeClusterDimension;
+        at[1].val.clusterDim.x = A.mlp_cluster; at[1].val.clusterDim.y = 1; at[1].val.clusterDim.z = 1;
+        cfg.numAttrs = 2;
+    }
+    cfg.attrs = at;
+    return cudaLaunchKernelExC(&cfg, fn, args);
 }
 
 }  // namespace smol

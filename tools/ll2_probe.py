@@ -118,12 +118,25 @@ def timing(args):
         us = [run(args.frames) for _ in range(2)]
         print(f"n_ctas={n:4d}: {min(us):8.1f} us/frame")
     model.set_option("n_ctas", 0)
+    for fused in (1, 0, 1):   # the fused gated MLP (clusters, DSMEM) against the unfused program
+        model.set_option("ll_fused_mlp", fused)
+        run(8)
+        us = [run(args.frames) for _ in range(2)]
+        print(f"ll_fused_mlp={fused} (ran fused: {model.get_option('ll_last_fused')}, cluster {model.get_option('ll_mlp_cluster')} "
+              f"x {model.get_option('ll_mlp_clusters')}, grid {model.get_option('ll_mlp_cluster') * model.get_option('ll_mlp_clusters')}): "
+              f"{min(us):8.1f} us/frame")
+    model.set_option("ll_fused_mlp", args.trace_fused)
     # cycle trace at the default hold-off
     model.set_option("ll_holdoff", args.trace_holdoff)
     run(8)
     prof = model.set_profile(True)
     us = run(args.frames)
     model.set_profile(False)
+    fused = model.get_option("ll_last_fused") == 1
+
+    def kind_of(p):   # fused MLP: the W13 phase runs w13 and w2; the W2 phase has no work left
+        k = phase_kind(p, cfg.n_layer, cfg.n_fast_layer)
+        return k + ("+W2 (fused)" if k.endswith("W13") else " (empty)" if k.endswith("W2") else "") if fused else k
     trace = prof.cpu().numpy()[2 * 512 + 64: 2 * 512 + 64 + 2 * 512 * 8].reshape(2, 512, 8)
     print(f"profiling build, hold-off {args.trace_holdoff}: {us:.1f} us/frame")
     names = ["staged", "bar1", "bfrag", "weights", "mma", "bar2", "epilogue", "total"]
@@ -134,7 +147,7 @@ def timing(args):
             t = trace[slot, p].astype(float)
             if t[0] == 0:
                 continue
-            k = phase_kind(p, cfg.n_layer, cfg.n_fast_layer)
+            k = kind_of(p)
             if t[2] == 0:
                 d = [0, 0, 0, 0, 0, 0, 0, t[6] - t[0]]
             else:
@@ -147,7 +160,7 @@ def timing(args):
             acc[k] = ([x + y for x, y in zip(a0, d)], n0 + 1)
         tot = 0.0
         for k, (v, n) in acc.items():
-            print(f"  {label:8s} {k:12s} x{n:3d} " + " ".join(f"{x / n:8.0f}" for x in v))
+            print(f"  {label:8s} {k:24s} x{n:3d} " + " ".join(f"{x / n:8.0f}" for x in v))
             tot += v[7]
         print(f"  {label}: {tot:.0f} cycles per frame in phases")
     # skew trace: %globaltimer of every CTA when its input is staged (0) and at the end of the phase (1)
@@ -160,7 +173,7 @@ def timing(args):
             end_prev, arr, end = skew[:n_ctas, p - 1, 1], skew[:n_ctas, p, 0], skew[:n_ctas, p, 1]
             if (end_prev <= 0).any() or (end <= 0).any():
                 continue
-            k = phase_kind(p, cfg.n_layer, cfg.n_fast_layer)
+            k = kind_of(p)
             have = arr > 0
             a0 = acc.setdefault(k, [[], [], [], []])
             a0[0].append(end.max() - end_prev.max())                        # phase period: last end -> last end
@@ -219,6 +232,7 @@ def main():
     ap.add_argument("--trace-holdoff", type=int, default=400)
     ap.add_argument("--staggers", default="0,250,350")
     ap.add_argument("--trace-stagger", type=int, default=0)
+    ap.add_argument("--trace-fused", type=int, default=1, help="ll_fused_mlp of the cycle / skew trace")
     ap.add_argument("--n-ctas", default="", help="comma list of grid sizes to time")
     ap.add_argument("--skip-check", action="store_true")
     ap.add_argument("--skip-timing", action="store_true")
