@@ -70,6 +70,9 @@ struct SmolModel {
     int ll2_cluster = 0;       // CTAs per cluster of the fused MLP (0: no cluster size fits this model / GPU)
     int ll2_clusters = 0;      // clusters of the fused grid
     int ll2_last_fused = 0;    // the last data-flow launch ran the fused MLP
+    int ll2_psum_split = 1;    // option "ll_psum_split": the fused MLP's output is staged by each cluster together (1) or by
+                               // every CTA alone (0: each polls all 7 x dim partial-sum words)
+    int ll2_last_split = 0;    // the last data-flow launch staged the fused MLP's output cluster-split
     smol::ll2::SmemPlan ll2_sp;
     size_t ll2_smem = 0;
     bool packed_ready = false; // tensor-core GEMV layout of the bound weights (rebuilt after a weight / workspace bind)
@@ -554,7 +557,9 @@ static int enqueue(SmolModel* m, CallArgs A, cudaStream_t stream, bool whole_ite
             if (A.n_iter == 0) return SMOL_OK;
             A.team_ctas = A.batch == 1 ? ll2_solo_ctas(m) : m->n_ctas / A.batch;
             A.mlp_cluster = A.batch == 1 ? ll2_fused_cluster(m, &A.team_ctas) : 0;
+            A.psum_split = A.mlp_cluster > 0 ? m->ll2_psum_split : 0;
             m->ll2_last_fused = A.mlp_cluster > 0 ? 1 : 0;
+            m->ll2_last_split = A.psum_split;
             m->ll2_sp.holdoff = m->ll2_holdoff;
             m->ll2_sp.flags = m->ll_flags;
             CU(smol::ll2_launch(m->dm, A, m->ll2_sp, m->ll2_smem, A.team_ctas * A.batch, stream));
@@ -840,6 +845,10 @@ int smol_set_option(SmolModel* m, const char* name, int64_t value) {
         m->ll2_fused_mlp = value != 0 ? 1 : 0;
         return SMOL_OK;
     }
+    if (!std::strcmp(name, "ll_psum_split")) {
+        m->ll2_psum_split = value != 0 ? 1 : 0;
+        return SMOL_OK;
+    }
     if (!std::strcmp(name, "ll_max_batch")) {
         if (value < 0 || value > smol::kLL2MaxTeams) return fail(SMOL_ERR_INVALID, "ll_max_batch must be in [0, 8]");
         m->ll2_max_batch = (int)value;
@@ -874,6 +883,8 @@ int64_t smol_get_option(const SmolModel* m, const char* name) {
     if (!std::strcmp(name, "ll_mlp_cluster")) return (int64_t)m->ll2_cluster;
     if (!std::strcmp(name, "ll_mlp_clusters")) return (int64_t)m->ll2_clusters;
     if (!std::strcmp(name, "ll_last_fused")) return (int64_t)m->ll2_last_fused;
+    if (!std::strcmp(name, "ll_psum_split")) return (int64_t)m->ll2_psum_split;
+    if (!std::strcmp(name, "ll_last_split")) return (int64_t)m->ll2_last_split;
     return -1;
 }
 

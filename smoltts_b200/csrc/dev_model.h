@@ -173,6 +173,7 @@ struct CallArgs {
     int tc_split;     // tensor-core variant: cached positions per attention split (0 = default)
     int team_ctas;    // second-generation data-flow kernel: CTAs per sequence (one team each); grid = batch * team_ctas
     int mlp_cluster;  // data-flow kernel, batch 1: CTAs per thread-block cluster of the fused gated MLP (0 = unfused)
+    int psum_split;   // fused MLP: the CTAs of a cluster share the staging of the partial sums (ll2_kernel.cu: gather_psum_split)
     const int32_t* prompt;      // prefill: [B][n_rows][s_max]
     const int32_t* prompt_len;  // prefill: [B]
     int s_max;

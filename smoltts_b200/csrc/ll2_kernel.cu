@@ -183,6 +183,11 @@ __device__ __forceinline__ void st_async_v4(uint32_t a, uint32_t x, uint32_t y, 
     asm volatile("st.async.shared::cluster.mbarrier::complete_tx::bytes.v4.b32 [%0], {%1,%2,%3,%4}, [%5];"
                  ::"r"(a), "r"(x), "r"(y), "r"(z), "r"(w), "r"(bar) : "memory");
 }
+// 8 bytes, likewise
+__device__ __forceinline__ void st_async_v2(uint32_t a, uint32_t x, uint32_t y, uint32_t bar) {
+    asm volatile("st.async.shared::cluster.mbarrier::complete_tx::bytes.v2.b32 [%0], {%1,%2}, [%3];"
+                 ::"r"(a), "r"(x), "r"(y), "r"(bar) : "memory");
+}
 __device__ __forceinline__ void cluster_sync_all() {
     asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
 }
@@ -191,6 +196,7 @@ __device__ __forceinline__ void cluster_sync_all() {
 __shared__ __align__(8) uint64_t s_full[kMaxSlots];
 __shared__ __align__(8) uint64_t s_empty[kMaxSlots];
 __shared__ __align__(8) uint64_t s_actbar;   // fused MLP: the slice's act values have arrived from the cluster
+__shared__ __align__(8) uint64_t s_psumbar;  // fused MLP, split staging: the whole output vector has arrived from the cluster
 __shared__ SampleScratch s_sc;
 __shared__ float s_ssq[kNW];            // per-warp partial sums of squares (RMSNorm)
 __shared__ uint32_t s_best;             // HEAD phases: the CTA's best (logit, index) candidate
@@ -214,12 +220,14 @@ struct Team {
 //         4-5  out      LL region this phase publishes to (this team, replica 0)
 //         6-7  aux      QKV: RoPE table | HEAD: fp32 logits dump
 //         8-9  wptr     packed weights: first 8-row group of this CTA
-//        10    e_back | src_kind << 8 | nrep << 12 | res_sel << 20 | gather << 21
+//        10    e_back | src_kind << 8 | nrep << 12 | res_sel << 20 | gather << 21 | psum << 22 (input = a fused MLP's
+//              partial sums: 1 every CTA polls all of them, gather_psum; 2 the cluster splits them, gather_psum_split)
 //        11    K | n_items << 16
 //        12    kind | fast << 4 | layer << 8 | depth_pos << 16
 //        13    first item of this CTA
 //        14    fused MLP (W13 and W2 phases): lo | hi << 8 | n_units << 16 -- the K-slice [lo, hi) (k-blocks of w2) of this
 //              CTA's cluster and the W2 row tiles this CTA carries (i0, i0 + S, ..); 0 = not fused / no work
+//              psum == 2 (the phase after a W2 phase): j0 | n_quads << 16 -- the quads of the input vector this CTA stages
 //        15    len_out (words per replica of the output region) | n_src_words << 16
 //
 // Fused gated MLP (batch 1, A.mlp_cluster = S > 0; grid = clusters of S CTAs).  The 7 consumer warps split a w2 tile's
@@ -228,7 +236,8 @@ struct Team {
 // hand them to each other through DSMEM, and then run warp c's chain of every w2 row tile, one warp per tile, publishing
 // the fp32 partial sums with the W2 phase's epoch.  The consumers of the W2 region add the 7 partials in range order and
 // the residual (the bf16 roundings of the unfused epilogue): bit for bit the unfused result, with one L2 exchange per
-// MLP instead of two.  The W2 phase itself has no tiles and no input.
+// MLP instead of two.  The W2 phase itself has no tiles and no input: it stays in the program (epochs, descriptors and the
+// producer's stream are those of the unfused program) but the consumer warps never visit it.
 __device__ __forceinline__ int phase_rows(const DevModel& M, const Phase& ph) {
     const bool fast = ph.fast != 0;
     switch (ph.kind) {
@@ -273,7 +282,7 @@ __device__ __forceinline__ unsigned long long* psum_region(const DevModel& M, in
     return M.ll2_psum + ((size_t)w2 * kLLRep + rep) * kNW * M.dim;
 }
 
-__device__ __forceinline__ void build_desc(const DevModel& M, const Team& tm, int S, int p, uint32_t dsc) {
+__device__ __forceinline__ void build_desc(const DevModel& M, const Team& tm, int S, int split, int p, uint32_t dsc) {
     const int rep = tm.cta % kLLRep;
     const Phase ph = unpack_phase(M.prog[p]);
     const bool fast = ph.fast != 0;
@@ -321,6 +330,14 @@ __device__ __forceinline__ void build_desc(const DevModel& M, const Team& tm, in
                 psum = 1;
                 n_src = kNW * K;
                 src = (unsigned long long)psum_region(M, p_src, rep);
+                // Split staging (gather_psum_split) where its early DSMEM stores are safe: in the phase right after the
+                // W2 phase (not the depth-0 QKV, which follows HEAD + SAMPLE) and in a slice cluster (not the idle one)
+                const int slice = tm.cta / S, r = tm.cta - slice * S, q = K / 4;
+                if (split && p_src == p - 1 && slice < kNW && 2 * ((q + S - 1) / S) <= kCons) {
+                    psum = 2;
+                    const int j0 = (q * r) / S, j1 = (q * (r + 1)) / S;
+                    w[14] = (uint32_t)j0 | ((uint32_t)(j1 - j0) << 16);
+                }
             }
         }
         e_back = p - p_src;
@@ -335,8 +352,9 @@ __device__ __forceinline__ void build_desc(const DevModel& M, const Team& tm, in
             nrep = 1;  // logits words are read by the team's sampler CTA only (greedy rows use the candidate words)
         }
         const unsigned long long wp = (unsigned long long)(phase_weights(M, ph) + (size_t)i0 * 16 * K);   // 16 K elements per tile
-        // normed phases stage the residual stream for everybody (the wo / w2 epilogues need their rows of it)
-        gather = (kind == PH_QKV || kind == PH_W13) ? 1 : (n_items > 0 ? 1 : 0);
+        // normed phases stage the residual stream for everybody (the wo / w2 epilogues need their rows of it); a split
+        // staging needs every CTA of the cluster, tiles or not
+        gather = (kind == PH_QKV || kind == PH_W13 || psum == 2) ? 1 : (n_items > 0 ? 1 : 0);
         w[0] = (uint32_t)src; w[1] = (uint32_t)(src >> 32);
         w[2] = (uint32_t)(unsigned long long)nw; w[3] = (uint32_t)((unsigned long long)nw >> 32);
         w[4] = (uint32_t)out; w[5] = (uint32_t)(out >> 32);
@@ -585,6 +603,77 @@ __device__ __noinline__ float gather_psum(const unsigned long long* src, int K, 
     const uint32_t o0 = pack_bf16(x[0], x[1]), o1 = pack_bf16(x[2], x[3]);
     sts_v2(dst + (uint32_t)tid * 8u, o0, o1);
     if (dst2) sts_v2(dst2 + (uint32_t)tid * 8u, o0, o1);
+    float ss = 0.f;
+#pragma unroll
+    for (int e = 0; e < 4; ++e) ss = fmaf(x[e], x[e], ss);
+    return ss;
+}
+
+// The same staging shared by the S CTAs of a slice cluster (psum == 2): the CTA of cluster rank r polls only the quads
+// [j0, j0 + nq) = [q r / S, q (r + 1) / S) of the vector (q = K / 4; thread 2 j + h: elements 4 (j0 + j) + 2 h, + 1, all 7
+// partials in flight together), computes them exactly as gather_psum does and sends each quad (8 bytes, st.async) to its
+// place in dst (and dst2) of every CTA of the cluster, itself included.  Everybody then waits on s_psumbar (K * 2 bytes
+// per destination buffer) and takes its sum of squares from dst with gather_words's thread -> element map.
+//
+// The peers' stores may land before this CTA is done with the previous phase.  That is safe:
+//  * A peer forwards its quads only once all 7 slice clusters have published their partials.  This CTA's own cluster
+//    publishes only after every one of its CTAs has sent its act values, and this CTA sends its last ones after its last
+//    W13 tile pass (every CTA of a slice cluster has a w13 tile: ll2_mlp_cluster).  From there on it reads neither xbuf
+//    (the w2 chains read act and the ring) nor res_x (read by WO only), and this phase follows the W2 phase directly.
+//    The idle cluster has no w13 tile and the depth-0 QKV follows HEAD + SAMPLE, which read xbuf: both use gather_psum.
+//  * The bytes of the next split staging cannot reach s_psumbar before this one completes: that staging's input is the
+//    next MLP's partials, which need this CTA's act values of that MLP, sent after the wait below.  So one barrier phase
+//    per staging, with the parity carried by the caller.
+__device__ __noinline__ float gather_psum_split(const unsigned long long* src, int K, uint32_t e_src, uint32_t dst, uint32_t dst2,
+                                                uint32_t resh, uint32_t quads, int S, uint32_t parity) {
+    const int tid = threadIdx.x, lane = tid & 31;
+    const uint32_t bar = smem_u32(&s_psumbar);
+    if (tid == 0) mbar_expect_tx(bar, (uint32_t)K * (dst2 ? 4u : 2u));
+    const int j0 = (int)(quads & 0xffffu), n2 = 2 * (int)(quads >> 16);
+    if ((tid & ~31) < n2) {   // the warps that hold a quad (n2 is even: both halves of a quad are in one warp)
+        const bool mine = tid < n2;
+        const int e = 4 * j0 + 2 * tid;
+        uint4 v[kNW];
+#pragma unroll
+        for (int s = 0; s < kNW; ++s) {
+            v[s] = make_uint4(0u, e_src, 0u, e_src);
+            if (mine) v[s] = ld_relaxed_v4(src + s * K + e);
+        }
+        uint32_t spins = 0;
+        for (;;) {
+            bool ready = true;
+#pragma unroll
+            for (int s = 0; s < kNW; ++s)
+                if (v[s].y != e_src || v[s].w != e_src) { ready = false; v[s] = ld_relaxed_v4(src + s * K + e); }
+            if (ready) break;
+            LL2_SPIN_GUARD(spins);
+        }
+        uint32_t w = 0u;
+        if (mine) {
+            const uint32_t hw = lds_u32(resh + (uint32_t)e * 2u);
+            float a0 = 0.f, a1 = 0.f;
+#pragma unroll
+            for (int s = 0; s < kNW; ++s) {
+                a0 = __fadd_rn(a0, __uint_as_float(v[s].x));
+                a1 = __fadd_rn(a1, __uint_as_float(v[s].z));
+            }
+            w = pack_bf16(bf16_round(__fadd_rn(bf_lo(hw), bf16_round(a0))), bf16_round(__fadd_rn(bf_hi(hw), bf16_round(a1))));
+        }
+        const uint32_t w_other = __shfl_xor_sync(0xffffffffu, w, 1);
+        if (mine) {   // the two threads of a quad share its destinations: ranks h, h + 2, ..
+            const uint32_t lo = (lane & 1) ? w_other : w, hi = (lane & 1) ? w : w_other;
+            const uint32_t off = (uint32_t)(e & ~3) * 2u;
+            for (int d = lane & 1; d < S; d += 2) {
+                const uint32_t rb = mapa(bar, (uint32_t)d);
+                st_async_v2(mapa(dst + off, (uint32_t)d), lo, hi, rb);
+                if (dst2) st_async_v2(mapa(dst2 + off, (uint32_t)d), lo, hi, rb);
+            }
+        }
+    }
+    mbar_wait(bar, parity);
+    if (4 * tid >= K) return 0.f;
+    const uint32_t x01 = lds_u32(dst + (uint32_t)tid * 8u), x23 = lds_u32(dst + (uint32_t)tid * 8u + 4u);
+    const float x[4] = {bf_lo(x01), bf_hi(x01), bf_lo(x23), bf_hi(x23)};
     float ss = 0.f;
 #pragma unroll
     for (int e = 0; e < 4; ++e) ss = fmaf(x[e], x[e], ss);
@@ -1224,6 +1313,7 @@ smol_ll2_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Call
         if (tid == 0) {
             for (int i = 0; i < SP.n_slots; ++i) { mbar_init(full0 + 8u * i, 1u); mbar_init(empty0 + 8u * i, (uint32_t)kNW); }
             mbar_init(smem_u32(&s_actbar), 1u);
+            mbar_init(smem_u32(&s_psumbar), 1u);
             asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
             s_pos = ldcg_i32(sq.seq_len);
             s_step = sq.step ? ldcg_i32(sq.step) : 0;
@@ -1231,12 +1321,12 @@ smol_ll2_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Call
             s_best = 0u;
         }
         if (tid < M.n_rows) { s_tok[tid] = ldcg_i32(sq.tokens + tid); s_nw[tid] = 0; }
-        for (int p = tid; p < per_iter; p += kLL2Threads) build_desc(M, tm, A.mlp_cluster, p, DSC0 + (uint32_t)p * (kDescWords * 4u));
+        for (int p = tid; p < per_iter; p += kLL2Threads) build_desc(M, tm, A.mlp_cluster, A.psum_split, p, DSC0 + (uint32_t)p * (kDescWords * 4u));
         for (int i = tid; i < kBtabCache && i < A.b.max_pages; i += kLL2Threads) s_btab[i] = ldcg_i32(sq.btab + i);
     }
     __syncthreads();
     if (tid == 0) s_epoch0 = (uint32_t)ldcg_i32(M.ll_epoch);
-    if (A.mlp_cluster > 0) cluster_sync_all();   // every act barrier of the cluster is initialised before the first DSMEM store
+    if (A.mlp_cluster > 0) cluster_sync_all();   // every act / psum barrier of the cluster is initialised before the first DSMEM store
     __syncthreads();
 
     if (warp == kNW) {  // the TMA producer warp
@@ -1260,15 +1350,20 @@ smol_ll2_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Call
     uint32_t pass_ctr = 0;   // passes so far: parity of the partial-sum buffer
     uint32_t cslot = 0, cpar = 0;   // ring slot and parity of the next stage this CTA consumes
     uint32_t mlp_par = 0;           // fused MLP: parity of the act barrier's next phase
+    uint32_t psum_par = 0;          // fused MLP, split staging: parity of the psum barrier's next phase
     const int g = lane >> 2, c = lane & 3;
     uint32_t t_end = clock32_now();
     for (int it = 0; it < A.n_iter; ++it) {
+        int step = 1;
 #pragma unroll 1
-        for (int p = 0; p < per_iter; ++p) {
+        for (int p = 0; p < per_iter; p += step) {
             const uint32_t dsc = DSC0 + (uint32_t)p * (kDescWords * 4u);
             const uint32_t epoch = s_epoch0 + (uint32_t)(it * per_iter + p) + 1u;
             const uint4 d2 = lds_v4(dsc + 32u), d3 = lds_v4(dsc + 48u);
             const int kind = (int)(d3.x & 15u);
+            // fused MLP: a W13 phase is always followed by its W2 phase, whose work it does -- the consumer warps skip that
+            // phase (no descriptor, no barrier; t_end stays the W13 phase's end)
+            step = (A.mlp_cluster > 0 && kind == PH_W13) ? 2 : 1;
             const bool fast = (d3.x >> 4) & 1u;
             const int layer = (int)((d3.x >> 8) & 255u), depth_pos = (int)((d3.x >> 16) & 255u);
             LL2_TRACE(0);
@@ -1290,6 +1385,7 @@ smol_ll2_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Call
             const int kb = K >> 5;
             const int src_kind = (int)((d2.z >> 8) & 15u), nrep = (int)((d2.z >> 12) & 63u);
             const bool do_gather = (d2.z >> 21) & 1u;
+            const uint32_t psum = (d2.z >> 22) & 3u;   // input: a fused MLP's partial sums (1: gather_psum, 2: gather_psum_split)
             const uint32_t e_src = epoch - (d2.z & 255u);
             const uint32_t res = ((d2.z >> 20) & 1u) ? RESH : RESX;
             const bool normed = kind == PH_QKV || kind == PH_W13 || kind == PH_HEAD;
@@ -1334,7 +1430,10 @@ smol_ll2_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Call
             } else if (do_gather) {
                 if (SP.holdoff > 0) { while (clock32_now() - t_end < (uint32_t)SP.holdoff) {} }
                 if (kind == PH_WO && fast) fast_attention(M, layer, depth_pos, src, e_src, FQ, FKV, XB);
-                else if ((d2.z >> 22) & 1u) ss = gather_psum(src, K, e_src, XB, (normed && kind != PH_HEAD) ? res : 0u, RESH);
+                else if (psum == 2u) {
+                    ss = gather_psum_split(src, K, e_src, XB, (normed && kind != PH_HEAD) ? res : 0u, RESH, d3.z, A.mlp_cluster, psum_par);
+                    psum_par ^= 1u;
+                } else if (psum == 1u) ss = gather_psum(src, K, e_src, XB, (normed && kind != PH_HEAD) ? res : 0u, RESH);
                 else ss = gather_words(src, n_src, e_src, XB, (normed && kind != PH_HEAD) ? res : 0u);
             }
             LL2_TRACE(1);

@@ -118,14 +118,17 @@ def timing(args):
         us = [run(args.frames) for _ in range(2)]
         print(f"n_ctas={n:4d}: {min(us):8.1f} us/frame")
     model.set_option("n_ctas", 0)
-    for fused in (1, 0, 1):   # the fused gated MLP (clusters, DSMEM) against the unfused program
+    # the fused gated MLP (clusters, DSMEM) with split / per-CTA staging of its partial sums, against the unfused program
+    for fused, split in ((1, 1), (1, 0), (0, 1), (1, 1)):
         model.set_option("ll_fused_mlp", fused)
+        model.set_option("ll_psum_split", split)
         run(8)
         us = [run(args.frames) for _ in range(2)]
-        print(f"ll_fused_mlp={fused} (ran fused: {model.get_option('ll_last_fused')}, cluster {model.get_option('ll_mlp_cluster')} "
-              f"x {model.get_option('ll_mlp_clusters')}, grid {model.get_option('ll_mlp_cluster') * model.get_option('ll_mlp_clusters')}): "
-              f"{min(us):8.1f} us/frame")
+        print(f"ll_fused_mlp={fused} ll_psum_split={split} (ran fused: {model.get_option('ll_last_fused')}, split: "
+              f"{model.get_option('ll_last_split')}, cluster {model.get_option('ll_mlp_cluster')} x {model.get_option('ll_mlp_clusters')}, "
+              f"grid {model.get_option('ll_mlp_cluster') * model.get_option('ll_mlp_clusters')}): {min(us):8.1f} us/frame")
     model.set_option("ll_fused_mlp", args.trace_fused)
+    model.set_option("ll_psum_split", args.trace_split)
     # cycle trace at the default hold-off
     model.set_option("ll_holdoff", args.trace_holdoff)
     run(8)
@@ -134,18 +137,20 @@ def timing(args):
     model.set_profile(False)
     fused = model.get_option("ll_last_fused") == 1
 
-    def kind_of(p):   # fused MLP: the W13 phase runs w13 and w2; the W2 phase has no work left
+    def kind_of(p):   # fused MLP: the W13 phase runs w13 and w2; the W2 phase is not visited
         k = phase_kind(p, cfg.n_layer, cfg.n_fast_layer)
-        return k + ("+W2 (fused)" if k.endswith("W13") else " (empty)" if k.endswith("W2") else "") if fused else k
+        return k + ("+W2 (fused)" if k.endswith("W13") else " (skipped)" if k.endswith("W2") else "") if fused else k
     trace = prof.cpu().numpy()[2 * 512 + 64: 2 * 512 + 64 + 2 * 512 * 8].reshape(2, 512, 8)
     print(f"profiling build, hold-off {args.trace_holdoff}: {us:.1f} us/frame")
     names = ["staged", "bar1", "bfrag", "weights", "mma", "bar2", "epilogue", "total"]
     print("cycle trace of the last frame, mean cycles per phase kind: " + " | ".join(names))
     for slot, label in ((0, "CTA 0"), (1, "CTA n/2")):
-        acc = {}
+        acc, skipped = {}, {}
         for p in range(model.phase_count):
             t = trace[slot, p].astype(float)
-            if t[0] == 0:
+            if t[0] == 0:   # a phase the consumer warps did not visit
+                k = kind_of(p)
+                skipped[k] = skipped.get(k, 0) + 1
                 continue
             k = kind_of(p)
             if t[2] == 0:
@@ -162,18 +167,25 @@ def timing(args):
         for k, (v, n) in acc.items():
             print(f"  {label:8s} {k:24s} x{n:3d} " + " ".join(f"{x / n:8.0f}" for x in v))
             tot += v[7]
+        for k, n in skipped.items():
+            print(f"  {label:8s} {k:24s} x{n:3d} skipped")
         print(f"  {label}: {tot:.0f} cycles per frame in phases")
     # skew trace: %globaltimer of every CTA when its input is staged (0) and at the end of the phase (1)
     skew = prof.cpu().numpy()[2 * 512 + 64 + 2 * 512 * 8:].reshape(256, 512, 2).astype(float)
     n_ctas = int((skew[:, 0, 1] > 0).sum())
     if n_ctas > 1:
         P = model.phase_count
-        acc = {}
+        acc, skipped = {}, {}
+        prev = 0   # the last phase the CTAs ran: a skipped phase is no one's predecessor
         for p in range(1, P):
-            end_prev, arr, end = skew[:n_ctas, p - 1, 1], skew[:n_ctas, p, 0], skew[:n_ctas, p, 1]
+            end_prev, arr, end = skew[:n_ctas, prev, 1], skew[:n_ctas, p, 0], skew[:n_ctas, p, 1]
+            k = kind_of(p)
+            if (end <= 0).all():
+                skipped[k] = skipped.get(k, 0) + 1
+                continue
+            prev = p
             if (end_prev <= 0).any() or (end <= 0).any():
                 continue
-            k = kind_of(p)
             have = arr > 0
             a0 = acc.setdefault(k, [[], [], [], []])
             a0[0].append(end.max() - end_prev.max())                        # phase period: last end -> last end
@@ -184,8 +196,10 @@ def timing(args):
         print(f"skew trace of the last frame over {n_ctas} CTAs (ns): period (last end -> last end) | end spread (max - median) | "
               f"last end of the previous phase -> median input staged | median staged -> last end")
         for k, (per, sp, gap, chain) in acc.items():
-            print(f"  {k:12s} x{len(per):3d} period {np.mean(per):7.0f} | spread {np.mean(sp):6.0f} | hand-off "
+            print(f"  {k:20s} x{len(per):3d} period {np.mean(per):7.0f} | spread {np.mean(sp):6.0f} | hand-off "
                   f"{(np.mean(gap) if gap else float('nan')):6.0f} | chain {(np.mean(chain) if chain else float('nan')):6.0f}")
+        for k, n in skipped.items():
+            print(f"  {k:20s} x{n:3d} skipped")
 
 
 def teams(args):
@@ -233,6 +247,7 @@ def main():
     ap.add_argument("--staggers", default="0,250,350")
     ap.add_argument("--trace-stagger", type=int, default=0)
     ap.add_argument("--trace-fused", type=int, default=1, help="ll_fused_mlp of the cycle / skew trace")
+    ap.add_argument("--trace-split", type=int, default=1, help="ll_psum_split of the cycle / skew trace")
     ap.add_argument("--n-ctas", default="", help="comma list of grid sizes to time")
     ap.add_argument("--skip-check", action="store_true")
     ap.add_argument("--skip-timing", action="store_true")
