@@ -91,6 +91,24 @@ class SmolMimiWeights(C.Structure):
         ("conv_out", SmolMimiConv), ("rope", C.c_void_p)]
 
 
+class SmolMimiEncoderConfig(C.Structure):
+    _fields_ = [(n, C.c_int32) for n in (
+        "n_q", "codebook_size", "codebook_dim", "dim", "n_layers", "n_heads", "head_dim", "ffn", "n_filters", "n_ratios")] + [
+        ("ratios", C.c_int32 * SMOL_MIMI_MAX_RATIOS)] + [(n, C.c_int32) for n in (
+            "kernel", "res_kernel", "last_kernel", "max_clips", "max_samples", "window")] + [
+        ("norm_eps", C.c_float), ("codebook_eps", C.c_float)]
+
+
+class SmolMimiEncoderWeights(C.Structure):
+    _fields_ = [
+        ("embed_sum", C.c_void_p * SMOL_MIMI_MAX_Q), ("cluster_usage", C.c_void_p * SMOL_MIMI_MAX_Q),
+        ("semantic_input_proj", C.c_void_p), ("acoustic_input_proj", C.c_void_p), ("downsample", C.c_void_p),
+        ("layers", SmolMimiLayerWeights * SMOL_MIMI_MAX_LAYERS),
+        ("conv_in", SmolMimiConv), ("res_conv1", SmolMimiConv * SMOL_MIMI_MAX_RATIOS),
+        ("res_conv2", SmolMimiConv * SMOL_MIMI_MAX_RATIOS), ("conv_down", SmolMimiConv * SMOL_MIMI_MAX_RATIOS),
+        ("conv_out", SmolMimiConv), ("rope", C.c_void_p)]
+
+
 # name -> (restype, argtypes); every symbol the headers declare
 PROTOTYPES = {
     "smol_abi_version": (C.c_int, []),
@@ -133,6 +151,14 @@ PROTOTYPES = {
     "smol_mimi_debug_buffer": (C.c_void_p, [C.c_void_p, C.c_char_p, C.POINTER(C.c_int64)]),
     "smol_mimi_launches_per_step": (C.c_int32, [C.c_void_p]),
     "smol_mimi_error_word": (C.c_void_p, [C.c_void_p]),
+    "smol_mimi_encoder_create": (C.c_int, [C.POINTER(SmolMimiEncoderConfig), C.POINTER(C.c_void_p)]),
+    "smol_mimi_encoder_destroy": (None, [C.c_void_p]),
+    "smol_mimi_encoder_samples_per_frame": (C.c_int32, [C.c_void_p]),
+    "smol_mimi_encoder_workspace_bytes": (C.c_size_t, [C.c_void_p]),
+    "smol_mimi_encoder_bind": (C.c_int, [C.c_void_p, C.POINTER(SmolMimiEncoderWeights), C.c_void_p, C.c_size_t, C.c_void_p]),
+    "smol_mimi_encode": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(C.c_int64), C.c_int32, C.c_void_p, C.c_void_p]),
+    "smol_mimi_encoder_debug_buffer": (C.c_void_p, [C.c_void_p, C.c_char_p]),
+    "smol_mimi_encoder_launches": (C.c_int32, [C.c_void_p]),
 }
 
 _lib = None

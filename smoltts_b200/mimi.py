@@ -11,8 +11,10 @@ Same names and argument meaning here; what differs is what an engine for many co
 * all compute is CUDA (``csrc/mimi_kernels.cu`` behind ``include/smoltts_b200_mimi.h``); there is no CPU path -- the
   constructor raises without a CUDA device.
 
-Checkpoint layout: kyutai/mimi's ``model.safetensors`` keys and torch layouts (what ``load_mimi`` reads); only the decode
-half is used (``quantizer.*``, ``upsample``, ``decoder_transformer``, ``decoder``).
+Checkpoint layout: kyutai/mimi's ``model.safetensors`` keys and torch layouts (what ``load_mimi`` reads).  The decode half
+(``quantizer.*``, ``upsample``, ``decoder_transformer``, ``decoder``) is always bound; the encode half (``encoder``,
+``encoder_transformer``, ``downsample``, the quantizers' ``input_proj``) only with ``encode_max_samples > 0``, for
+``encode`` (audio -> codes, ``csrc/mimi_encoder.cu``, pinned to transformers' ``MimiModel.encode``).
 """
 from __future__ import annotations
 
@@ -92,10 +94,15 @@ class MimiModel:
     """The decode half of the reference's ``MimiModel`` on one CUDA device."""
 
     def __init__(self, config: Optional[MimiConfig] = None, num_codebooks: int = 8, max_streams: int = 1, max_frames: int = 2048,
-                 window: int = 0, upsample_carry: bool = False, mode: str = "graph", device: Union[str, torch.device, None] = None):
+                 window: int = 0, upsample_carry: bool = False, mode: str = "graph", device: Union[str, torch.device, None] = None,
+                 encode_max_samples: int = 0, encode_max_clips: int = 1):
         """mode: "graph" -- a step's 57 launches are captured once per (batch, buffers) and replayed as one CUDA graph (the
         default); "eager" -- plain launches with programmatic dependent launch (also what a caller's own graph capture
-        records).  Both compute the same bits."""
+        records).  Both compute the same bits.
+
+        encode_max_samples > 0 builds the encoder too (``encode``) for up to ``encode_max_clips`` clips and
+        ``encode_max_samples`` samples in all per call; its workspace grows with ``encode_max_samples`` (about 660 bytes per
+        sample).  At 0 nothing of the encoder is allocated or bound."""
         if not torch.cuda.is_available():
             raise RuntimeError("smoltts_b200.MimiModel needs a CUDA device (there is no CPU path)")
         self.config = config or MimiConfig()
@@ -135,18 +142,36 @@ class MimiModel:
         self._frames = [0] * max_streams
         self._io: Dict[int, tuple] = {}   # batch -> (codes, slots, pcm) device buffers with stable addresses (graph replay)
         self._io_slots: Dict[int, tuple] = {}
+        self.encode_max_samples, self.encode_max_clips = int(encode_max_samples), int(encode_max_clips)
+        self._enc = None
+        self._enc_ws: Optional[torch.Tensor] = None
+        if self.encode_max_samples > 0:
+            ec = _capi.SmolMimiEncoderConfig()
+            for name in ("n_q", "codebook_size", "codebook_dim", "dim", "n_layers", "n_heads", "head_dim", "ffn", "n_filters", "n_ratios",
+                         "kernel", "res_kernel", "last_kernel", "norm_eps", "codebook_eps"):
+                setattr(ec, name, getattr(cfg, name))
+            for i, r in enumerate(c.seanet.ratios):
+                ec.ratios[i] = r
+            ec.max_clips, ec.max_samples, ec.window = self.encode_max_clips, self.encode_max_samples, c.transformer.context
+            he = C.c_void_p()
+            _capi.check(self._lib.smol_mimi_encoder_create(C.byref(ec), C.byref(he)))
+            self._enc = he
 
     def __del__(self):
         try:
             if getattr(self, "_h", None):
                 self._lib.smol_mimi_destroy(self._h)
                 self._h = None
+            if getattr(self, "_enc", None):
+                self._lib.smol_mimi_encoder_destroy(self._enc)
+                self._enc = None
         except Exception:
             pass
 
     # ---- weights ------------------------------------------------------------------------------------------------------
     def load_state_dict(self, sd: Dict[str, torch.Tensor]) -> None:
-        """kyutai/mimi keys (the encoder half, `input_proj`, `initialized` buffers and unused codebooks are ignored)."""
+        """kyutai/mimi keys (`initialized` buffers and unused codebooks are ignored, and so are the encoder half and
+        `input_proj` unless the encoder was built)."""
         c, n_q = self.config, self.num_codebooks
         dev = self.device
         keep: List[torch.Tensor] = []
@@ -208,6 +233,110 @@ class MimiModel:
             torch.cuda.current_stream().synchronize()   # the source tensors in `keep` may go now: everything was repacked
         self._free = list(range(self.max_streams - 1, -1, -1))
         self._frames = [0] * self.max_streams
+        if self._enc is not None:
+            self._bind_encoder(sd)
+
+    def _bind_encoder(self, sd: Dict[str, torch.Tensor]) -> None:
+        c, n_q, dev = self.config, self.num_codebooks, self.device
+        keep: List[torch.Tensor] = []
+
+        def t(key: str, shape: Sequence[int]) -> int:
+            if key not in sd:
+                raise KeyError(f"MimiModel.load_state_dict: missing encoder key {key}")
+            v = sd[key]
+            if tuple(v.shape) != tuple(shape):
+                raise ValueError(f"MimiModel.load_state_dict: {key} has shape {tuple(v.shape)}, expected {tuple(shape)}")
+            v = v.detach().to(device=dev, dtype=torch.float32).contiguous()
+            keep.append(v)
+            return v.data_ptr()
+
+        w = _capi.SmolMimiEncoderWeights()
+        D, cd, cs = c.transformer.d_model, c.rvq.codebook_dim, c.rvq.codebook_size
+        for i in range(n_q):
+            p = ("quantizer.semantic_residual_vector_quantizer.layers.0" if i == 0
+                 else f"quantizer.acoustic_residual_vector_quantizer.layers.{i - 1}")
+            w.embed_sum[i] = t(p + ".codebook.embed_sum", (cs, cd))
+            w.cluster_usage[i] = t(p + ".codebook.cluster_usage", (cs,))
+        w.semantic_input_proj = t("quantizer.semantic_residual_vector_quantizer.input_proj.weight", (cd, D, 1))
+        w.acoustic_input_proj = t("quantizer.acoustic_residual_vector_quantizer.input_proj.weight", (cd, D, 1))
+        w.downsample = t("downsample.conv.weight", (D, D, 4))
+        F = c.transformer.dim_feedforward
+        for l in range(c.transformer.num_layers):
+            p = f"encoder_transformer.layers.{l}."
+            L = w.layers[l]
+            L.q_proj, L.k_proj = t(p + "self_attn.q_proj.weight", (D, D)), t(p + "self_attn.k_proj.weight", (D, D))
+            L.v_proj, L.o_proj = t(p + "self_attn.v_proj.weight", (D, D)), t(p + "self_attn.o_proj.weight", (D, D))
+            L.fc1, L.fc2 = t(p + "mlp.fc1.weight", (F, D)), t(p + "mlp.fc2.weight", (D, F))
+            L.ln1_w, L.ln1_b = t(p + "input_layernorm.weight", (D,)), t(p + "input_layernorm.bias", (D,))
+            L.ln2_w, L.ln2_b = t(p + "post_attention_layernorm.weight", (D,)), t(p + "post_attention_layernorm.bias", (D,))
+            L.scale_attn, L.scale_mlp = t(p + "self_attn_layer_scale.scale", (D,)), t(p + "mlp_layer_scale.scale", (D,))
+        s = c.seanet
+        ch = s.n_filters
+        w.conv_in.weight, w.conv_in.bias = t("encoder.layers.0.conv.weight", (ch, 1, s.kernel_size)), t("encoder.layers.0.conv.bias", (ch,))
+        idx = 1
+        for i, r in enumerate(reversed(s.ratios)):
+            w.res_conv1[i].weight = t(f"encoder.layers.{idx}.block.1.conv.weight", (ch // 2, ch, s.residual_kernel_size))
+            w.res_conv1[i].bias = t(f"encoder.layers.{idx}.block.1.conv.bias", (ch // 2,))
+            w.res_conv2[i].weight = t(f"encoder.layers.{idx}.block.3.conv.weight", (ch, ch // 2, 1))
+            w.res_conv2[i].bias = t(f"encoder.layers.{idx}.block.3.conv.bias", (ch,))
+            w.conv_down[i].weight = t(f"encoder.layers.{idx + 2}.conv.weight", (2 * ch, ch, 2 * r))
+            w.conv_down[i].bias = t(f"encoder.layers.{idx + 2}.conv.bias", (2 * ch,))
+            ch, idx = 2 * ch, idx + 3
+        w.conv_out.weight = t(f"encoder.layers.{idx + 1}.conv.weight", (D, ch, s.last_kernel_size))
+        w.conv_out.bias = t(f"encoder.layers.{idx + 1}.conv.bias", (D,))
+        hop = math.prod(s.ratios)
+        rope = mimi_rope_table(c.transformer.head_dim, c.transformer.rope_theta, -(-self.encode_max_samples // hop)).to(dev)
+        keep.append(rope)
+        w.rope = rope.data_ptr()
+        n = int(self._lib.smol_mimi_encoder_workspace_bytes(self._enc))
+        self._enc_ws = torch.empty(n + 256, dtype=torch.uint8, device=dev)
+        base = (self._enc_ws.data_ptr() + 255) // 256 * 256
+        with torch.cuda.device(dev):
+            stream = torch.cuda.current_stream().cuda_stream
+            _capi.check(self._lib.smol_mimi_encoder_bind(self._enc, C.byref(w), C.c_void_p(base), C.c_size_t(n), C.c_void_p(stream)))
+            torch.cuda.current_stream().synchronize()
+
+    # ---- encode (audio -> codes) --------------------------------------------------------------------------------------
+    def encode(self, x: Union[torch.Tensor, Sequence[torch.Tensor]]) -> Union[torch.Tensor, List[torch.Tensor]]:
+        """24 kHz mono fp32 PCM -> Mimi codes, as transformers' ``MimiModel.encode``: ``[B, 1, L]`` -> int64
+        ``[B, n_q, ceil(L / 1920)]``, or a list of 1-D clips of any lengths -> a list of int64 ``[n_q, T_b]``.  Every clip is
+        encoded exactly as it would be alone, in one call for all of them.  Asynchronous on the current CUDA stream."""
+        if self._enc is None:
+            raise RuntimeError("MimiModel.encode: this codec was built without an encoder (pass encode_max_samples > 0)")
+        if self._enc_ws is None:
+            raise RuntimeError("MimiModel: load_state_dict() first")
+        batched = isinstance(x, torch.Tensor)
+        if batched:
+            if x.dim() != 3 or x.shape[1] != 1:
+                raise ValueError(f"MimiModel.encode: expected [B, 1, L] mono audio, got {tuple(x.shape)}")
+            clips = [x[b, 0] for b in range(x.shape[0])]
+        else:
+            clips = [torch.as_tensor(c) for c in x]
+            if any(c.dim() != 1 for c in clips):
+                raise ValueError("MimiModel.encode: every clip of a list must be 1-D mono audio")
+        if not clips:
+            return torch.zeros(0, self.num_codebooks, 0, dtype=torch.int64, device=self.device) if batched else []
+        lens = [int(c.shape[0]) for c in clips]
+        pcm = torch.cat([c.to(device=self.device, dtype=torch.float32) for c in clips]).contiguous()
+        spf = self.samples_per_frame
+        frames = [-(-n // spf) for n in lens]
+        codes = torch.empty(sum(frames), self.num_codebooks, dtype=torch.int32, device=self.device)
+        h_lens = (C.c_int64 * len(lens))(*lens)
+        _capi.check(self._lib.smol_mimi_encode(self._enc, C.c_void_p(pcm.data_ptr()), h_lens, len(lens), C.c_void_p(codes.data_ptr()),
+                                               C.c_void_p(self._stream())))
+        self._enc_frames = sum(frames)
+        per_clip = [c.t().to(torch.int64) for c in torch.split(codes, frames)]
+        return torch.stack(per_clip) if batched else per_clip
+
+    def encoder_latent(self) -> torch.Tensor:
+        """Test hook: the pre-quantizer latent z of the last ``encode`` call, ``[sum_b T_b, dim]`` (clips back to back)."""
+        p = self._lib.smol_mimi_encoder_debug_buffer(self._enc, b"latent")
+        base = (self._enc_ws.data_ptr() + 255) // 256 * 256
+        n = int(self._lib.smol_mimi_encoder_workspace_bytes(self._enc))
+        flat = self._enc_ws[base - self._enc_ws.data_ptr(): base - self._enc_ws.data_ptr() + n].view(torch.float32)
+        off = (p - base) // 4
+        D = self.config.transformer.d_model
+        return flat[off: off + self._enc_frames * D].view(self._enc_frames, D).clone()
 
     @classmethod
     def from_safetensors(cls, path: str, **kw) -> "MimiModel":
@@ -335,9 +464,10 @@ class MimiModel:
         return bool(self._flat(torch.int32)[(p - self._base()) // 4].item())
 
 
-def load_mimi(path: str, format: str = "fp32", **kw) -> MimiModel:
+def load_mimi(path: str, format: str = "fp32", encode_max_samples: int = 0, encode_max_clips: int = 1, **kw) -> MimiModel:
     """codec/mimi.py:107 -- from a local model.safetensors (there is no hub access here).  Only fp32 is built: it is the
-    reference's default and what its callers use (`load_mimi()` in __init__.py:54)."""
+    reference's default and what its callers use (`load_mimi()` in __init__.py:54).  ``encode_max_samples > 0`` also
+    builds the encoder (``MimiModel.encode``) for that many samples per call."""
     if format != "fp32":
         raise ValueError("load_mimi: only format='fp32' is built")
-    return MimiModel.from_safetensors(path, **kw)
+    return MimiModel.from_safetensors(path, encode_max_samples=encode_max_samples, encode_max_clips=encode_max_clips, **kw)

@@ -163,10 +163,11 @@ def teacher_grid(cfg: RQTransformerModelArgs, n_text: int, n_audio: int, batch: 
 # ---- Mimi decoder (SURVEY §8(f)-2): seeded weights under kyutai/mimi's state-dict keys ----------------------------------
 def mimi_state_dict_shapes(n_q: int = 8, codebook_size: int = 2048, codebook_dim: int = 256, dim: int = 512, n_layers: int = 8,
                            ffn: int = 2048, n_filters: int = 64, ratios=(8, 6, 5, 4), kernel: int = 7, res_kernel: int = 3,
-                           last_kernel: int = 3) -> Dict[str, tuple]:
+                           last_kernel: int = 3, encoder: bool = False) -> Dict[str, tuple]:
     """Key -> shape of the decode half of kyutai/mimi's model.safetensors (the keys the reference's load_mimi() maps onto
     its module tree, mlx_inference/src/smoltts_mlx/codec/mimi.py:107-156; torch layouts: Conv1d [out, in, k],
-    ConvTranspose1d [in, out, k])."""
+    ConvTranspose1d [in, out, k]).  ``encoder=True`` appends the encode half (``encoder.*``, ``encoder_transformer.*``,
+    ``downsample`` and the quantizers' ``input_proj``) after those keys."""
     s: Dict[str, tuple] = {}
     for half, n in (("semantic", 1), ("acoustic", n_q - 1)):
         p = f"quantizer.{half}_residual_vector_quantizer"
@@ -201,12 +202,58 @@ def mimi_state_dict_shapes(n_q: int = 8, codebook_size: int = 2048, codebook_dim
         idx += 3
     s[f"decoder.layers.{idx + 1}.conv.weight"] = (1, ch, last_kernel)
     s[f"decoder.layers.{idx + 1}.conv.bias"] = (1,)
+    if encoder:
+        # SEANet encoder: conv k7, then per ratio (reversed) [residual block, ELU, conv k = 2 r, stride r], ELU, conv k3
+        s["encoder.layers.0.conv.weight"] = (n_filters, 1, kernel)
+        s["encoder.layers.0.conv.bias"] = (n_filters,)
+        ch, idx = n_filters, 1
+        for r in reversed(ratios):
+            s[f"encoder.layers.{idx}.block.1.conv.weight"] = (ch // 2, ch, res_kernel)
+            s[f"encoder.layers.{idx}.block.1.conv.bias"] = (ch // 2,)
+            s[f"encoder.layers.{idx}.block.3.conv.weight"] = (ch, ch // 2, 1)
+            s[f"encoder.layers.{idx}.block.3.conv.bias"] = (ch,)
+            s[f"encoder.layers.{idx + 2}.conv.weight"] = (2 * ch, ch, 2 * r)
+            s[f"encoder.layers.{idx + 2}.conv.bias"] = (2 * ch,)
+            ch, idx = 2 * ch, idx + 3
+        s[f"encoder.layers.{idx + 1}.conv.weight"] = (dim, ch, last_kernel)
+        s[f"encoder.layers.{idx + 1}.conv.bias"] = (dim,)
+        for l in range(n_layers):
+            p = f"encoder_transformer.layers.{l}"
+            for w in ("q_proj", "k_proj", "v_proj", "o_proj"):
+                s[f"{p}.self_attn.{w}.weight"] = (dim, dim)
+            s[f"{p}.mlp.fc1.weight"] = (ffn, dim)
+            s[f"{p}.mlp.fc2.weight"] = (dim, ffn)
+            for nm in ("input_layernorm", "post_attention_layernorm"):
+                s[f"{p}.{nm}.weight"] = (dim,)
+                s[f"{p}.{nm}.bias"] = (dim,)
+            s[f"{p}.self_attn_layer_scale.scale"] = (dim,)
+            s[f"{p}.mlp_layer_scale.scale"] = (dim,)
+        s["downsample.conv.weight"] = (dim, dim, 4)
+        for half in ("semantic", "acoustic"):
+            s[f"quantizer.{half}_residual_vector_quantizer.input_proj.weight"] = (codebook_dim, dim, 1)
     return s
 
 
+def make_test_audio(seed: int, n_samples: int, sampling_rate: int = 24_000) -> torch.Tensor:
+    """Seeded 1-D fp32 test clip: three sines (seeded frequencies 80 .. 2000 Hz, amplitudes 0.1 .. 0.3) plus seeded Gaussian
+    noise of std 0.05.  Computed in float64 with numpy's PCG64 and rounded once to fp32, so every machine regenerates the
+    same samples."""
+    import numpy as np
+
+    rng = np.random.default_rng(seed)
+    freq = rng.uniform(80.0, 2000.0, 3)
+    amp = rng.uniform(0.1, 0.3, 3)
+    phase = rng.uniform(0.0, 2 * np.pi, 3)
+    t = np.arange(n_samples, dtype=np.float64) / sampling_rate
+    x = (amp[:, None] * np.sin(2 * np.pi * freq[:, None] * t[None, :] + phase[:, None])).sum(0)
+    x = x + 0.05 * rng.standard_normal(n_samples)
+    return torch.from_numpy(x.astype(np.float32))
+
+
 def make_mimi_state_dict(seed: int = 0, **dims) -> Dict[str, torch.Tensor]:
-    """Seeded fp32 weights of the Mimi decoder.  Scales keep every stage O(1) (fan-in scaled weights, layer scales of
-    0.1 .. 0.3 instead of the trained 0.01 .. so that all eight transformer layers matter in a parity check)."""
+    """Seeded fp32 weights of the Mimi decoder (and with ``encoder=True`` of the encoder too).  Scales keep every stage O(1)
+    (fan-in scaled weights, layer scales of 0.1 .. 0.3 instead of the trained 0.01 .. so that all eight transformer layers
+    matter in a parity check).  Every key is seeded by its name: the encoder keys leave the decoder's values unchanged."""
     out: Dict[str, torch.Tensor] = {}
     for name, shape in mimi_state_dict_shapes(**dims).items():
         g = torch.Generator(device="cpu")

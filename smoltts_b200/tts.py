@@ -43,6 +43,22 @@ class SmolTTS:
         return self.prompt_encoder.tts_prompt(input, speaker=voice_id, sysprompt=sysprompt)[None]
 
     def create_speaker(self, samples: Sequence[dict], system_prompt: Optional[str] = None) -> torch.Tensor:
+        """Voice-clone prefix (__init__.py:97-118) from ``{"text", "audio"}`` samples -- 1-D float PCM at 24 kHz, mono -- or
+        ``{"text", "codes"}`` samples with ready-made Mimi codes.  The audio of all samples is encoded in one
+        ``MimiModel.encode`` call (the codec must have been built with ``encode_max_samples > 0``)."""
+        samples = list(samples)
+        with_audio = [i for i, s in enumerate(samples) if "audio" in s and "codes" not in s]
+        if with_audio:
+            codec = next((c for c in (self.codec, self.codec_full) if c._enc is not None), None)
+            if codec is None:
+                raise ValueError("create_speaker: samples carry 'audio' but the codec has no encoder "
+                                 "(build the MimiModel with encode_max_samples > 0, or pass 'codes')")
+            clips = [torch.as_tensor(samples[i]["audio"], dtype=torch.float32).reshape(-1) for i in with_audio]
+            codes = codec.encode(clips)
+            samples = [dict(s) for s in samples]
+            for i, c in zip(with_audio, codes):
+                samples[i].pop("audio")
+                samples[i]["codes"] = c.cpu()
         return self.prompt_encoder.create_speaker(samples, system_prompt)
 
     # ---- one utterance (:64-83) ----
