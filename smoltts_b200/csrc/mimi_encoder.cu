@@ -34,21 +34,14 @@
 
 #include "../../include/smoltts_b200.h"
 #include "../../include/smoltts_b200_mimi.h"
+#include "mimi_common.cuh"
 
 namespace smol {
-int capi_fail(int code, const std::string& msg);
-int capi_cuda_fail(cudaError_t e, const char* what);
-
 namespace mimi_enc {
+using namespace smol::mimi;
 
-constexpr int kThreads = 256;
-constexpr int kWarps = kThreads / 32;
 constexpr int kMaxClips = 256;
 constexpr int kMaxWindow = 1024;
-constexpr int kTM = 64, kTN = 64, kTK = 16;
-
-enum { PRO_NONE = 0, PRO_ELU = 1 };
-enum { EPI_BIAS = 0, EPI_RES = 1, EPI_SCALE_RES = 2, EPI_GELU = 3 };
 
 // Row offsets of the clips of one call at one level: clip b owns output rows out_off[b] .. out_off[b + 1] and reads input
 // rows in_off[b] .. in_off[b + 1].  n = 0: one sequence (a Linear: output row = input row).
@@ -67,107 +60,53 @@ __device__ __forceinline__ int seg_find(const Segs& s, int row) {   // the clip 
     return lo;
 }
 
-__device__ __forceinline__ float warp_sum(float v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-__device__ __forceinline__ float elu1(float x) { return x > 0.f ? x : expm1f(x); }
-__device__ __forceinline__ float gelu_erf(float x) { return 0.5f * x * (1.0f + erff(x * 0.70710678118654752440f)); }
-
-// out[row][n] = epilogue( sum_k A(row, k) W[n][k] ), A(row, tap j * cin + c) = prologue( in[clip row t stride - pad + j][c] )
+// out[row][n] = epilogue( sum_k A(row, k) W[n][k] ), A(row, tap j * cin + c) = prologue( in[clip row t stride - pad + j][c] ):
+// the rows of tile_kernel<EncOp>.  A source row outside its clip reads 0, or with `replicate` the clip's edge row.
 struct EncOp {
     const float* in; int cin, stride, pad, replicate, pro;
     const float* W; const float* bias; int N, K;
     float* out; int epi; const float* res; const float* scale;
     int rows;
     Segs seg;
-};
 
-// 64 x 64 output tile per CTA, K in steps of 16 through shared memory, 4 x 4 outputs per thread, each a sequential FMA chain
-// over k = 0 .. K-1 (the decoder's tile_kernel arithmetic, with the ragged row map and the padding rules of the encoder).
-__global__ void __launch_bounds__(kThreads, 2) enc_tile_kernel(const EncOp op) {
-    __shared__ __align__(16) float As[kTK][kTM + 4];
-    __shared__ __align__(16) float Ws[kTK][kTN + 4];
-    const int tid = threadIdx.x;
-    const int row0 = blockIdx.x * kTM, n0 = blockIdx.y * kTN;   // (rows on x: up to millions of tiles)
-    const int lm = tid >> 2, lk = (tid & 3) << 2;
-    // the A row this thread loads: clip base row, first tap's source row, clip length
-    const int arow = row0 + lm;
-    const bool a_ok = arow < op.rows;
-    long long a_base = 0;
-    int a_t0 = 0, a_tin = 1;
-    if (a_ok) {
-        if (op.seg.n == 0) { a_t0 = arow * op.stride - op.pad; a_tin = op.rows; }
-        else {
-            const int b = seg_find(op.seg, arow);
-            a_base = op.seg.in_off[b];
-            a_t0 = (arow - op.seg.out_off[b]) * op.stride - op.pad;
-            a_tin = op.seg.in_off[b + 1] - op.seg.in_off[b];
+    struct Rows {};                                     // (a row's clip is found per thread: no shared row table)
+    __device__ void map_rows(Rows&, int) const {}
+    struct ARow { long long base; int t0, tin; bool ok; };   // clip base row, first tap's source row, clip length
+    __device__ ARow a_row(const Rows&, int row0, int m) const {
+        const int arow = row0 + m;
+        ARow a{0, 0, 1, arow < rows};
+        if (a.ok) {
+            if (seg.n == 0) { a.t0 = arow * stride - pad; a.tin = rows; }
+            else {
+                const int b = seg_find(seg, arow);
+                a.base = seg.in_off[b];
+                a.t0 = (arow - seg.out_off[b]) * stride - pad;
+                a.tin = seg.in_off[b + 1] - seg.in_off[b];
+            }
         }
+        return a;
     }
-    const bool w_ok = n0 + lm < op.N;
-    const float* w_base = op.W + (long long)(n0 + lm) * op.K;
-    auto load_a = [&](int k) -> float4 {
+    __device__ float4 load_a(const ARow& a, int k) const {
         float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (a_ok) {
-            const int j = k / op.cin, c = k - j * op.cin;
-            int sr = a_t0 + j;
-            if (op.replicate) sr = min(max(sr, 0), a_tin - 1);
-            if (sr >= 0 && sr < a_tin) {
-                v = *reinterpret_cast<const float4*>(op.in + (a_base + sr) * op.cin + c);
-                if (op.pro == PRO_ELU) { v.x = elu1(v.x); v.y = elu1(v.y); v.z = elu1(v.z); v.w = elu1(v.w); }
+        if (a.ok) {
+            const int j = k / cin, c = k - j * cin;
+            int sr = a.t0 + j;
+            if (replicate) sr = min(max(sr, 0), a.tin - 1);
+            if (sr >= 0 && sr < a.tin) {
+                v = *reinterpret_cast<const float4*>(in + (a.base + sr) * cin + c);
+                if (pro == PRO_ELU) v = elu4(v);
             }
         }
         return v;
-    };
-    auto load_w = [&](int k) -> float4 {
-        return w_ok ? __ldg(reinterpret_cast<const float4*>(w_base + k)) : make_float4(0.f, 0.f, 0.f, 0.f);
-    };
-    const int ty = tid >> 4, tx = tid & 15;
-    float acc[4][4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
-    float4 ra = load_a(lk), rw = load_w(lk);
-    for (int k0 = 0; k0 < op.K; k0 += kTK) {
-        As[lk + 0][lm] = ra.x; As[lk + 1][lm] = ra.y; As[lk + 2][lm] = ra.z; As[lk + 3][lm] = ra.w;
-        Ws[lk + 0][lm] = rw.x; Ws[lk + 1][lm] = rw.y; Ws[lk + 2][lm] = rw.z; Ws[lk + 3][lm] = rw.w;
-        __syncthreads();
-        if (k0 + kTK < op.K) { ra = load_a(k0 + kTK + lk); rw = load_w(k0 + kTK + lk); }
-#pragma unroll
-        for (int k = 0; k < kTK; ++k) {
-            const float4 a = *reinterpret_cast<const float4*>(&As[k][ty * 4]);
-            const float4 w = *reinterpret_cast<const float4*>(&Ws[k][tx * 4]);
-            acc[0][0] = fmaf(a.x, w.x, acc[0][0]); acc[0][1] = fmaf(a.x, w.y, acc[0][1]); acc[0][2] = fmaf(a.x, w.z, acc[0][2]); acc[0][3] = fmaf(a.x, w.w, acc[0][3]);
-            acc[1][0] = fmaf(a.y, w.x, acc[1][0]); acc[1][1] = fmaf(a.y, w.y, acc[1][1]); acc[1][2] = fmaf(a.y, w.z, acc[1][2]); acc[1][3] = fmaf(a.y, w.w, acc[1][3]);
-            acc[2][0] = fmaf(a.z, w.x, acc[2][0]); acc[2][1] = fmaf(a.z, w.y, acc[2][1]); acc[2][2] = fmaf(a.z, w.z, acc[2][2]); acc[2][3] = fmaf(a.z, w.w, acc[2][3]);
-            acc[3][0] = fmaf(a.w, w.x, acc[3][0]); acc[3][1] = fmaf(a.w, w.y, acc[3][1]); acc[3][2] = fmaf(a.w, w.z, acc[3][2]); acc[3][3] = fmaf(a.w, w.w, acc[3][3]);
-        }
-        __syncthreads();
     }
-    const int n = n0 + tx * 4;
-    if (n >= op.N) return;                      // (N is a multiple of 4)
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        const int m = row0 + ty * 4 + i;
-        if (m >= op.rows) continue;
-        const long long e = (long long)m * op.N + n;
-        float4 y = make_float4(acc[i][0], acc[i][1], acc[i][2], acc[i][3]);
-        if (op.bias) { y.x += op.bias[n]; y.y += op.bias[n + 1]; y.z += op.bias[n + 2]; y.w += op.bias[n + 3]; }
-        if (op.epi == EPI_RES) {
-            const float4 r = *reinterpret_cast<const float4*>(op.res + e);
-            y.x = r.x + y.x; y.y = r.y + y.y; y.z = r.z + y.z; y.w = r.w + y.w;
-        } else if (op.epi == EPI_SCALE_RES) {
-            const float4 r = *reinterpret_cast<const float4*>(op.res + e);
-            y.x = r.x + y.x * op.scale[n]; y.y = r.y + y.y * op.scale[n + 1]; y.z = r.z + y.z * op.scale[n + 2]; y.w = r.w + y.w * op.scale[n + 3];
-        } else if (op.epi == EPI_GELU) {
-            y.x = gelu_erf(y.x); y.y = gelu_erf(y.y); y.z = gelu_erf(y.z); y.w = gelu_erf(y.w);
-        }
-        *reinterpret_cast<float4*>(op.out + e) = y;
+    __device__ bool out_row(const Rows&, int row0, int m, long long& oe, long long& re) const {
+        const int row = row0 + m;
+        if (row >= rows) return false;
+        oe = re = (long long)row * N;
+        return true;
     }
-}
+    __device__ int bias_col(int n) const { return n; }
+};
 
 // The one-channel first convolution (K = kernel does not fit the tiles): one thread per (sample row, output channel).
 __global__ void __launch_bounds__(kThreads) enc_conv_in_kernel(const float* __restrict__ pcm, const float* __restrict__ w,
@@ -297,11 +236,7 @@ __global__ void __launch_bounds__(kThreads) enc_argmin_kernel(const float* __res
     for (int c = lane; c < cd; c += 32) r[c] = r[c] - e[c];
 }
 
-// ---- bind-time packing ------------------------------------------------------------------------------------------------
-__global__ void enc_pack_codebook_kernel(float* dst, const float* es, const float* cu, int rows, int dim, float eps) {
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < (long long)rows * dim; i += (long long)gridDim.x * blockDim.x)
-        dst[i] = es[i] / fmaxf(cu[i / dim], eps);
-}
+// ---- bind-time packing (codebooks and Conv1d: mimi_common.cuh) ------------------------------------------------------
 // |e_j|^2 of the packed rows, a sequential sum per row
 __global__ void enc_row_norm_kernel(float* dst, const float* rows_, int rows, int dim) {
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
@@ -311,15 +246,6 @@ __global__ void enc_row_norm_kernel(float* dst, const float* rows_, int rows, in
     for (int c = 0; c < dim; ++c) s = fmaf(r[c], r[c], s);
     dst[j] = s;
 }
-// Conv1d [Co][Ci][k] -> [Co][j * Ci + ci]
-__global__ void enc_pack_conv_kernel(float* dst, const float* w, int Co, int Ci, int k) {
-    const long long total = (long long)Co * Ci * k;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
-        const int ci = (int)(i % Ci); const long long r = i / Ci; const int j = (int)(r % k); const int co = (int)(r / k);
-        dst[i] = w[((long long)co * Ci + ci) * k + j];
-    }
-}
-
 }  // namespace mimi_enc
 }  // namespace smol
 
@@ -335,15 +261,13 @@ struct SmolMimiEncoder {
     long long cap_frames = 0, max_pos = 0;
     // workspace layout (bytes)
     size_t o_conv_in = 0, o_r1[SMOL_MIMI_MAX_RATIOS], o_r2[SMOL_MIMI_MAX_RATIOS], o_dn[SMOL_MIMI_MAX_RATIOS], o_conv_out = 0, o_bias = 0;
-    size_t o_qkv[SMOL_MIMI_MAX_LAYERS], o_o[SMOL_MIMI_MAX_LAYERS], o_fc1[SMOL_MIMI_MAX_LAYERS], o_fc2[SMOL_MIMI_MAX_LAYERS], o_vec[SMOL_MIMI_MAX_LAYERS];
+    LayerOffsets o_layer[SMOL_MIMI_MAX_LAYERS];
     size_t o_ds = 0, o_proj = 0, o_books = 0, o_norms = 0, o_rope = 0;
     size_t o_P = 0, o_Q = 0, o_H = 0, o_X = 0, o_Hn = 0, o_QKV = 0, o_ATT = 0, o_FF = 0, o_Z = 0, o_RS = 0, o_RA = 0, o_S = 0, total = 0;
     unsigned char* ws = nullptr;
     bool bound = false;
     int launches = 0;
 };
-
-static size_t enc_al(size_t v) { return (v + 255) / 256 * 256; }
 
 static void enc_plan(SmolMimiEncoder* e) {
     const SmolMimiEncoderConfig& c = e->cfg;
@@ -363,47 +287,40 @@ static void enc_plan(SmolMimiEncoder* e) {
     e->max_pos = (c.max_samples + div - 1) / div;
     e->cap_frames = c.max_samples / (2 * div) + c.max_clips;
     const long long R = e->cap_rows[c.n_ratios];
-    size_t o = 0;
-    auto take = [&](size_t floats) { const size_t r = o; o = enc_al(o + floats * 4); return r; };
-    e->o_conv_in = take((size_t)c.n_filters * c.kernel);
+    WsPlan p;
+    e->o_conv_in = p.take((size_t)c.n_filters * c.kernel);
     int ch = c.n_filters;
     size_t nb = c.n_filters;
     for (int i = 0; i < c.n_ratios; ++i) {
-        e->o_r1[i] = take((size_t)(ch / 2) * ch * c.res_kernel);
-        e->o_r2[i] = take((size_t)ch * (ch / 2));
-        e->o_dn[i] = take((size_t)2 * ch * ch * 2 * e->ratio[i]);
+        e->o_r1[i] = p.take((size_t)(ch / 2) * ch * c.res_kernel);
+        e->o_r2[i] = p.take((size_t)ch * (ch / 2));
+        e->o_dn[i] = p.take((size_t)2 * ch * ch * 2 * e->ratio[i]);
         nb += (size_t)ch / 2 + ch + 2 * ch;
         ch *= 2;
     }
-    e->o_conv_out = take((size_t)c.dim * ch * c.last_kernel);
+    e->o_conv_out = p.take((size_t)c.dim * ch * c.last_kernel);
     nb += c.dim;
-    e->o_bias = take(nb);
-    for (int l = 0; l < c.n_layers; ++l) {
-        e->o_qkv[l] = take((size_t)3 * c.dim * c.dim);
-        e->o_o[l] = take((size_t)c.dim * c.dim);
-        e->o_fc1[l] = take((size_t)c.ffn * c.dim);
-        e->o_fc2[l] = take((size_t)c.dim * c.ffn);
-        e->o_vec[l] = take((size_t)6 * c.dim);
-    }
-    e->o_ds = take((size_t)c.dim * c.dim * 4);
-    e->o_proj = take((size_t)2 * c.codebook_dim * c.dim);
-    e->o_books = take((size_t)c.n_q * c.codebook_size * c.codebook_dim);
-    e->o_norms = take((size_t)c.n_q * c.codebook_size);
-    e->o_rope = take((size_t)e->max_pos * c.head_dim);
+    e->o_bias = p.take(nb);
+    for (int l = 0; l < c.n_layers; ++l) e->o_layer[l] = plan_layer(p, c.dim, c.ffn);
+    e->o_ds = p.take((size_t)c.dim * c.dim * 4);
+    e->o_proj = p.take((size_t)2 * c.codebook_dim * c.dim);
+    e->o_books = p.take((size_t)c.n_q * c.codebook_size * c.codebook_dim);
+    e->o_norms = p.take((size_t)c.n_q * c.codebook_size);
+    e->o_rope = p.take((size_t)e->max_pos * c.head_dim);
     // activations: SEANet ping-pong (P, Q) and residual hidden rows (H); transformer rows; latent and RVQ
-    e->o_P = take(big);
-    e->o_Q = take(big);
-    e->o_H = take(half);
-    e->o_X = take((size_t)R * c.dim);
-    e->o_Hn = take((size_t)R * c.dim);
-    e->o_QKV = take((size_t)R * 3 * c.dim);
-    e->o_ATT = take((size_t)R * c.dim);
-    e->o_FF = take((size_t)R * c.ffn);
-    e->o_Z = take((size_t)e->cap_frames * c.dim);
-    e->o_RS = take((size_t)e->cap_frames * c.codebook_dim);
-    e->o_RA = take((size_t)e->cap_frames * c.codebook_dim);
-    e->o_S = take((size_t)e->cap_frames * c.codebook_size);
-    e->total = o;
+    e->o_P = p.take(big);
+    e->o_Q = p.take(big);
+    e->o_H = p.take(half);
+    e->o_X = p.take((size_t)R * c.dim);
+    e->o_Hn = p.take((size_t)R * c.dim);
+    e->o_QKV = p.take((size_t)R * 3 * c.dim);
+    e->o_ATT = p.take((size_t)R * c.dim);
+    e->o_FF = p.take((size_t)R * c.ffn);
+    e->o_Z = p.take((size_t)e->cap_frames * c.dim);
+    e->o_RS = p.take((size_t)e->cap_frames * c.codebook_dim);
+    e->o_RA = p.take((size_t)e->cap_frames * c.codebook_dim);
+    e->o_S = p.take((size_t)e->cap_frames * c.codebook_size);
+    e->total = p.total;
 }
 
 extern "C" int smol_mimi_encoder_create(const SmolMimiEncoderConfig* cfg, SmolMimiEncoder** out) {
@@ -435,8 +352,6 @@ extern "C" int32_t smol_mimi_encoder_samples_per_frame(const SmolMimiEncoder* e)
 extern "C" size_t smol_mimi_encoder_workspace_bytes(const SmolMimiEncoder* e) { return e ? e->total : 0; }
 extern "C" int32_t smol_mimi_encoder_launches(const SmolMimiEncoder* e) { return e ? e->launches : 0; }
 
-#define ECU(call) do { cudaError_t e__ = (call); if (e__ != cudaSuccess) return smol::capi_cuda_fail(e__, #call); } while (0)
-
 static float* ews(SmolMimiEncoder* e, size_t off) { return reinterpret_cast<float*>(e->ws + off); }
 
 extern "C" int smol_mimi_encoder_bind(SmolMimiEncoder* e, const SmolMimiEncoderWeights* w, void* d_workspace, size_t workspace_bytes,
@@ -449,11 +364,7 @@ extern "C" int smol_mimi_encoder_bind(SmolMimiEncoder* e, const SmolMimiEncoderW
     bool ok = w->semantic_input_proj && w->acoustic_input_proj && w->downsample && w->rope && w->conv_in.weight && w->conv_in.bias &&
               w->conv_out.weight && w->conv_out.bias;
     for (int i = 0; i < c.n_q; ++i) ok = ok && w->embed_sum[i] && w->cluster_usage[i];
-    for (int l = 0; l < c.n_layers; ++l) {
-        const SmolMimiLayerWeights& L = w->layers[l];
-        ok = ok && L.q_proj && L.k_proj && L.v_proj && L.o_proj && L.fc1 && L.fc2 && L.ln1_w && L.ln1_b && L.ln2_w && L.ln2_b &&
-             L.scale_attn && L.scale_mlp;
-    }
+    for (int l = 0; l < c.n_layers; ++l) ok = ok && layer_weights_ok(w->layers[l]);
     for (int i = 0; i < c.n_ratios; ++i)
         ok = ok && w->res_conv1[i].weight && w->res_conv1[i].bias && w->res_conv2[i].weight && w->res_conv2[i].bias &&
              w->conv_down[i].weight && w->conv_down[i].bias;
@@ -462,45 +373,37 @@ extern "C" int smol_mimi_encoder_bind(SmolMimiEncoder* e, const SmolMimiEncoderW
     cudaStream_t st = (cudaStream_t)stream;
     const size_t f4 = sizeof(float);
     auto d2d = [&](size_t off, const float* src, size_t floats) { return cudaMemcpyAsync(e->ws + off, src, floats * f4, cudaMemcpyDeviceToDevice, st); };
-    ECU(d2d(e->o_conv_in, w->conv_in.weight, (size_t)c.n_filters * c.kernel));
+    MIMI_CUDA(d2d(e->o_conv_in, w->conv_in.weight, (size_t)c.n_filters * c.kernel));
     size_t bo = e->o_bias;
-    ECU(d2d(bo, w->conv_in.bias, c.n_filters)); bo += (size_t)c.n_filters * f4;
+    MIMI_CUDA(d2d(bo, w->conv_in.bias, c.n_filters)); bo += (size_t)c.n_filters * f4;
     int ch = c.n_filters;
     for (int i = 0; i < c.n_ratios; ++i) {
-        enc_pack_conv_kernel<<<256, 256, 0, st>>>(ews(e, e->o_r1[i]), w->res_conv1[i].weight, ch / 2, ch, c.res_kernel);
-        ECU(d2d(e->o_r2[i], w->res_conv2[i].weight, (size_t)ch * (ch / 2)));
-        enc_pack_conv_kernel<<<512, 256, 0, st>>>(ews(e, e->o_dn[i]), w->conv_down[i].weight, 2 * ch, ch, 2 * e->ratio[i]);
-        ECU(d2d(bo, w->res_conv1[i].bias, ch / 2)); bo += (size_t)(ch / 2) * f4;
-        ECU(d2d(bo, w->res_conv2[i].bias, ch)); bo += (size_t)ch * f4;
-        ECU(d2d(bo, w->conv_down[i].bias, 2 * ch)); bo += (size_t)2 * ch * f4;
+        pack_conv_kernel<<<256, 256, 0, st>>>(ews(e, e->o_r1[i]), w->res_conv1[i].weight, ch / 2, ch, c.res_kernel);
+        MIMI_CUDA(d2d(e->o_r2[i], w->res_conv2[i].weight, (size_t)ch * (ch / 2)));
+        pack_conv_kernel<<<512, 256, 0, st>>>(ews(e, e->o_dn[i]), w->conv_down[i].weight, 2 * ch, ch, 2 * e->ratio[i]);
+        MIMI_CUDA(d2d(bo, w->res_conv1[i].bias, ch / 2)); bo += (size_t)(ch / 2) * f4;
+        MIMI_CUDA(d2d(bo, w->res_conv2[i].bias, ch)); bo += (size_t)ch * f4;
+        MIMI_CUDA(d2d(bo, w->conv_down[i].bias, 2 * ch)); bo += (size_t)2 * ch * f4;
         ch *= 2;
     }
-    enc_pack_conv_kernel<<<512, 256, 0, st>>>(ews(e, e->o_conv_out), w->conv_out.weight, c.dim, ch, c.last_kernel);
-    ECU(d2d(bo, w->conv_out.bias, c.dim));
+    pack_conv_kernel<<<512, 256, 0, st>>>(ews(e, e->o_conv_out), w->conv_out.weight, c.dim, ch, c.last_kernel);
+    MIMI_CUDA(d2d(bo, w->conv_out.bias, c.dim));
     for (int l = 0; l < c.n_layers; ++l) {
-        const SmolMimiLayerWeights& L = w->layers[l];
-        const size_t dd = (size_t)c.dim * c.dim;
-        ECU(d2d(e->o_qkv[l], L.q_proj, dd));
-        ECU(d2d(e->o_qkv[l] + dd * f4, L.k_proj, dd));
-        ECU(d2d(e->o_qkv[l] + 2 * dd * f4, L.v_proj, dd));
-        ECU(d2d(e->o_o[l], L.o_proj, dd));
-        ECU(d2d(e->o_fc1[l], L.fc1, (size_t)c.ffn * c.dim));
-        ECU(d2d(e->o_fc2[l], L.fc2, (size_t)c.ffn * c.dim));
-        const float* vecs[6] = {L.ln1_w, L.ln1_b, L.ln2_w, L.ln2_b, L.scale_attn, L.scale_mlp};
-        for (int i = 0; i < 6; ++i) ECU(d2d(e->o_vec[l] + (size_t)i * c.dim * f4, vecs[i], c.dim));
+        const int rc = bind_layer(e->ws, e->o_layer[l], w->layers[l], c.dim, c.ffn, st);
+        if (rc != SMOL_OK) return rc;
     }
-    enc_pack_conv_kernel<<<512, 256, 0, st>>>(ews(e, e->o_ds), w->downsample, c.dim, c.dim, 4);
-    ECU(d2d(e->o_proj, w->semantic_input_proj, (size_t)c.codebook_dim * c.dim));
-    ECU(d2d(e->o_proj + (size_t)c.codebook_dim * c.dim * f4, w->acoustic_input_proj, (size_t)c.codebook_dim * c.dim));
+    pack_conv_kernel<<<512, 256, 0, st>>>(ews(e, e->o_ds), w->downsample, c.dim, c.dim, 4);
+    MIMI_CUDA(d2d(e->o_proj, w->semantic_input_proj, (size_t)c.codebook_dim * c.dim));
+    MIMI_CUDA(d2d(e->o_proj + (size_t)c.codebook_dim * c.dim * f4, w->acoustic_input_proj, (size_t)c.codebook_dim * c.dim));
     const size_t book = (size_t)c.codebook_size * c.codebook_dim;
     for (int i = 0; i < c.n_q; ++i) {
-        enc_pack_codebook_kernel<<<256, 256, 0, st>>>(ews(e, e->o_books) + i * book, w->embed_sum[i], w->cluster_usage[i], c.codebook_size,
+        pack_codebook_kernel<<<256, 256, 0, st>>>(ews(e, e->o_books) + i * book, w->embed_sum[i], w->cluster_usage[i], c.codebook_size,
                                                       c.codebook_dim, c.codebook_eps);
         enc_row_norm_kernel<<<(c.codebook_size + 255) / 256, 256, 0, st>>>(ews(e, e->o_norms) + (size_t)i * c.codebook_size,
                                                                            ews(e, e->o_books) + i * book, c.codebook_size, c.codebook_dim);
     }
-    ECU(d2d(e->o_rope, w->rope, (size_t)e->max_pos * c.head_dim));
-    ECU(cudaGetLastError());
+    MIMI_CUDA(d2d(e->o_rope, w->rope, (size_t)e->max_pos * c.head_dim));
+    MIMI_CUDA(cudaGetLastError());
     e->bound = true;
     return SMOL_OK;
 }
@@ -532,7 +435,7 @@ extern "C" int smol_mimi_encode(SmolMimiEncoder* e, const float* d_pcm, const in
     int launches = 0;
     auto tile = [&](const EncOp& op) -> cudaError_t {
         const dim3 grid((op.rows + kTM - 1) / kTM, (op.N + kTN - 1) / kTN);
-        enc_tile_kernel<<<grid, kThreads, 0, st>>>(op);
+        tile_kernel<EncOp><<<grid, kThreads, 0, st>>>(op);
         ++launches;
         return cudaGetLastError();
     };
@@ -557,18 +460,18 @@ extern "C" int smol_mimi_encode(SmolMimiEncoder* e, const float* d_pcm, const in
         enc_conv_in_kernel<<<(unsigned)((cnt + kThreads - 1) / kThreads), kThreads, 0, st>>>(d_pcm, ews(e, e->o_conv_in), bias, P, lvl[0][n],
                                                                                            c.n_filters, c.kernel, segs(0, 0));
         ++launches;
-        ECU(cudaGetLastError());
+        MIMI_CUDA(cudaGetLastError());
         bias += c.n_filters;
     }
     int ch = c.n_filters;
     for (int i = 0; i < e->n_st; ++i) {
         // residual block: ELU -> conv k3 (C -> C/2) -> ELU -> conv k1 (C/2 -> C), + skip (in place on P)
-        ECU(conv(P, ch, c.res_kernel, 1, 0, PRO_ELU, ews(e, e->o_r1[i]), bias, ch / 2, H, EPI_BIAS, nullptr, i, i));
+        MIMI_CUDA(conv(P, ch, c.res_kernel, 1, 0, PRO_ELU, ews(e, e->o_r1[i]), bias, ch / 2, H, EPI_BIAS, nullptr, i, i));
         bias += ch / 2;
-        ECU(conv(H, ch / 2, 1, 1, 0, PRO_ELU, ews(e, e->o_r2[i]), bias, ch, P, EPI_RES, P, i, i));
+        MIMI_CUDA(conv(H, ch / 2, 1, 1, 0, PRO_ELU, ews(e, e->o_r2[i]), bias, ch, P, EPI_RES, P, i, i));
         bias += ch;
         // ELU -> conv k = 2 r, stride r (C -> 2 C)
-        ECU(conv(P, ch, 2 * e->ratio[i], e->ratio[i], 0, PRO_ELU, ews(e, e->o_dn[i]), bias, 2 * ch, Q, EPI_BIAS, nullptr, i, i + 1));
+        MIMI_CUDA(conv(P, ch, 2 * e->ratio[i], e->ratio[i], 0, PRO_ELU, ews(e, e->o_dn[i]), bias, 2 * ch, Q, EPI_BIAS, nullptr, i, i + 1));
         bias += 2 * ch;
         ch *= 2;
         std::swap(P, Q);
@@ -576,43 +479,44 @@ extern "C" int smol_mimi_encode(SmolMimiEncoder* e, const float* d_pcm, const in
     const int L = e->n_st;          // the 25 Hz level
     const int R = lvl[L][n];
     float *X = ews(e, e->o_X), *Hn = ews(e, e->o_Hn), *QKV = ews(e, e->o_QKV), *ATT = ews(e, e->o_ATT), *FF = ews(e, e->o_FF);
-    ECU(conv(P, ch, c.last_kernel, 1, 0, PRO_ELU, ews(e, e->o_conv_out), bias, c.dim, X, EPI_BIAS, nullptr, L, L));
+    MIMI_CUDA(conv(P, ch, c.last_kernel, 1, 0, PRO_ELU, ews(e, e->o_conv_out), bias, c.dim, X, EPI_BIAS, nullptr, L, L));
     // ---- encoder transformer ----
     const Segs rows_seg = segs(L, L);
     const size_t attn_smem = (size_t)kWarps * (c.head_dim + ((c.window + 3) & ~3)) * 4;
     for (int l = 0; l < c.n_layers; ++l) {
-        const float* vec = ews(e, e->o_vec[l]);
+        const LayerOffsets& lo = e->o_layer[l];
+        const float* vec = ews(e, lo.vec);
         enc_ln_kernel<<<(R + kWarps - 1) / kWarps, kThreads, 0, st>>>(X, vec, vec + c.dim, Hn, R, c.dim, c.norm_eps);
         ++launches;
-        ECU(linear(Hn, c.dim, ews(e, e->o_qkv[l]), 3 * c.dim, QKV, EPI_BIAS, nullptr, nullptr, R));
+        MIMI_CUDA(linear(Hn, c.dim, ews(e, lo.qkv), 3 * c.dim, QKV, EPI_BIAS, nullptr, nullptr, R));
         const long long pairs = (long long)R * (c.dim / 2);
         enc_rope_kernel<<<(unsigned)((pairs + kThreads - 1) / kThreads), kThreads, 0, st>>>(QKV, ews(e, e->o_rope), R, c.dim, c.head_dim, rows_seg);
         enc_attn_kernel<<<dim3((R + kWarps - 1) / kWarps, c.n_heads), kThreads, attn_smem, st>>>(QKV, ATT, R, c.dim, c.head_dim, c.window, rows_seg);
         launches += 3;
-        ECU(cudaGetLastError());
-        ECU(linear(ATT, c.dim, ews(e, e->o_o[l]), c.dim, X, EPI_SCALE_RES, X, vec + 4 * c.dim, R));
+        MIMI_CUDA(cudaGetLastError());
+        MIMI_CUDA(linear(ATT, c.dim, ews(e, lo.o), c.dim, X, EPI_SCALE_RES, X, vec + 4 * c.dim, R));
         enc_ln_kernel<<<(R + kWarps - 1) / kWarps, kThreads, 0, st>>>(X, vec + 2 * c.dim, vec + 3 * c.dim, Hn, R, c.dim, c.norm_eps);
         ++launches;
-        ECU(linear(Hn, c.dim, ews(e, e->o_fc1[l]), c.ffn, FF, EPI_GELU, nullptr, nullptr, R));
-        ECU(linear(FF, c.ffn, ews(e, e->o_fc2[l]), c.dim, X, EPI_SCALE_RES, X, vec + 5 * c.dim, R));
+        MIMI_CUDA(linear(Hn, c.dim, ews(e, lo.fc1), c.ffn, FF, EPI_GELU, nullptr, nullptr, R));
+        MIMI_CUDA(linear(FF, c.ffn, ews(e, lo.fc2), c.dim, X, EPI_SCALE_RES, X, vec + 5 * c.dim, R));
     }
     // ---- downsample (replicate padding, no bias) -> z ----
     const int Fr = lvl[L + 1][n];
     float *Z = ews(e, e->o_Z), *RS = ews(e, e->o_RS), *RA = ews(e, e->o_RA), *S = ews(e, e->o_S);
-    ECU(conv(X, c.dim, 4, 2, 1, PRO_NONE, ews(e, e->o_ds), nullptr, c.dim, Z, EPI_BIAS, nullptr, L, L + 1));
+    MIMI_CUDA(conv(X, c.dim, 4, 2, 1, PRO_NONE, ews(e, e->o_ds), nullptr, c.dim, Z, EPI_BIAS, nullptr, L, L + 1));
     // ---- split RVQ ----
     const float* proj = ews(e, e->o_proj);
-    ECU(linear(Z, c.dim, proj, c.codebook_dim, RS, EPI_BIAS, nullptr, nullptr, Fr));
-    ECU(linear(Z, c.dim, proj + (size_t)c.codebook_dim * c.dim, c.codebook_dim, RA, EPI_BIAS, nullptr, nullptr, Fr));
+    MIMI_CUDA(linear(Z, c.dim, proj, c.codebook_dim, RS, EPI_BIAS, nullptr, nullptr, Fr));
+    MIMI_CUDA(linear(Z, c.dim, proj + (size_t)c.codebook_dim * c.dim, c.codebook_dim, RA, EPI_BIAS, nullptr, nullptr, Fr));
     const size_t book = (size_t)c.codebook_size * c.codebook_dim;
     for (int q = 0; q < c.n_q; ++q) {
         float* r = q == 0 ? RS : RA;
         const float* bk = ews(e, e->o_books) + q * book;
-        ECU(linear(r, c.codebook_dim, bk, c.codebook_size, S, EPI_BIAS, nullptr, nullptr, Fr));
+        MIMI_CUDA(linear(r, c.codebook_dim, bk, c.codebook_size, S, EPI_BIAS, nullptr, nullptr, Fr));
         enc_argmin_kernel<<<(Fr + kWarps - 1) / kWarps, kThreads, 0, st>>>(S, ews(e, e->o_norms) + (size_t)q * c.codebook_size, bk, r, d_codes,
                                                                           Fr, c.codebook_size, c.codebook_dim, c.n_q, q);
         ++launches;
-        ECU(cudaGetLastError());
+        MIMI_CUDA(cudaGetLastError());
     }
     e->launches = launches;
     return SMOL_OK;

@@ -26,27 +26,19 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
-#include <cstdlib>
 #include <cstring>
 #include <string>
 #include <vector>
 
 #include "../../include/smoltts_b200.h"
 #include "../../include/smoltts_b200_mimi.h"
+#include "mimi_common.cuh"
 
 namespace smol {
-int capi_fail(int code, const std::string& msg);              // capi.cu: sets smol_last_error()
-int capi_cuda_fail(cudaError_t e, const char* what);
-
 namespace mimi {
 
-constexpr int kThreads = 256;
-constexpr int kWarps = kThreads / 32;
 constexpr int kStageFloats = 8192;   // shared-memory staging area of rows_kernel: R rows x (8192 / R) floats
 constexpr int kMaxBufs = 24;
-
-enum { PRO_NONE = 0, PRO_ELU = 1, PRO_LN = 2 };
-enum { EPI_BIAS = 0, EPI_GELU = 1, EPI_SCALE_RES = 2, EPI_RES = 3, EPI_UPSAMPLE = 4 };
 
 struct RowOp {
     // input rows: slot arena + in_off, `in_hs` history rows before the step's T rows, in_c floats per row;
@@ -60,22 +52,43 @@ struct RowOp {
     const float* scale;
     const float* wup; float* up_prev; int carry;   // EPI_UPSAMPLE
     const int32_t* slots; int batch;
+
+    // tile_kernel's row map: row = b T + t of the batch's streams, b's stream in slot slots[b]
+    struct Rows { int slot[kTM], t[kTM], b[kTM]; };
+    __device__ void map_rows(Rows& s, int row0) const {   // (the slot table is constant during a step: read before the dependency wait)
+        const int tid = threadIdx.x;
+        if (tid < kTM) {
+            const int row = row0 + tid;
+            int b = 0, t = 0, slot = -1;
+            if (row < batch * T) { b = row / T; t = row - b * T; slot = slots ? slots[b] : b; }
+            s.slot[tid] = slot; s.t[tid] = t; s.b[tid] = b;
+        }
+        __syncthreads();
+    }
+    struct ARow { const float* base; int slot; };
+    __device__ ARow a_row(const Rows& s, int, int m) const {
+        const int slot = s.slot[m];
+        return {in + (long long)(slot < 0 ? 0 : slot) * in_stride + (long long)(in_hs + s.t[m] + tap0) * in_c, slot};
+    }
+    __device__ float4 load_a(const ARow& a, int k) const {
+        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (a.slot >= 0) {
+            const int j = k / in_c, c = k - j * in_c;
+            v = *reinterpret_cast<const float4*>(a.base + (long long)j * tapstep * in_c + c);
+            if (pro == PRO_ELU) v = elu4(v);
+        }
+        return v;
+    }
+    __device__ bool out_row(const Rows& s, int, int m, long long& oe, long long& re) const {
+        const int slot = s.slot[m];
+        if (slot < 0) return false;
+        oe = (long long)(out_by_row ? s.b[m] : slot) * out_stride + out_off0 + (long long)s.t[m] * N;
+        re = (long long)slot * res_stride + res_off0 + (long long)s.t[m] * N;
+        return true;
+    }
+    __device__ int bias_col(int n) const { return n % bias_mod; }   // (bias_mod: a channel count, a multiple of 4)
 };
 
-__device__ __forceinline__ float warp_sum(float v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-__device__ __forceinline__ float elu1(float x) { return x > 0.f ? x : expm1f(x); }
-__device__ __forceinline__ float gelu_erf(float x) { return 0.5f * x * (1.0f + erff(x * 0.70710678118654752440f)); }
-
-// Programmatic dependent launch: every kernel of a step is launched with the programmatic-serialization attribute, so its
-// CTAs may start while the previous kernel still runs.  Before pdl_wait() a kernel touches only what no kernel of the step
-// writes (weights: prefetched into L2); pdl_wait() returns when the previous kernel has completed and its writes are
-// visible; pdl_go() lets the next kernel's CTAs start their own prefetch.
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_go() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
 
 // Y[row][n] = epilogue( sum_k A(row, k) W[n][k] ): R staged rows per CTA, one weight row per warp (8 per CTA).
@@ -342,101 +355,12 @@ __global__ void __launch_bounds__(kThreads) lin_kernel(const RowOp op) {
     }
 }
 
-// The same product for MANY rows (12+ streams x the 16 .. 1920 rows of a SEANet stage): a 64 x 64 output tile per CTA, K in
-// steps of 16 through shared memory, 4 x 4 outputs per thread -- 16 FMAs per pair of 16-byte shared-memory loads instead of
-// the 4 of rows_kernel, whose one-weight-row-per-warp shape is built for a handful of rows.  Every output is one sequential
-// FMA chain over k = 0 .. K-1: deterministic and independent of what shares the launch, but a different order than
-// rows_kernel's lane-interleaved sums -- which kernel runs is decided by the BATCH SIZE alone (12+ streams), so a stream's bits
-// are the same in any batch of the same class (< 12 streams, 12+).  Prologues none | ELU | LayerNorm (row statistics in a pre-pass), epilogues bias |
-// residual | layer scale + residual | GELU: every operation of a step except the upsampler and the one-channel last convolution
-// (rowdot_kernel below).
-constexpr int kTM = 64, kTN = 64, kTK = 16, kTU = kTK / 16;   // kTU 16-byte pieces of A and of W per thread and K step
-// (K steps of 32: the many-row stages 15 .. 30 % slower -- fewer resident CTAs -- measured at 64 streams.)
-__global__ void __launch_bounds__(kThreads, 2) tile_kernel(const RowOp op) {
-    __shared__ __align__(16) float As[kTK][kTM + 4];
-    __shared__ __align__(16) float Ws[kTK][kTN + 4];
-    __shared__ int s_slot[kTM], s_t[kTM], s_b[kTM];
-    const int tid = threadIdx.x;
-    const int rows = op.batch * op.T;
-    const int row0 = blockIdx.y * kTM, n0 = blockIdx.x * kTN;
-    if (tid < kTM) {
-        const int row = row0 + tid;
-        int b = 0, t = 0, slot = -1;
-        if (row < rows) { b = row / op.T; t = row - b * op.T; slot = op.slots ? op.slots[b] : b; }
-        s_slot[tid] = slot; s_t[tid] = t; s_b[tid] = b;
-    }
-    __syncthreads();
-    pdl_wait();
-    pdl_go();
-    const int lm = tid >> 2, lk = (tid & 3) << 2;      // this thread's row (of A and of W) and k offset of the 16-byte pieces it loads
-    const int a_slot = s_slot[lm];
-    const float* a_base = op.in + (long long)(a_slot < 0 ? 0 : a_slot) * op.in_stride + (long long)(op.in_hs + s_t[lm] + op.tap0) * op.in_c;
-    const bool w_ok = n0 + lm < op.N;
-    const float* w_base = op.W + (long long)(n0 + lm) * op.K;
-    auto load_a = [&](int k) -> float4 {
-        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (a_slot >= 0) {
-            const int j = k / op.in_c, c = k - j * op.in_c;
-            v = *reinterpret_cast<const float4*>(a_base + (long long)j * op.tapstep * op.in_c + c);
-            if (op.pro == PRO_ELU) { v.x = elu1(v.x); v.y = elu1(v.y); v.z = elu1(v.z); v.w = elu1(v.w); }
-        }
-        return v;
-    };
-    auto load_w = [&](int k) -> float4 {
-        return w_ok ? __ldg(reinterpret_cast<const float4*>(w_base + k)) : make_float4(0.f, 0.f, 0.f, 0.f);
-    };
-    const int ty = tid >> 4, tx = tid & 15;
-    float acc[4][4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
-    float4 ra[kTU], rw[kTU];
-#pragma unroll
-    for (int u = 0; u < kTU; ++u) { ra[u] = load_a(lk + 16 * u); rw[u] = load_w(lk + 16 * u); }
-    for (int k0 = 0; k0 < op.K; k0 += kTK) {
-#pragma unroll
-        for (int u = 0; u < kTU; ++u) {
-            const int kk = lk + 16 * u;
-            As[kk + 0][lm] = ra[u].x; As[kk + 1][lm] = ra[u].y; As[kk + 2][lm] = ra[u].z; As[kk + 3][lm] = ra[u].w;
-            Ws[kk + 0][lm] = rw[u].x; Ws[kk + 1][lm] = rw[u].y; Ws[kk + 2][lm] = rw[u].z; Ws[kk + 3][lm] = rw[u].w;
-        }
-        __syncthreads();
-        if (k0 + kTK < op.K) {   // next step's pieces in flight during the FMAs
-#pragma unroll
-            for (int u = 0; u < kTU; ++u) { ra[u] = load_a(k0 + kTK + lk + 16 * u); rw[u] = load_w(k0 + kTK + lk + 16 * u); }
-        }
-#pragma unroll
-        for (int k = 0; k < kTK; ++k) {
-            const float4 a = *reinterpret_cast<const float4*>(&As[k][ty * 4]);
-            const float4 w = *reinterpret_cast<const float4*>(&Ws[k][tx * 4]);
-            acc[0][0] = fmaf(a.x, w.x, acc[0][0]); acc[0][1] = fmaf(a.x, w.y, acc[0][1]); acc[0][2] = fmaf(a.x, w.z, acc[0][2]); acc[0][3] = fmaf(a.x, w.w, acc[0][3]);
-            acc[1][0] = fmaf(a.y, w.x, acc[1][0]); acc[1][1] = fmaf(a.y, w.y, acc[1][1]); acc[1][2] = fmaf(a.y, w.z, acc[1][2]); acc[1][3] = fmaf(a.y, w.w, acc[1][3]);
-            acc[2][0] = fmaf(a.z, w.x, acc[2][0]); acc[2][1] = fmaf(a.z, w.y, acc[2][1]); acc[2][2] = fmaf(a.z, w.z, acc[2][2]); acc[2][3] = fmaf(a.z, w.w, acc[2][3]);
-            acc[3][0] = fmaf(a.w, w.x, acc[3][0]); acc[3][1] = fmaf(a.w, w.y, acc[3][1]); acc[3][2] = fmaf(a.w, w.z, acc[3][2]); acc[3][3] = fmaf(a.w, w.w, acc[3][3]);
-        }
-        __syncthreads();
-    }
-    const int n = n0 + tx * 4;
-    if (n >= op.N) return;                      // (N is a multiple of 4: the four columns of a thread are all in or all out)
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        const int m = ty * 4 + i;
-        const int slot = s_slot[m];
-        if (slot < 0) continue;
-        const long long e = (long long)op.out_off0 + (long long)s_t[m] * op.N + n;
-        float4 y = make_float4(acc[i][0], acc[i][1], acc[i][2], acc[i][3]);
-        if (op.bias) {
-            y.x += op.bias[n % op.bias_mod]; y.y += op.bias[(n + 1) % op.bias_mod];
-            y.z += op.bias[(n + 2) % op.bias_mod]; y.w += op.bias[(n + 3) % op.bias_mod];
-        }
-        if (op.epi == EPI_RES) {
-            const float4 r = *reinterpret_cast<const float4*>(op.res + (long long)slot * op.res_stride + op.res_off0 + (long long)s_t[m] * op.N + n);
-            y.x = r.x + y.x; y.y = r.y + y.y; y.z = r.z + y.z; y.w = r.w + y.w;
-        }
-        *reinterpret_cast<float4*>(op.out + (long long)(op.out_by_row ? s_b[m] : slot) * op.out_stride + e) = y;
-    }
-}
+// The same product for MANY rows: the SEANet stages from 12 streams on (16 .. 1920 rows per stream) run through the shared
+// tile_kernel<RowOp> (mimi_common.cuh), whose 4 x 4 outputs per thread make 16 FMAs per pair of 16-byte shared-memory loads
+// instead of the 4 of rows_kernel, built for a handful of rows.  Every output there is one sequential FMA chain over k: a
+// different order than rows_kernel's lane-interleaved sums, so which kernel runs is decided by the BATCH SIZE alone (12+
+// streams) and a stream's bits are the same in any batch of the same class (< 12 streams, 12+).  It takes the ELU or no
+// prologue and the bias or residual epilogue: the convolutions, transposed convolutions and residual-block convolutions.
 
 // The last convolution (one output channel) for many rows: one thread per output sample, the weight vector in shared memory.
 __global__ void __launch_bounds__(kThreads) rowdot_kernel(const RowOp op) {
@@ -696,19 +620,7 @@ struct OpRec {
     union { RowOp row; AttnArgs attn; EmbedArgs emb; ShiftArgs shift; };
 };
 
-// ---- bind-time packing ---------------------------------------------------------------------------------------------
-__global__ void pack_codebook_kernel(float* dst, const float* es, const float* cu, int rows, int dim, float eps) {
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < (long long)rows * dim; i += (long long)gridDim.x * blockDim.x)
-        dst[i] = es[i] / fmaxf(cu[i / dim], eps);
-}
-// Conv1d [Co][Ci][k] -> [Co][j * Ci + ci]
-__global__ void pack_conv_kernel(float* dst, const float* w, int Co, int Ci, int k) {
-    const long long total = (long long)Co * Ci * k;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
-        const int ci = (int)(i % Ci); const long long r = i / Ci; const int j = (int)(r % k); const int co = (int)(r / k);
-        dst[i] = w[((long long)co * Ci + ci) * k + j];
-    }
-}
+// ---- bind-time packing (codebooks and Conv1d: mimi_common.cuh) -----------------------------------------------------
 // ConvTranspose1d [Ci][Co][2 s] -> [(r, co)][(u, ci)] = w[ci][co][r + u s]   (u = 0: this input row, u = 1: the previous one)
 __global__ void pack_convtr_kernel(float* dst, const float* w, int Ci, int Co, int s) {
     const long long total = (long long)s * Co * 2 * Ci;
@@ -745,7 +657,7 @@ struct SmolMimi {
     size_t arena_floats = 0;
     // workspace layout (bytes)
     size_t o_books = 0, o_wcat = 0, o_up = 0, o_rope = 0, o_small = 0, o_conv_in = 0, o_conv_out = 0;
-    size_t o_qkv[SMOL_MIMI_MAX_LAYERS], o_o[SMOL_MIMI_MAX_LAYERS], o_fc1[SMOL_MIMI_MAX_LAYERS], o_fc2[SMOL_MIMI_MAX_LAYERS], o_vec[SMOL_MIMI_MAX_LAYERS];
+    LayerOffsets o_layer[SMOL_MIMI_MAX_LAYERS];
     size_t o_ct[SMOL_MIMI_MAX_RATIOS], o_r1[SMOL_MIMI_MAX_RATIOS], o_r2[SMOL_MIMI_MAX_RATIOS], o_bias = 0;
     size_t o_arena = 0, o_kv = 0, o_pos = 0, o_upprev = 0, o_err = 0, total = 0;
     unsigned char* ws = nullptr;
@@ -762,8 +674,6 @@ struct SmolMimi {
     void drop_steps() { for (Step& s : steps) if (s.graph) cudaGraphExecDestroy(s.graph); steps.clear(); }
 };
 constexpr size_t kMaxSteps = 16;
-
-static size_t al(size_t v) { return (v + 255) / 256 * 256; }
 
 static int mimi_plan(SmolMimi* m) {
     const SmolMimiConfig& c = m->cfg;
@@ -788,38 +698,31 @@ static int mimi_plan(SmolMimi* m) {
     m->arena_floats = (off + 63) / 64 * 64;
     if ((int)m->bufs.size() > kMaxBufs) return -1;
     // workspace
-    size_t o = 0;
-    auto take = [&](size_t floats) { const size_t r = o; o = al(o + floats * 4); return r; };
-    m->o_books = take((size_t)c.n_q * c.codebook_size * c.codebook_dim);
-    m->o_wcat = take((size_t)c.dim * 2 * c.codebook_dim);
-    m->o_up = take((size_t)c.dim * 4);
-    m->o_rope = take((size_t)c.max_positions * c.head_dim);
-    for (int l = 0; l < c.n_layers; ++l) {
-        m->o_qkv[l] = take((size_t)3 * c.dim * c.dim);
-        m->o_o[l] = take((size_t)c.dim * c.dim);
-        m->o_fc1[l] = take((size_t)c.ffn * c.dim);
-        m->o_fc2[l] = take((size_t)c.dim * c.ffn);
-        m->o_vec[l] = take((size_t)6 * c.dim);   // ln1 w|b, ln2 w|b, scale_attn, scale_mlp
-    }
-    m->o_conv_in = take((size_t)m->ch0 * c.dim * c.kernel);
+    WsPlan p;
+    m->o_books = p.take((size_t)c.n_q * c.codebook_size * c.codebook_dim);
+    m->o_wcat = p.take((size_t)c.dim * 2 * c.codebook_dim);
+    m->o_up = p.take((size_t)c.dim * 4);
+    m->o_rope = p.take((size_t)c.max_positions * c.head_dim);
+    for (int l = 0; l < c.n_layers; ++l) m->o_layer[l] = plan_layer(p, c.dim, c.ffn);
+    m->o_conv_in = p.take((size_t)m->ch0 * c.dim * c.kernel);
     ch = m->ch0;
     for (int i = 0; i < c.n_ratios; ++i) {
-        m->o_ct[i] = take((size_t)ch * (ch / 2) * 2 * c.ratios[i]);
+        m->o_ct[i] = p.take((size_t)ch * (ch / 2) * 2 * c.ratios[i]);
         ch /= 2;
-        m->o_r1[i] = take((size_t)(ch / 2) * ch * c.res_kernel);
-        m->o_r2[i] = take((size_t)ch * (ch / 2));
+        m->o_r1[i] = p.take((size_t)(ch / 2) * ch * c.res_kernel);
+        m->o_r2[i] = p.take((size_t)ch * (ch / 2));
     }
-    m->o_conv_out = take((size_t)ch * c.last_kernel);
-    m->o_bias = take((size_t)4 * m->ch0 + 16);   // all SEANet biases, back to back
-    m->o_arena = take(m->arena_floats * (size_t)c.max_streams);
-    m->o_kv = take((size_t)c.max_streams * c.n_layers * 2 * c.max_positions * c.dim);
-    m->o_pos = take((size_t)c.max_streams);
-    m->o_upprev = take((size_t)c.max_streams * c.dim);
-    m->o_err = take(4);
+    m->o_conv_out = p.take((size_t)ch * c.last_kernel);
+    m->o_bias = p.take((size_t)4 * m->ch0 + 16);   // all SEANet biases, back to back
+    m->o_arena = p.take(m->arena_floats * (size_t)c.max_streams);
+    m->o_kv = p.take((size_t)c.max_streams * c.n_layers * 2 * c.max_positions * c.dim);
+    m->o_pos = p.take((size_t)c.max_streams);
+    m->o_upprev = p.take((size_t)c.max_streams * c.dim);
+    m->o_err = p.take(4);
     m->max_splits = (c.max_positions + kAttnChunk - 1) / kAttnChunk;
-    m->o_part = take((size_t)c.max_streams * c.n_heads * m->max_splits * 2 * (c.head_dim + 2));
-    m->o_arrive = take((size_t)c.max_streams * c.n_heads);
-    m->total = o;
+    m->o_part = p.take((size_t)c.max_streams * c.n_heads * m->max_splits * 2 * (c.head_dim + 2));
+    m->o_arrive = p.take((size_t)c.max_streams * c.n_heads);
+    m->total = p.total;
     m->attn_smem = (size_t)(2 * c.head_dim + 2 * kThreads + 2 * kAttnChunk) * 4;
     m->max_splits = (c.max_positions + kAttnChunk - 1) / kAttnChunk;
     return 0;
@@ -857,8 +760,6 @@ extern "C" size_t smol_mimi_workspace_bytes(const SmolMimi* m) { return m ? m->t
 extern "C" int32_t smol_mimi_launches_per_step(const SmolMimi* m) { return m ? m->launches : 0; }
 extern "C" int32_t* smol_mimi_error_word(SmolMimi* m) { return (m && m->bound) ? reinterpret_cast<int32_t*>(m->ws + m->o_err) : nullptr; }
 
-#define MCU(call) do { cudaError_t e__ = (call); if (e__ != cudaSuccess) return smol::capi_cuda_fail(e__, #call); } while (0)
-
 static float* wsf(SmolMimi* m, size_t off) { return reinterpret_cast<float*>(m->ws + off); }
 
 static ShiftArgs shift_args(SmolMimi* m, const int32_t* slots, int reset) {
@@ -877,7 +778,7 @@ extern "C" int smol_mimi_reset(SmolMimi* m, const int32_t* d_slots, int32_t n, v
     ShiftArgs a = shift_args(m, d_slots, 1);
     a.batch = n;
     shift_kernel<<<dim3(n, a.n_bufs + 1), kThreads, 0, (cudaStream_t)stream>>>(a);
-    MCU(cudaGetLastError());
+    MIMI_CUDA(cudaGetLastError());
     return SMOL_OK;
 }
 
@@ -891,11 +792,7 @@ extern "C" int smol_mimi_bind(SmolMimi* m, const SmolMimiWeights* w, void* d_wor
     bool ok = need(w->semantic_output_proj) && need(w->acoustic_output_proj) && need(w->upsample) && need(w->rope) &&
               need(w->conv_in.weight) && need(w->conv_in.bias) && need(w->conv_out.weight) && need(w->conv_out.bias);
     for (int i = 0; i < c.n_q; ++i) ok = ok && need(w->embed_sum[i]) && need(w->cluster_usage[i]);
-    for (int l = 0; l < c.n_layers; ++l) {
-        const SmolMimiLayerWeights& L = w->layers[l];
-        ok = ok && need(L.q_proj) && need(L.k_proj) && need(L.v_proj) && need(L.o_proj) && need(L.fc1) && need(L.fc2) && need(L.ln1_w) &&
-             need(L.ln1_b) && need(L.ln2_w) && need(L.ln2_b) && need(L.scale_attn) && need(L.scale_mlp);
-    }
+    for (int l = 0; l < c.n_layers; ++l) ok = ok && layer_weights_ok(w->layers[l]);
     for (int i = 0; i < c.n_ratios; ++i)
         ok = ok && need(w->convtr[i].weight) && need(w->convtr[i].bias) && need(w->res_conv1[i].weight) && need(w->res_conv1[i].bias) &&
              need(w->res_conv2[i].weight) && need(w->res_conv2[i].bias);
@@ -908,53 +805,44 @@ extern "C" int smol_mimi_bind(SmolMimi* m, const SmolMimiWeights* w, void* d_wor
         pack_codebook_kernel<<<256, 256, 0, st>>>(wsf(m, m->o_books) + (size_t)i * c.codebook_size * c.codebook_dim, w->embed_sum[i],
                                                    w->cluster_usage[i], c.codebook_size, c.codebook_dim, c.codebook_eps);
     pack_hcat_kernel<<<256, 256, 0, st>>>(wsf(m, m->o_wcat), w->semantic_output_proj, w->acoustic_output_proj, c.dim, c.codebook_dim);
-    MCU(d2d(m->o_up, w->upsample, (size_t)c.dim * 4));
-    MCU(d2d(m->o_rope, w->rope, (size_t)c.max_positions * c.head_dim));
+    MIMI_CUDA(d2d(m->o_up, w->upsample, (size_t)c.dim * 4));
+    MIMI_CUDA(d2d(m->o_rope, w->rope, (size_t)c.max_positions * c.head_dim));
     for (int l = 0; l < c.n_layers; ++l) {
-        const SmolMimiLayerWeights& L = w->layers[l];
-        const size_t dd = (size_t)c.dim * c.dim;
-        MCU(d2d(m->o_qkv[l], L.q_proj, dd));
-        MCU(d2d(m->o_qkv[l] + dd * f4, L.k_proj, dd));
-        MCU(d2d(m->o_qkv[l] + 2 * dd * f4, L.v_proj, dd));
-        MCU(d2d(m->o_o[l], L.o_proj, dd));
-        MCU(d2d(m->o_fc1[l], L.fc1, (size_t)c.ffn * c.dim));
-        MCU(d2d(m->o_fc2[l], L.fc2, (size_t)c.ffn * c.dim));
-        const float* vecs[6] = {L.ln1_w, L.ln1_b, L.ln2_w, L.ln2_b, L.scale_attn, L.scale_mlp};
-        for (int i = 0; i < 6; ++i) MCU(d2d(m->o_vec[l] + (size_t)i * c.dim * f4, vecs[i], c.dim));
+        const int rc = bind_layer(m->ws, m->o_layer[l], w->layers[l], c.dim, c.ffn, st);
+        if (rc != SMOL_OK) return rc;
     }
     pack_conv_kernel<<<512, 256, 0, st>>>(wsf(m, m->o_conv_in), w->conv_in.weight, m->ch0, c.dim, c.kernel);
     size_t bo = m->o_bias;
-    MCU(d2d(bo, w->conv_in.bias, m->ch0)); bo += (size_t)m->ch0 * f4;
+    MIMI_CUDA(d2d(bo, w->conv_in.bias, m->ch0)); bo += (size_t)m->ch0 * f4;
     int ch = m->ch0;
     for (int i = 0; i < c.n_ratios; ++i) {
         pack_convtr_kernel<<<512, 256, 0, st>>>(wsf(m, m->o_ct[i]), w->convtr[i].weight, ch, ch / 2, c.ratios[i]);
         ch /= 2;
         pack_conv_kernel<<<256, 256, 0, st>>>(wsf(m, m->o_r1[i]), w->res_conv1[i].weight, ch / 2, ch, c.res_kernel);
-        MCU(d2d(m->o_r2[i], w->res_conv2[i].weight, (size_t)ch * (ch / 2)));
-        MCU(d2d(bo, w->convtr[i].bias, ch)); bo += (size_t)ch * f4;
-        MCU(d2d(bo, w->res_conv1[i].bias, ch / 2)); bo += (size_t)(ch / 2) * f4;
-        MCU(d2d(bo, w->res_conv2[i].bias, ch)); bo += (size_t)ch * f4;
+        MIMI_CUDA(d2d(m->o_r2[i], w->res_conv2[i].weight, (size_t)ch * (ch / 2)));
+        MIMI_CUDA(d2d(bo, w->convtr[i].bias, ch)); bo += (size_t)ch * f4;
+        MIMI_CUDA(d2d(bo, w->res_conv1[i].bias, ch / 2)); bo += (size_t)(ch / 2) * f4;
+        MIMI_CUDA(d2d(bo, w->res_conv2[i].bias, ch)); bo += (size_t)ch * f4;
     }
     pack_conv_kernel<<<16, 256, 0, st>>>(wsf(m, m->o_conv_out), w->conv_out.weight, 1, ch, c.last_kernel);
-    MCU(d2d(bo, w->conv_out.bias, 1));
-    MCU(cudaGetLastError());
-    MCU(cudaMemsetAsync(m->ws + m->o_err, 0, 16, st));
-    MCU(cudaMemsetAsync(m->ws + m->o_arrive, 0, (size_t)c.max_streams * c.n_heads * 4, st));
-    if (m->attn_smem > 48 * 1024) MCU(cudaFuncSetAttribute(attn_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->attn_smem));
+    MIMI_CUDA(d2d(bo, w->conv_out.bias, 1));
+    MIMI_CUDA(cudaGetLastError());
+    MIMI_CUDA(cudaMemsetAsync(m->ws + m->o_err, 0, 16, st));
+    MIMI_CUDA(cudaMemsetAsync(m->ws + m->o_arrive, 0, (size_t)c.max_streams * c.n_heads * 4, st));
+    if (m->attn_smem > 48 * 1024) MIMI_CUDA(cudaFuncSetAttribute(attn_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)m->attn_smem));
     m->bound = true;
     return smol_mimi_reset(m, nullptr, c.max_streams, stream);
 }
 
-// Launch with the programmatic-serialization attribute (see pdl_wait); SMOL_MIMI_PDL=0 launches plainly (A/B).
-static bool g_pdl = true;
+// Launch with the programmatic-serialization attribute (see pdl_wait) if `pdl`, plainly otherwise.
 template <class Args>
-static cudaError_t launch_pdl(void (*kern)(const Args), dim3 grid, dim3 block, size_t smem, cudaStream_t st, const Args& a) {
+static cudaError_t launch_pdl(bool pdl, void (*kern)(const Args), dim3 grid, dim3 block, size_t smem, cudaStream_t st, const Args& a) {
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = g_pdl ? 1 : 0;
+    cfg.attrs = attr; cfg.numAttrs = pdl ? 1 : 0;
     return cudaLaunchKernelEx(&cfg, kern, a);
 }
 // (Measured and dropped: splitting a weight row over 2 .. 8 warps to get 256+ CTAs per operation changed nothing at one
@@ -966,61 +854,57 @@ static int rows_R(int rows) { return rows <= 2 ? 2 : rows <= 4 ? 4 : rows <= 8 ?
 // 12+ streams: the many-row stages go through the tile kernel (decided by the batch size alone, see tile_kernel)
 constexpr int kTileMinBatch = 12;   // measured: 8 streams 1.13 ms per step on rows_kernel vs 1.23 on the tiles; 12 streams 1.35 vs 1.30
 static bool use_tile(const RowOp& op) {
-    static const int min_batch = [] { const char* e = getenv("SMOL_MIMI_TILE_MIN_BATCH"); return e ? atoi(e) : kTileMinBatch; }();
-    return op.batch >= min_batch && op.T >= 16 && op.N >= 16 && op.N % 4 == 0 && op.K % kTK == 0 &&
+    return op.batch >= kTileMinBatch && op.T >= 16 && op.N >= 16 && op.N % 4 == 0 && op.K % kTK == 0 &&
            (op.pro == PRO_NONE || op.pro == PRO_ELU) && (op.epi == EPI_BIAS || op.epi == EPI_RES);
 }
 static bool use_rowdot(const RowOp& op) {
-    static const int min_batch = [] { const char* e = getenv("SMOL_MIMI_TILE_MIN_BATCH"); return e ? atoi(e) : kTileMinBatch; }();
-    return op.batch >= min_batch && op.N == 1 && op.K <= 1024 && op.K % 4 == 0 && op.tapstep > 0 && op.epi == EPI_BIAS && op.pro != PRO_LN;
+    return op.batch >= kTileMinBatch && op.N == 1 && op.K <= 1024 && op.K % 4 == 0 && op.tapstep > 0 && op.epi == EPI_BIAS && op.pro != PRO_LN;
 }
 
 // the two-row Linears of up to 8 streams: the lean form of rows_kernel<R, 1> (same bits)
 static bool use_lin(const RowOp& op) {
-    static const bool off = [] { const char* e = getenv("SMOL_MIMI_LIN2"); return e && e[0] == '0'; }();
     const int R = rows_R(op.batch * op.T);
-    return !off && op.batch <= 8 && op.T == 2 && op.K == op.in_c && op.tapstep > 0 && op.tap0 == 0 && op.N % kWarps == 0 && op.K >= 512 &&
+    return op.batch <= 8 && op.T == 2 && op.K == op.in_c && op.tapstep > 0 && op.tap0 == 0 && op.N % kWarps == 0 && op.K >= 512 &&
            op.K <= kStageFloats / R && op.K % 128 == 0 && op.bias == nullptr && op.out_by_row == 0 &&
            ((op.pro == PRO_LN && (op.epi == EPI_BIAS || op.epi == EPI_GELU)) || (op.pro == PRO_NONE && op.epi == EPI_SCALE_RES));
 }
 template <int R>
-static cudaError_t launch_lin(const RowOp& op, cudaStream_t st) {
+static cudaError_t launch_lin(const RowOp& op, cudaStream_t st, bool pdl) {
     const dim3 grid(op.N / kWarps);
-    if (op.pro == PRO_LN && op.epi == EPI_BIAS) return launch_pdl(lin_kernel<R, PRO_LN, EPI_BIAS>, grid, dim3(kThreads), 0, st, op);
-    if (op.pro == PRO_LN) return launch_pdl(lin_kernel<R, PRO_LN, EPI_GELU>, grid, dim3(kThreads), 0, st, op);
-    return launch_pdl(lin_kernel<R, PRO_NONE, EPI_SCALE_RES>, grid, dim3(kThreads), 0, st, op);
+    if (op.pro == PRO_LN && op.epi == EPI_BIAS) return launch_pdl(pdl, lin_kernel<R, PRO_LN, EPI_BIAS>, grid, dim3(kThreads), 0, st, op);
+    if (op.pro == PRO_LN) return launch_pdl(pdl, lin_kernel<R, PRO_LN, EPI_GELU>, grid, dim3(kThreads), 0, st, op);
+    return launch_pdl(pdl, lin_kernel<R, PRO_NONE, EPI_SCALE_RES>, grid, dim3(kThreads), 0, st, op);
 }
 
-static cudaError_t launch_rows(const RowOp& op, cudaStream_t st) {
+static cudaError_t launch_rows(const RowOp& op, cudaStream_t st, bool pdl) {
     if (use_lin(op)) {
         switch (rows_R(op.batch * op.T)) {
-            case 2: return launch_lin<2>(op, st);
-            case 4: return launch_lin<4>(op, st);
-            case 8: return launch_lin<8>(op, st);
-            default: return launch_lin<16>(op, st);
+            case 2: return launch_lin<2>(op, st, pdl);
+            case 4: return launch_lin<4>(op, st, pdl);
+            case 8: return launch_lin<8>(op, st, pdl);
+            default: return launch_lin<16>(op, st, pdl);
         }
     }
     if (use_tile(op)) {
-        const dim3 grid((op.N + kTN - 1) / kTN, (op.batch * op.T + kTM - 1) / kTM);
-        return launch_pdl(tile_kernel, grid, dim3(kThreads), 0, st, op);
+        const dim3 grid((op.batch * op.T + kTM - 1) / kTM, (op.N + kTN - 1) / kTN);
+        return launch_pdl(pdl, tile_kernel<RowOp>, grid, dim3(kThreads), 0, st, op);
     }
-    if (use_rowdot(op)) return launch_pdl(rowdot_kernel, dim3((op.batch * op.T + kThreads - 1) / kThreads), dim3(kThreads), 0, st, op);
+    if (use_rowdot(op)) return launch_pdl(pdl, rowdot_kernel, dim3((op.batch * op.T + kThreads - 1) / kThreads), dim3(kThreads), 0, st, op);
     const int rows = op.batch * op.T;
     const int R = rows_R(rows);
     // 64+ rows (the SEANet stages below 12 streams, the two-row operations from 32 streams on): four weight rows per warp -- the
     // same bits, fewer and fatter CTAs.  Measured per step: 4 streams 825 -> 748 us, 32 streams 1.99 -> 1.73 ms, 64 streams
     // 3.22 -> 2.41 ms; operations of 16 rows (8 streams' Linears) lose 12 % with it, hence the bar.
-    static const int cpw_n = [] { const char* e = getenv("SMOL_MIMI_CPW_MIN_N"); return e ? atoi(e) : 64; }();
-    if (R == 16 && rows >= 64 && op.N >= cpw_n) {
+    if (R == 16 && rows >= 64 && op.N >= 64) {
         const dim3 grid4((op.N + 4 * kWarps - 1) / (4 * kWarps), (rows + R - 1) / R);
-        return launch_pdl(rows_kernel<16, 4>, grid4, dim3(kThreads), 0, st, op);
+        return launch_pdl(pdl, rows_kernel<16, 4>, grid4, dim3(kThreads), 0, st, op);
     }
     const dim3 grid((op.N + kWarps - 1) / kWarps, (rows + R - 1) / R);
     switch (R) {
-        case 2: return launch_pdl(rows_kernel<2, 1>, grid, dim3(kThreads), 0, st, op);
-        case 4: return launch_pdl(rows_kernel<4, 1>, grid, dim3(kThreads), 0, st, op);
-        case 8: return launch_pdl(rows_kernel<8, 1>, grid, dim3(kThreads), 0, st, op);
-        default: return launch_pdl(rows_kernel<16, 1>, grid, dim3(kThreads), 0, st, op);
+        case 2: return launch_pdl(pdl, rows_kernel<2, 1>, grid, dim3(kThreads), 0, st, op);
+        case 4: return launch_pdl(pdl, rows_kernel<4, 1>, grid, dim3(kThreads), 0, st, op);
+        case 8: return launch_pdl(pdl, rows_kernel<8, 1>, grid, dim3(kThreads), 0, st, op);
+        default: return launch_pdl(pdl, rows_kernel<16, 1>, grid, dim3(kThreads), 0, st, op);
     }
 }
 
@@ -1054,12 +938,13 @@ static void mimi_program(SmolMimi* m, const int32_t* d_codes, const int32_t* d_s
         push_rows(op);
     }
     for (int l = 0; l < c.n_layers; ++l) {
-        const float* vec = wsf(m, m->o_vec[l]);
+        const LayerOffsets& lo = m->o_layer[l];
+        const float* vec = wsf(m, lo.vec);
         {   // LayerNorm -> q | k | v
             RowOp op = base_op();
             set_in(op, m->bX0, 1, false);
             op.pro = PRO_LN; op.ln_w = vec; op.ln_b = vec + c.dim; op.eps = c.norm_eps;
-            op.W = wsf(m, m->o_qkv[l]); op.N = 3 * c.dim; op.epi = EPI_BIAS;
+            op.W = wsf(m, lo.qkv); op.N = 3 * c.dim; op.epi = EPI_BIAS;
             set_out(op, m->bQKV);
             push_rows(op);
         }
@@ -1077,7 +962,7 @@ static void mimi_program(SmolMimi* m, const int32_t* d_codes, const int32_t* d_s
         {   // o_proj, layer scale, residual (in place on the stream)
             RowOp op = base_op();
             set_in(op, m->bATT, 1, false);
-            op.W = wsf(m, m->o_o[l]); op.N = c.dim; op.epi = EPI_SCALE_RES; op.scale = vec + 4 * c.dim;
+            op.W = wsf(m, lo.o); op.N = c.dim; op.epi = EPI_SCALE_RES; op.scale = vec + 4 * c.dim;
             set_out(op, m->bX0); set_res(op, m->bX0);
             push_rows(op);
         }
@@ -1085,14 +970,14 @@ static void mimi_program(SmolMimi* m, const int32_t* d_codes, const int32_t* d_s
             RowOp op = base_op();
             set_in(op, m->bX0, 1, false);
             op.pro = PRO_LN; op.ln_w = vec + 2 * c.dim; op.ln_b = vec + 3 * c.dim; op.eps = c.norm_eps;
-            op.W = wsf(m, m->o_fc1[l]); op.N = c.ffn; op.epi = EPI_GELU;
+            op.W = wsf(m, lo.fc1); op.N = c.ffn; op.epi = EPI_GELU;
             set_out(op, m->bFF);
             push_rows(op);
         }
         {   // fc2, layer scale, residual
             RowOp op = base_op();
             set_in(op, m->bFF, 1, false);
-            op.W = wsf(m, m->o_fc2[l]); op.N = c.dim; op.epi = EPI_SCALE_RES; op.scale = vec + 5 * c.dim;
+            op.W = wsf(m, lo.fc2); op.N = c.dim; op.epi = EPI_SCALE_RES; op.scale = vec + 5 * c.dim;
             set_out(op, m->bX0); set_res(op, m->bX0);
             push_rows(op);
         }
@@ -1150,14 +1035,14 @@ static void mimi_program(SmolMimi* m, const int32_t* d_codes, const int32_t* d_s
     }
 }
 
-// one launch per operation, in order
-static int mimi_enqueue(SmolMimi* m, const std::vector<OpRec>& prog, cudaStream_t st) {
+// one launch per operation, in order, with programmatic dependent launch if `pdl`
+static int mimi_enqueue(SmolMimi* m, const std::vector<OpRec>& prog, cudaStream_t st, bool pdl) {
     for (const OpRec& r : prog) {
         switch (r.kind) {
-            case OP_ROWS: MCU(launch_rows(r.row, st)); break;
-            case OP_ATTN: MCU(launch_pdl(attn_kernel, dim3(r.attn.batch, r.attn.heads, r.attn.max_splits), dim3(kThreads), m->attn_smem, st, r.attn)); break;
-            case OP_EMBED: MCU(launch_pdl(embed_kernel, dim3(r.emb.batch), dim3(256), 0, st, r.emb)); break;
-            default: MCU(launch_pdl(shift_kernel, dim3(r.shift.batch, r.shift.n_bufs + 1), dim3(kThreads), 0, st, r.shift)); break;
+            case OP_ROWS: MIMI_CUDA(launch_rows(r.row, st, pdl)); break;
+            case OP_ATTN: MIMI_CUDA(launch_pdl(pdl, attn_kernel, dim3(r.attn.batch, r.attn.heads, r.attn.max_splits), dim3(kThreads), m->attn_smem, st, r.attn)); break;
+            case OP_EMBED: MIMI_CUDA(launch_pdl(pdl, embed_kernel, dim3(r.emb.batch), dim3(256), 0, st, r.emb)); break;
+            default: MIMI_CUDA(launch_pdl(pdl, shift_kernel, dim3(r.shift.batch, r.shift.n_bufs + 1), dim3(kThreads), 0, st, r.shift)); break;
         }
     }
     m->launches = (int)prog.size();
@@ -1173,9 +1058,8 @@ extern "C" int smol_mimi_decode_step(SmolMimi* m, const int32_t* d_codes, const 
     // programmatic dependent launch: every kernel fetches its first weights and prefetches its rows into L2 before the
     // dependency wait.  Measured per step at one stream: plain launches 632 -> 549 us; inside the replayed graph 462 -> 434 us
     // with the final kernels (an earlier, heavier kernel prologue had made it 510 -> 536); at 64 streams it costs 5 % inside the graph
-    // (2.40 -> 2.52 ms; nothing either way at 10 streams), so from 12 streams on it is off; SMOL_MIMI_PDL=0/1 forces it
-    const char* pe = getenv("SMOL_MIMI_PDL");
-    g_pdl = pe ? pe[0] != '0' : (mode == 0 || batch < kTileMinBatch);
+    // (2.40 -> 2.52 ms; nothing either way at 10 streams), so from 12 streams on it is off there
+    const bool pdl = mode == 0 || batch < kTileMinBatch;
     SmolMimi::Step* step = nullptr;
     for (SmolMimi::Step& c : m->steps)
         if (c.codes == d_codes && c.slots == d_slots && c.pcm == d_pcm && c.batch == batch) { step = &c; break; }
@@ -1193,20 +1077,20 @@ extern "C" int smol_mimi_decode_step(SmolMimi* m, const int32_t* d_codes, const 
     step->used = ++m->tick;
     cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
     const bool capturing = st != nullptr && cudaStreamIsCapturing(st, &cs) == cudaSuccess && cs != cudaStreamCaptureStatusNone;
-    if (mode == 0 || capturing) return mimi_enqueue(m, step->prog, st);   // (capturing: become part of the caller's graph)
+    if (mode == 0 || capturing) return mimi_enqueue(m, step->prog, st, pdl);   // (capturing: become part of the caller's graph)
     if (!step->graph) {
-        if (!m->cap_stream) MCU(cudaStreamCreateWithFlags(&m->cap_stream, cudaStreamNonBlocking));
-        MCU(cudaStreamBeginCapture(m->cap_stream, cudaStreamCaptureModeThreadLocal));
-        const int rc = mimi_enqueue(m, step->prog, m->cap_stream);
+        if (!m->cap_stream) MIMI_CUDA(cudaStreamCreateWithFlags(&m->cap_stream, cudaStreamNonBlocking));
+        MIMI_CUDA(cudaStreamBeginCapture(m->cap_stream, cudaStreamCaptureModeThreadLocal));
+        const int rc = mimi_enqueue(m, step->prog, m->cap_stream, pdl);
         cudaGraph_t g = nullptr;
         const cudaError_t ee = cudaStreamEndCapture(m->cap_stream, &g);
         if (rc != SMOL_OK) { if (g) cudaGraphDestroy(g); return rc; }
-        MCU(ee);
+        MIMI_CUDA(ee);
         const cudaError_t ei = cudaGraphInstantiate(&step->graph, g, 0);
         cudaGraphDestroy(g);
-        MCU(ei);
+        MIMI_CUDA(ei);
     }
-    MCU(cudaGraphLaunch(step->graph, st));
+    MIMI_CUDA(cudaGraphLaunch(step->graph, st));
     return SMOL_OK;
 }
 

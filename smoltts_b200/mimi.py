@@ -90,6 +90,64 @@ def mimi_rope_table(head_dim: int, theta: float, n_pos: int) -> torch.Tensor:
     return torch.cat([ang.cos(), ang.sin()], dim=1).contiguous()
 
 
+def _aligned(ws: torch.Tensor) -> int:
+    """The 256-byte-aligned start of a workspace allocated 256 bytes larger than the engine asked for."""
+    return (ws.data_ptr() + 255) // 256 * 256
+
+
+class _Binder:
+    """What the decoder's and the encoder's bind share: state-dict tensors checked and made fp32 on the device (kept
+    alive until the engine has repacked them), the codebooks, the transformer layers, the RoPE table and the workspace."""
+
+    def __init__(self, sd: Dict[str, torch.Tensor], device: torch.device):
+        self.sd, self.device = sd, device
+        self.keep: List[torch.Tensor] = []
+
+    def _hold(self, v: torch.Tensor) -> int:
+        self.keep.append(v)
+        return v.data_ptr()
+
+    def __call__(self, key: str, shape: Sequence[int]) -> int:
+        if key not in self.sd:
+            raise KeyError(f"MimiModel.load_state_dict: missing key {key}")
+        v = self.sd[key]
+        if tuple(v.shape) != tuple(shape):
+            raise ValueError(f"MimiModel.load_state_dict: {key} has shape {tuple(v.shape)}, expected {tuple(shape)}")
+        return self._hold(v.detach().to(device=self.device, dtype=torch.float32).contiguous())
+
+    def codebooks(self, w, n_q: int, c: RVQConfig) -> None:
+        for i in range(n_q):
+            p = ("quantizer.semantic_residual_vector_quantizer.layers.0" if i == 0
+                 else f"quantizer.acoustic_residual_vector_quantizer.layers.{i - 1}")
+            w.embed_sum[i] = self(p + ".codebook.embed_sum", (c.codebook_size, c.codebook_dim))
+            w.cluster_usage[i] = self(p + ".codebook.cluster_usage", (c.codebook_size,))
+
+    def layers(self, w, prefix: str, c: MimiTransformerConfig) -> None:
+        D, F = c.d_model, c.dim_feedforward
+        for l in range(c.num_layers):
+            p = f"{prefix}.layers.{l}."
+            L = w.layers[l]
+            L.q_proj, L.k_proj = self(p + "self_attn.q_proj.weight", (D, D)), self(p + "self_attn.k_proj.weight", (D, D))
+            L.v_proj, L.o_proj = self(p + "self_attn.v_proj.weight", (D, D)), self(p + "self_attn.o_proj.weight", (D, D))
+            L.fc1, L.fc2 = self(p + "mlp.fc1.weight", (F, D)), self(p + "mlp.fc2.weight", (D, F))
+            L.ln1_w, L.ln1_b = self(p + "input_layernorm.weight", (D,)), self(p + "input_layernorm.bias", (D,))
+            L.ln2_w, L.ln2_b = self(p + "post_attention_layernorm.weight", (D,)), self(p + "post_attention_layernorm.bias", (D,))
+            L.scale_attn, L.scale_mlp = self(p + "self_attn_layer_scale.scale", (D,)), self(p + "mlp_layer_scale.scale", (D,))
+
+    def rope(self, c: MimiTransformerConfig, n_pos: int) -> int:
+        return self._hold(mimi_rope_table(c.head_dim, c.rope_theta, n_pos).to(self.device))
+
+    def bind(self, workspace_bytes, bind, handle, w) -> torch.Tensor:
+        """Allocates the engine's workspace, binds `w` into it and waits for the repacking; returns the workspace."""
+        n = int(workspace_bytes(handle))
+        ws = torch.empty(n + 256, dtype=torch.uint8, device=self.device)
+        with torch.cuda.device(self.device):
+            stream = torch.cuda.current_stream().cuda_stream
+            _capi.check(bind(handle, C.byref(w), C.c_void_p(_aligned(ws)), C.c_size_t(n), C.c_void_p(stream)))
+            torch.cuda.current_stream().synchronize()   # the source tensors in `keep` may go now: everything was repacked
+        return ws
+
+
 class MimiModel:
     """The decode half of the reference's ``MimiModel`` on one CUDA device."""
 
@@ -172,40 +230,15 @@ class MimiModel:
     def load_state_dict(self, sd: Dict[str, torch.Tensor]) -> None:
         """kyutai/mimi keys (`initialized` buffers and unused codebooks are ignored, and so are the encoder half and
         `input_proj` unless the encoder was built)."""
-        c, n_q = self.config, self.num_codebooks
-        dev = self.device
-        keep: List[torch.Tensor] = []
-
-        def t(key: str, shape: Sequence[int]) -> int:
-            if key not in sd:
-                raise KeyError(f"MimiModel.load_state_dict: missing key {key}")
-            v = sd[key]
-            if tuple(v.shape) != tuple(shape):
-                raise ValueError(f"MimiModel.load_state_dict: {key} has shape {tuple(v.shape)}, expected {tuple(shape)}")
-            v = v.detach().to(device=dev, dtype=torch.float32).contiguous()
-            keep.append(v)
-            return v.data_ptr()
-
+        c = self.config
+        t = _Binder(sd, self.device)
         w = _capi.SmolMimiWeights()
-        D, cd, cs = c.transformer.d_model, c.rvq.codebook_dim, c.rvq.codebook_size
-        for i in range(n_q):
-            p = ("quantizer.semantic_residual_vector_quantizer.layers.0" if i == 0
-                 else f"quantizer.acoustic_residual_vector_quantizer.layers.{i - 1}")
-            w.embed_sum[i] = t(p + ".codebook.embed_sum", (cs, cd))
-            w.cluster_usage[i] = t(p + ".codebook.cluster_usage", (cs,))
+        D, cd = c.transformer.d_model, c.rvq.codebook_dim
+        t.codebooks(w, self.num_codebooks, c.rvq)
         w.semantic_output_proj = t("quantizer.semantic_residual_vector_quantizer.output_proj.weight", (D, cd, 1))
         w.acoustic_output_proj = t("quantizer.acoustic_residual_vector_quantizer.output_proj.weight", (D, cd, 1))
         w.upsample = t("upsample.conv.weight", (D, 1, 4))
-        F = c.transformer.dim_feedforward
-        for l in range(c.transformer.num_layers):
-            p = f"decoder_transformer.layers.{l}."
-            L = w.layers[l]
-            L.q_proj, L.k_proj = t(p + "self_attn.q_proj.weight", (D, D)), t(p + "self_attn.k_proj.weight", (D, D))
-            L.v_proj, L.o_proj = t(p + "self_attn.v_proj.weight", (D, D)), t(p + "self_attn.o_proj.weight", (D, D))
-            L.fc1, L.fc2 = t(p + "mlp.fc1.weight", (F, D)), t(p + "mlp.fc2.weight", (D, F))
-            L.ln1_w, L.ln1_b = t(p + "input_layernorm.weight", (D,)), t(p + "input_layernorm.bias", (D,))
-            L.ln2_w, L.ln2_b = t(p + "post_attention_layernorm.weight", (D,)), t(p + "post_attention_layernorm.bias", (D,))
-            L.scale_attn, L.scale_mlp = t(p + "self_attn_layer_scale.scale", (D,)), t(p + "mlp_layer_scale.scale", (D,))
+        t.layers(w, "decoder_transformer", c.transformer)
         s = c.seanet
         ch = s.n_filters * 2 ** len(s.ratios)
         w.conv_in.weight, w.conv_in.bias = t("decoder.layers.0.conv.weight", (ch, D, s.kernel_size)), t("decoder.layers.0.conv.bias", (ch,))
@@ -221,55 +254,23 @@ class MimiModel:
             idx += 3
         w.conv_out.weight = t(f"decoder.layers.{idx + 1}.conv.weight", (1, ch, s.last_kernel_size))
         w.conv_out.bias = t(f"decoder.layers.{idx + 1}.conv.bias", (1,))
-        rope = mimi_rope_table(c.transformer.head_dim, c.transformer.rope_theta, 2 * self.max_frames).to(dev)
-        keep.append(rope)
-        w.rope = rope.data_ptr()
-        n = int(self._lib.smol_mimi_workspace_bytes(self._h))
-        self._ws = torch.empty(n + 256, dtype=torch.uint8, device=dev)
-        base = (self._ws.data_ptr() + 255) // 256 * 256
-        with torch.cuda.device(dev):
-            stream = torch.cuda.current_stream().cuda_stream
-            _capi.check(self._lib.smol_mimi_bind(self._h, C.byref(w), C.c_void_p(base), C.c_size_t(n), C.c_void_p(stream)))
-            torch.cuda.current_stream().synchronize()   # the source tensors in `keep` may go now: everything was repacked
+        w.rope = t.rope(c.transformer, 2 * self.max_frames)
+        self._ws = t.bind(self._lib.smol_mimi_workspace_bytes, self._lib.smol_mimi_bind, self._h, w)
         self._free = list(range(self.max_streams - 1, -1, -1))
         self._frames = [0] * self.max_streams
         if self._enc is not None:
             self._bind_encoder(sd)
 
     def _bind_encoder(self, sd: Dict[str, torch.Tensor]) -> None:
-        c, n_q, dev = self.config, self.num_codebooks, self.device
-        keep: List[torch.Tensor] = []
-
-        def t(key: str, shape: Sequence[int]) -> int:
-            if key not in sd:
-                raise KeyError(f"MimiModel.load_state_dict: missing encoder key {key}")
-            v = sd[key]
-            if tuple(v.shape) != tuple(shape):
-                raise ValueError(f"MimiModel.load_state_dict: {key} has shape {tuple(v.shape)}, expected {tuple(shape)}")
-            v = v.detach().to(device=dev, dtype=torch.float32).contiguous()
-            keep.append(v)
-            return v.data_ptr()
-
+        c = self.config
+        t = _Binder(sd, self.device)
         w = _capi.SmolMimiEncoderWeights()
-        D, cd, cs = c.transformer.d_model, c.rvq.codebook_dim, c.rvq.codebook_size
-        for i in range(n_q):
-            p = ("quantizer.semantic_residual_vector_quantizer.layers.0" if i == 0
-                 else f"quantizer.acoustic_residual_vector_quantizer.layers.{i - 1}")
-            w.embed_sum[i] = t(p + ".codebook.embed_sum", (cs, cd))
-            w.cluster_usage[i] = t(p + ".codebook.cluster_usage", (cs,))
+        D, cd = c.transformer.d_model, c.rvq.codebook_dim
+        t.codebooks(w, self.num_codebooks, c.rvq)
         w.semantic_input_proj = t("quantizer.semantic_residual_vector_quantizer.input_proj.weight", (cd, D, 1))
         w.acoustic_input_proj = t("quantizer.acoustic_residual_vector_quantizer.input_proj.weight", (cd, D, 1))
         w.downsample = t("downsample.conv.weight", (D, D, 4))
-        F = c.transformer.dim_feedforward
-        for l in range(c.transformer.num_layers):
-            p = f"encoder_transformer.layers.{l}."
-            L = w.layers[l]
-            L.q_proj, L.k_proj = t(p + "self_attn.q_proj.weight", (D, D)), t(p + "self_attn.k_proj.weight", (D, D))
-            L.v_proj, L.o_proj = t(p + "self_attn.v_proj.weight", (D, D)), t(p + "self_attn.o_proj.weight", (D, D))
-            L.fc1, L.fc2 = t(p + "mlp.fc1.weight", (F, D)), t(p + "mlp.fc2.weight", (D, F))
-            L.ln1_w, L.ln1_b = t(p + "input_layernorm.weight", (D,)), t(p + "input_layernorm.bias", (D,))
-            L.ln2_w, L.ln2_b = t(p + "post_attention_layernorm.weight", (D,)), t(p + "post_attention_layernorm.bias", (D,))
-            L.scale_attn, L.scale_mlp = t(p + "self_attn_layer_scale.scale", (D,)), t(p + "mlp_layer_scale.scale", (D,))
+        t.layers(w, "encoder_transformer", c.transformer)
         s = c.seanet
         ch = s.n_filters
         w.conv_in.weight, w.conv_in.bias = t("encoder.layers.0.conv.weight", (ch, 1, s.kernel_size)), t("encoder.layers.0.conv.bias", (ch,))
@@ -284,17 +285,8 @@ class MimiModel:
             ch, idx = 2 * ch, idx + 3
         w.conv_out.weight = t(f"encoder.layers.{idx + 1}.conv.weight", (D, ch, s.last_kernel_size))
         w.conv_out.bias = t(f"encoder.layers.{idx + 1}.conv.bias", (D,))
-        hop = math.prod(s.ratios)
-        rope = mimi_rope_table(c.transformer.head_dim, c.transformer.rope_theta, -(-self.encode_max_samples // hop)).to(dev)
-        keep.append(rope)
-        w.rope = rope.data_ptr()
-        n = int(self._lib.smol_mimi_encoder_workspace_bytes(self._enc))
-        self._enc_ws = torch.empty(n + 256, dtype=torch.uint8, device=dev)
-        base = (self._enc_ws.data_ptr() + 255) // 256 * 256
-        with torch.cuda.device(dev):
-            stream = torch.cuda.current_stream().cuda_stream
-            _capi.check(self._lib.smol_mimi_encoder_bind(self._enc, C.byref(w), C.c_void_p(base), C.c_size_t(n), C.c_void_p(stream)))
-            torch.cuda.current_stream().synchronize()
+        w.rope = t.rope(c.transformer, -(-self.encode_max_samples // math.prod(s.ratios)))
+        self._enc_ws = t.bind(self._lib.smol_mimi_encoder_workspace_bytes, self._lib.smol_mimi_encoder_bind, self._enc, w)
 
     # ---- encode (audio -> codes) --------------------------------------------------------------------------------------
     def encode(self, x: Union[torch.Tensor, Sequence[torch.Tensor]]) -> Union[torch.Tensor, List[torch.Tensor]]:
@@ -331,7 +323,7 @@ class MimiModel:
     def encoder_latent(self) -> torch.Tensor:
         """Test hook: the pre-quantizer latent z of the last ``encode`` call, ``[sum_b T_b, dim]`` (clips back to back)."""
         p = self._lib.smol_mimi_encoder_debug_buffer(self._enc, b"latent")
-        base = (self._enc_ws.data_ptr() + 255) // 256 * 256
+        base = _aligned(self._enc_ws)
         n = int(self._lib.smol_mimi_encoder_workspace_bytes(self._enc))
         flat = self._enc_ws[base - self._enc_ws.data_ptr(): base - self._enc_ws.data_ptr() + n].view(torch.float32)
         off = (p - base) // 4
@@ -440,7 +432,7 @@ class MimiModel:
 
     # ---- test / profiling hooks -----------------------------------------------------------------------------------------
     def _base(self) -> int:
-        return (self._ws.data_ptr() + 255) // 256 * 256
+        return _aligned(self._ws)
 
     def _flat(self, dtype) -> torch.Tensor:
         d = self._base() - self._ws.data_ptr()
