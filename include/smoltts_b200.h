@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define SMOL_ABI_VERSION 1
+#define SMOL_ABI_VERSION 2
 #define SMOL_MAX_LAYERS 64
 #define SMOL_MAX_FAST_LAYERS 16
 
@@ -81,6 +81,17 @@ typedef struct SmolWeights {
     SmolLayerWeights fast_layers[SMOL_MAX_FAST_LAYERS];
 } SmolWeights;
 
+/* One sequence's sampling parameters (SmolBatch.row_sampling): the fields of SmolSampling below that may differ
+ * between the rows of one call.  temp == 0 -> argmax slow id, fast_temp == 0 -> argmax depth codes.  32 bytes. */
+typedef struct SmolRowSampling {
+    float temp, fast_temp;
+    int32_t top_k;       /* slow token only; 0 = off */
+    float top_p;         /* slow token only; >= 1 = off */
+    float min_p;         /* "intended" min-p; 0 = off */
+    uint32_t pad;
+    uint64_t seed;
+} SmolRowSampling;
+
 /* Per-batch device state (the reference keeps these in Python: G:25-57, K:6-22). */
 typedef struct SmolBatch {
     int32_t* tokens;        /* [B, R] current input column: row 0 vocab id, rows 1.. depth codes (G:143-145) */
@@ -92,6 +103,11 @@ typedef struct SmolBatch {
     int32_t* step;          /* [B] frames emitted so far (RNG counter word, index into out_codes) */
     int32_t* out_codes;     /* [B, max_frames, R] every emitted column, or NULL */
     int32_t max_frames;
+    const SmolRowSampling* row_sampling; /* [B] device, or NULL: every row samples with the call's SmolSampling.  When set,
+                                            row b samples with row_sampling[b] and the call's SmolSampling supplies only
+                                            audio_only / ignore_stop.  Read by every launch that samples, never written:
+                                            new contents between calls need no other change (no graph recapture).
+                                            Forced ids (smol_set_force) still win. */
 } SmolBatch;
 
 /* GenerationSettings (G:12-16) + the north-star's top-k / top-p / seed. temp == 0 -> argmax. */
@@ -153,7 +169,7 @@ int smol_fast_step(SmolModel* m, const SmolBatch* b, int32_t batch, int32_t dept
 int smol_fast_embed(SmolModel* m, int32_t batch, const int32_t* d_codes, int32_t depth_pos, void* stream);
 
 /* Sampling on caller-provided logits (G:88-99,118-132): d_logits [B, n] fp32 -> d_out [B]. stream_id:
- * 0 = slow token, 1+i = depth code i (RNG counter word). */
+ * 0 = slow token, 1+i = depth code i (RNG counter word).  b may be NULL; b->row_sampling, when set, replaces s per row. */
 int smol_sample(SmolModel* m, const SmolBatch* b, int32_t batch, const float* d_logits, int32_t n,
                 const SmolSampling* s, int32_t stream_id, int32_t* d_out, void* stream);
 

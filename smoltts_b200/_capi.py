@@ -11,7 +11,7 @@ import os
 
 from . import build as _build
 
-SMOL_ABI_VERSION = 1
+SMOL_ABI_VERSION = 2
 SMOL_MAX_LAYERS = 64
 SMOL_MAX_FAST_LAYERS = 16
 
@@ -45,11 +45,17 @@ class SmolWeights(C.Structure):
         ("fast_layers", SmolLayerWeights * SMOL_MAX_FAST_LAYERS)]
 
 
+class SmolRowSampling(C.Structure):
+    _fields_ = [
+        ("temp", C.c_float), ("fast_temp", C.c_float), ("top_k", C.c_int32), ("top_p", C.c_float), ("min_p", C.c_float),
+        ("pad", C.c_uint32), ("seed", C.c_uint64)]
+
+
 class SmolBatch(C.Structure):
     _fields_ = [
         ("tokens", C.c_void_p), ("seq_len", C.c_void_p), ("block_table", C.c_void_p), ("max_pages", C.c_int32),
         ("finished", C.c_void_p), ("seq_id", C.c_void_p), ("step", C.c_void_p), ("out_codes", C.c_void_p),
-        ("max_frames", C.c_int32)]
+        ("max_frames", C.c_int32), ("row_sampling", C.c_void_p)]
 
 
 class SmolSampling(C.Structure):

@@ -22,8 +22,8 @@ cudaError_t decode_configure(int bt, size_t smem);
 cudaError_t decode_max_ctas(int bt, size_t smem, int* per_sm);
 cudaError_t decode_launch(const DevModel& M, const CallArgs& A, int bt, int n_ctas, size_t smem, int xs_bytes,
                           cudaStream_t stream);
-cudaError_t sample_launch(const float* logits, int n, int batch, const SmolSampling& s, int stream_id,
-                          const int32_t* seq_id, const int32_t* step, int32_t* out, cudaStream_t stream);
+cudaError_t sample_launch(const float* logits, int n, int batch, const SmolSampling& s, const SmolRowSampling* table,
+                          int stream_id, const int32_t* seq_id, const int32_t* step, int32_t* out, cudaStream_t stream);
 cudaError_t store_codes_launch(int32_t* frame_tokens, const int32_t* codes, int batch, int n_rows, int row,
                                cudaStream_t stream);
 cudaError_t silu_lut_launch(uint16_t* lut, cudaStream_t stream);
@@ -39,6 +39,8 @@ cudaError_t ll2_pack_launch(uint16_t* dst, const uint16_t* a, const uint16_t* b,
 
 using smol::CallArgs;
 using smol::DevModel;
+
+static_assert(sizeof(SmolRowSampling) == 32, "SmolRowSampling is 32 bytes (include/smoltts_b200.h)");
 
 struct GraphKey {
     SmolBatch b;
@@ -626,7 +628,7 @@ static CallArgs base_args(const SmolBatch* b, int batch, const SmolSampling* s) 
     std::memset(&A, 0, sizeof(A));
     A.b = *b;
     if (s) A.s = *s;
-    else { A.s.temp = 0.f; A.s.fast_temp = 0.f; A.s.top_p = 1.f; A.s.ignore_stop = 1; }
+    else { A.s.temp = 0.f; A.s.fast_temp = 0.f; A.s.top_p = 1.f; A.s.ignore_stop = 1; A.b.row_sampling = nullptr; }
     A.batch = batch;
     A.real_batch = batch;
     A.tile_t = 1;
@@ -708,8 +710,8 @@ int smol_sample(SmolModel* m, const SmolBatch* b, int32_t batch, const float* d_
     if (!m || !d_logits || !s || !d_out) return fail(SMOL_ERR_INVALID, "smol_sample: null argument");
     if (n <= 0 || n > smol::kThreads * 8) return fail(SMOL_ERR_UNSUPPORTED, "smol_sample: n outside [1, 4096]");
     if (batch <= 0) return fail(SMOL_ERR_INVALID, "smol_sample: bad batch");
-    CU(smol::sample_launch(d_logits, n, batch, *s, stream_id, b ? b->seq_id : nullptr, b ? b->step : nullptr, d_out,
-                           (cudaStream_t)stream));
+    CU(smol::sample_launch(d_logits, n, batch, *s, b ? b->row_sampling : nullptr, stream_id, b ? b->seq_id : nullptr,
+                           b ? b->step : nullptr, d_out, (cudaStream_t)stream));
     m->launches += 1;
     return SMOL_OK;
 }

@@ -814,9 +814,9 @@ __device__ void phase_sample(const DevModel& M, const CallArgs& A, const Ctx& c,
         __syncthreads();
         const uint32_t step = A.b.step ? (uint32_t)ldcg_i32(A.b.step + b) : 0u;
         const uint32_t seq_id = A.b.seq_id ? (uint32_t)ldcg_i32(A.b.seq_id + b) : (uint32_t)b;
-        const float temp = fast ? A.s.fast_temp : A.s.temp;
-        int tok = sample_row<kThreads>(c.xs, N, temp, fast ? 0 : A.s.top_k, fast ? 1.0f : A.s.top_p, A.s.min_p, A.s.seed,
-                             step, seq_id, (uint32_t)r, g_sc);
+        const SmolRowSampling prm = row_sampling(A.s, A.b.row_sampling, b);
+        int tok = sample_row<kThreads>(c.xs, N, fast ? prm.fast_temp : prm.temp, fast ? 0 : prm.top_k, fast ? 1.0f : prm.top_p,
+                             prm.min_p, prm.seed, step, seq_id, (uint32_t)r, g_sc);
         if (M.force != nullptr) tok = ldcg_i32(M.force + (size_t)b * R + r);
         if (c.tid == 0) {
             M.frame_tokens[(size_t)b * R + r] = tok;
@@ -1006,16 +1006,17 @@ smol_decode_kernel(const __grid_constant__ DevModel M, const __grid_constant__ C
 
 // Stand-alone sampler on caller-provided logits [B][n] (smol_sample): one CTA per sequence.
 __global__ void __launch_bounds__(kThreads, 1)
-smol_sample_kernel(const float* logits, int n, int batch, SmolSampling s, int stream_id, const int32_t* seq_id,
-                   const int32_t* step, int32_t* out) {
+smol_sample_kernel(const float* logits, int n, int batch, SmolSampling s, const SmolRowSampling* table, int stream_id,
+                   const int32_t* seq_id, const int32_t* step, int32_t* out) {
     extern __shared__ __align__(16) float smem_sample[];
     float* smem_dyn = smem_sample;
     for (int b = blockIdx.x; b < batch; b += gridDim.x) {
         for (int i = threadIdx.x; i < n; i += kThreads) smem_dyn[i] = logits[(size_t)b * n + i];
         __syncthreads();
         const bool fast = stream_id != 0;
-        const int tok = sample_row<kThreads>(smem_dyn, n, fast ? s.fast_temp : s.temp, fast ? 0 : s.top_k, fast ? 1.0f : s.top_p,
-                                   s.min_p, s.seed, step ? (uint32_t)step[b] : 0u, seq_id ? (uint32_t)seq_id[b] : (uint32_t)b,
+        const SmolRowSampling prm = row_sampling(s, table, b);
+        const int tok = sample_row<kThreads>(smem_dyn, n, fast ? prm.fast_temp : prm.temp, fast ? 0 : prm.top_k, fast ? 1.0f : prm.top_p,
+                                   prm.min_p, prm.seed, step ? (uint32_t)step[b] : 0u, seq_id ? (uint32_t)seq_id[b] : (uint32_t)b,
                                    (uint32_t)stream_id, g_sc);
         if (threadIdx.x == 0) out[b] = tok;
         __syncthreads();
@@ -1028,12 +1029,13 @@ __global__ void smol_store_codes_kernel(int32_t* frame_tokens, const int32_t* co
     if (b < batch) frame_tokens[(size_t)b * n_rows + row] = codes[b];
 }
 
-cudaError_t sample_launch(const float* logits, int n, int batch, const SmolSampling& s, int stream_id,
-                          const int32_t* seq_id, const int32_t* step, int32_t* out, cudaStream_t stream) {
+cudaError_t sample_launch(const float* logits, int n, int batch, const SmolSampling& s, const SmolRowSampling* table,
+                          int stream_id, const int32_t* seq_id, const int32_t* step, int32_t* out, cudaStream_t stream) {
     const size_t smem = (size_t)n * sizeof(float);
     cudaError_t e = cudaFuncSetAttribute(smol_sample_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
     if (e != cudaSuccess) return e;
-    smol_sample_kernel<<<batch < 1024 ? batch : 1024, kThreads, smem, stream>>>(logits, n, batch, s, stream_id, seq_id, step, out);
+    smol_sample_kernel<<<batch < 1024 ? batch : 1024, kThreads, smem, stream>>>(logits, n, batch, s, table, stream_id, seq_id,
+                                                                               step, out);
     return cudaGetLastError();
 }
 

@@ -201,6 +201,7 @@ __shared__ SampleScratch s_sc;
 __shared__ float s_ssq[kNW];            // per-warp partial sums of squares (RMSNorm)
 __shared__ uint32_t s_best;             // HEAD phases: the CTA's best (logit, index) candidate
 __shared__ int s_pos, s_step, s_fin;    // cached positions (seq_len) / frames emitted / stop flag, tracked by every CTA
+__shared__ SmolRowSampling s_rs;        // the team's sampling parameters (constant during a launch): every CTA reads the same
 __shared__ int s_tok[kMaxRows];         // pending input column
 __shared__ int s_nw[kMaxRows];          // ids chosen in the current frame
 __shared__ uint32_t s_epoch0;           // phases executed by earlier launches
@@ -446,9 +447,10 @@ __device__ __forceinline__ Seq seq_of(const DevModel& M, const CallArgs& A, int 
     s.frame_tokens = M.frame_tokens + (size_t)team * R;
     return s;
 }
-// Greedy rows (temperature 0) and forced ids need no sampler CTA: every CTA works the id out itself.
-__device__ __forceinline__ bool row_is_local(const DevModel& M, const CallArgs& A, int r) {
-    return M.force != nullptr || (r == 0 ? A.s.temp : A.s.fast_temp) == 0.0f;
+// Greedy rows (temperature 0) and forced ids need no sampler CTA: every CTA works the id out itself.  Greedy or sampled is
+// decided per team, from its own sampling parameters.
+__device__ __forceinline__ bool row_is_local(const DevModel& M, int r) {
+    return M.force != nullptr || (r == 0 ? s_rs.temp : s_rs.fast_temp) == 0.0f;
 }
 // (logit, index) packed so that unsigned max picks the larger logit and, among equal logits, the smaller index
 __device__ __forceinline__ uint32_t cand_pack(float v, int idx) {
@@ -467,7 +469,7 @@ __device__ __forceinline__ unsigned long long* cand_words(const DevModel& M, con
 // frame boundary: adopt the ids chosen in the previous frame (G:143-166).  e_prev0 = epoch of phase 0 of that frame.
 __device__ __noinline__ void frame_boundary(const DevModel& M, const CallArgs& A, const Team tm, uint32_t e_prev0) {
     const int tid = threadIdx.x;
-    if (tid < M.n_rows && !row_is_local(M, A, tid))
+    if (tid < M.n_rows && !row_is_local(M, tid))
         s_nw[tid] = (int)ll_get(tok_words(M, tm, tid) + tm.cta, e_prev0 + (uint32_t)sample_phase_index(M, tid));
     csync();
     if (tid == 0 && s_fin == 0) {
@@ -692,7 +694,7 @@ __device__ __noinline__ float stage_embedding(const DevModel& M, const CallArgs&
     } else {
         const int r = depth_pos;  // row of depth code depth_pos - 1
         int code;
-        if (row_is_local(M, A, r)) code = s_nw[r];
+        if (row_is_local(M, r)) code = s_nw[r];
         else {
             code = (int)ll_get(tok_words(M, tm, r) + tm.cta, epoch - (uint32_t)(p - sample_phase_index(M, r)));
             if (tid == 0) s_nw[r] = code;
@@ -1107,7 +1109,7 @@ __device__ __noinline__ void phase_sample(const DevModel& M, const CallArgs& A, 
     const int N = fast ? M.codebook_size : M.vocab;
     const int r = fast ? 1 + depth_pos : 0;
     const int R = M.n_rows;
-    const bool local = row_is_local(M, A, r);
+    const bool local = row_is_local(M, r);
     if (!local && tm.cta != 0) return;  // sampled rows: CTA 0 of the team samples, the others pick the id up when they need it
     int tok;
     if (sq.force != nullptr) {
@@ -1137,10 +1139,9 @@ __device__ __noinline__ void phase_sample(const DevModel& M, const CallArgs& A, 
             *reinterpret_cast<float4*>(lg + 4 * i) = make_float4(bf_lo(v.x), bf_hi(v.x), bf_lo(v.z), bf_hi(v.z));
         }
         csync();
-        const float temp = fast ? A.s.fast_temp : A.s.temp;
         const uint32_t seq_id = sq.seq_id ? (uint32_t)ldcg_i32(sq.seq_id) : 0u;
-        tok = sample_row<kCons, kSampPer>(lg, N, temp, fast ? 0 : A.s.top_k, fast ? 1.0f : A.s.top_p, A.s.min_p, A.s.seed,
-                                    (uint32_t)s_step, seq_id, (uint32_t)r, s_sc);
+        tok = sample_row<kCons, kSampPer>(lg, N, fast ? s_rs.fast_temp : s_rs.temp, fast ? 0 : s_rs.top_k, fast ? 1.0f : s_rs.top_p,
+                                    s_rs.min_p, s_rs.seed, (uint32_t)s_step, seq_id, (uint32_t)r, s_sc);
     }
     const bool last = fast && depth_pos == M.depth - 1;
     if (local) {
@@ -1318,6 +1319,7 @@ smol_ll2_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Call
             s_pos = ldcg_i32(sq.seq_len);
             s_step = sq.step ? ldcg_i32(sq.step) : 0;
             s_fin = sq.finished != nullptr ? (int)__ldcg(sq.finished) : 0;
+            s_rs = row_sampling(A.s, A.b.row_sampling, tm.team);
             s_best = 0u;
         }
         if (tid < M.n_rows) { s_tok[tid] = ldcg_i32(sq.tokens + tid); s_nw[tid] = 0; }
@@ -1444,7 +1446,7 @@ smol_ll2_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Call
             csync();
             LL2_TRACE(2);
             if (n_items == 0) {
-                if (kind == PH_HEAD && M.force == nullptr && (fast ? A.s.fast_temp : A.s.temp) == 0.0f && warp == 0 && lane < kLLRep)
+                if (kind == PH_HEAD && M.force == nullptr && (fast ? s_rs.fast_temp : s_rs.temp) == 0.0f && warp == 0 && lane < kLLRep)
                     st_relaxed_v2(cand_words(M, tm, fast ? 1 + depth_pos : 0, lane) + tm.cta, 0u, epoch);   // no rows here: the empty candidate
                 t_end = clock32_now();
                 LL2_TRACE(6);
@@ -1614,7 +1616,7 @@ smol_ll2_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Call
                 while (sl >= NSLOTS) { sl -= NSLOTS; cpar ^= 1u; }
                 cslot = sl;
             }
-            if (kind == PH_HEAD && M.force == nullptr && (fast ? A.s.fast_temp : A.s.temp) == 0.0f) {
+            if (kind == PH_HEAD && M.force == nullptr && (fast ? s_rs.fast_temp : s_rs.temp) == 0.0f) {
                 // greedy row: the CTA's best (logit, index) goes out as one word per replica
                 csync();
                 if (warp == 0 && lane < kLLRep)

@@ -219,4 +219,14 @@ static __device__ __forceinline__ int sample_row(const float* lg, int n, float t
     return sc.bcast_i32;
 }
 
+// The sampling parameters of row b: its entry of SmolBatch.row_sampling when the caller bound a table, the call's
+// SmolSampling otherwise.  Every kernel that samples takes them from here and hands them to sample_row unchanged.
+__device__ __forceinline__ SmolRowSampling row_sampling(const SmolSampling& s, const SmolRowSampling* table, int b) {
+    if (table != nullptr) return table[b];
+    SmolRowSampling r;
+    r.temp = s.temp; r.fast_temp = s.fast_temp; r.top_k = s.top_k; r.top_p = s.top_p; r.min_p = s.min_p;
+    r.pad = 0u; r.seed = s.seed;
+    return r;
+}
+
 }  // namespace smol

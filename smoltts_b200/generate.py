@@ -8,15 +8,20 @@
     added, and ``min_p`` follows the *intended* rule (the reference's is a no-op, SURVEY §8(g)-8)
     only when ``min_p_intended=True``;
   * ``generate_batch`` is new (the reference is bs=1 only): B utterances advance together inside
-    one persistent kernel launch per chunk of frames, with the stop rule evaluated on the device.
+    one persistent kernel launch per chunk of frames, with the stop rule evaluated on the device;
+    each utterance may carry its own ``GenerationSettings`` (a device table of per-row sampling
+    parameters, ``row_sampling_table``).
 """
 from __future__ import annotations
 
+import ctypes as C
+import math
 from dataclasses import dataclass
-from typing import Any, List, Optional, Sequence
+from typing import Any, List, Optional, Sequence, Union
 
 import torch
 
+from . import _capi
 from .model import DecodeBatch, RQTransformer, SlowCache
 
 
@@ -40,10 +45,39 @@ class VQToken:
     vq_tensor: Any
 
 
+def _min_p(s: GenerationSettings) -> float:
+    return float(s.min_p) if (s.min_p is not None and s.min_p_intended) else 0.0
+
+
 def _sampling(model: RQTransformer, s: GenerationSettings, audio_only: bool, ignore_stop: bool = False):
-    min_p = float(s.min_p) if (s.min_p is not None and s.min_p_intended) else 0.0
     return model.sampling(temp=s.default_temp, fast_temp=s.default_fast_temp or 0.0, top_k=s.top_k, top_p=s.top_p,
-                          min_p=min_p, seed=s.seed, audio_only=audio_only, ignore_stop=ignore_stop)
+                          min_p=_min_p(s), seed=s.seed, audio_only=audio_only, ignore_stop=ignore_stop)
+
+
+def _check_settings(s: GenerationSettings, where: str) -> None:
+    for name, t in (("default_temp", s.default_temp), ("default_fast_temp", s.default_fast_temp or 0.0)):
+        if not (math.isfinite(t) and t >= 0.0):
+            raise ValueError(f"{where}: {name} = {t} must be a finite number >= 0")
+    if s.top_k < 0:
+        raise ValueError(f"{where}: top_k = {s.top_k} must be >= 0")
+    if not (0.0 < s.top_p <= 1.0):
+        raise ValueError(f"{where}: top_p = {s.top_p} must lie in (0, 1]")
+    if s.min_p is not None and not (0.0 <= s.min_p < 1.0):
+        raise ValueError(f"{where}: min_p = {s.min_p} must lie in [0, 1)")
+
+
+def row_sampling_table(settings: Sequence[GenerationSettings]) -> torch.Tensor:
+    """Host tensor [B, 32] uint8: one ``SmolRowSampling`` record per settings object (include/smoltts_b200.h), the values
+    ``_sampling`` would put in a call's ``SmolSampling``.  Raises ``ValueError`` for parameters the sampler does not define."""
+    settings = list(settings)
+    if not settings:
+        raise ValueError("row_sampling_table: no settings")
+    recs = (_capi.SmolRowSampling * len(settings))()
+    for i, s in enumerate(settings):
+        _check_settings(s, f"settings[{i}]")
+        recs[i] = _capi.SmolRowSampling(temp=float(s.default_temp), fast_temp=float(s.default_fast_temp or 0.0), top_k=int(s.top_k),
+                                        top_p=float(s.top_p), min_p=_min_p(s), seed=int(s.seed))
+    return torch.frombuffer(bytearray(recs), dtype=torch.uint8).view(len(settings), C.sizeof(_capi.SmolRowSampling))
 
 
 class SingleBatchGenerator:
@@ -131,23 +165,34 @@ def pack_prompts(model: RQTransformer, prompts: Sequence[torch.Tensor]):
     return out.to(model.device, non_blocking=pin), lens_h.to(model.device, non_blocking=pin)
 
 
-def generate_batch(model: RQTransformer, prompts: Sequence[torch.Tensor], generation_settings: GenerationSettings,
+def generate_batch(model: RQTransformer, prompts: Sequence[torch.Tensor],
+                   generation_settings: Union[GenerationSettings, Sequence[GenerationSettings]],
                    audio_only: bool = True, fixed_frames: Optional[int] = None, chunk: int = 64,
                    seq_ids: Optional[Sequence[int]] = None, return_batch: bool = False):
     """B utterances decoded together; per-sequence semantics identical to the bs=1 loop.
 
     Returns a list of int32 tensors: audio_only -> codes [N, T_b] of the audio frames;
     otherwise [1+N, T_b] of every emitted column.  ``fixed_frames`` disables the stop rule
-    (benchmarks: random weights never emit <|im_end|> reliably, SURVEY §8(d))."""
-    s = generation_settings
+    (benchmarks: random weights never emit <|im_end|> reliably, SURVEY §8(d)).
+
+    ``generation_settings`` is one ``GenerationSettings`` for every utterance, or one per prompt: each then samples with
+    its own temperatures, top-k / top-p / min-p and seed, and keeps at most its own ``max_new_tokens + 1`` frames (the call
+    runs the largest budget; a row's frames do not depend on the others' settings or budgets)."""
     B = len(prompts)
+    per_row = not isinstance(generation_settings, GenerationSettings)
+    rows = list(generation_settings) if per_row else [generation_settings] * B
+    if len(rows) != B:
+        raise ValueError(f"{len(rows)} settings for {B} prompts")
+    budgets = [fixed_frames if fixed_frames is not None else r.max_new_tokens + 1 for r in rows]
+    table = model.row_sampling(rows) if per_row else None
     padded, lens = pack_prompts(model, prompts)
-    n_frames = fixed_frames if fixed_frames is not None else s.max_new_tokens + 1
+    n_frames = max(budgets)
     need = int(padded.shape[2]) + n_frames
     if need > model.max_seq_len:
         raise ValueError(f"prompt + frames = {need} positions exceed max_seq_len {model.max_seq_len}")
     batch = model.new_batch(B, max_positions=need, max_frames=n_frames, seq_ids=seq_ids)
-    sampling = _sampling(model, s, audio_only, ignore_stop=fixed_frames is not None)
+    batch.set_row_sampling(table)
+    sampling = _sampling(model, rows[0], audio_only, ignore_stop=fixed_frames is not None)
     model.prefill(batch, padded, lens)
     done = 0
     while done < n_frames:
@@ -156,7 +201,7 @@ def generate_batch(model: RQTransformer, prompts: Sequence[torch.Tensor], genera
         done += n
         if fixed_frames is None and done < n_frames and bool(batch.finished.all().item()):
             break
-    steps = batch.step.tolist()
+    steps = [min(st, bud) for st, bud in zip(batch.step.tolist(), budgets)]
     codes = batch.out_codes.cpu()
     tc, cfg = model.token_config, model.config
     outs: List[torch.Tensor] = []

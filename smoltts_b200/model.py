@@ -119,10 +119,23 @@ class DecodeBatch:
         # positions this batch may cache: its pages, and never past the RoPE table (max_seq_len rows)
         self.capacity = min(self.max_pages * ps, model.max_seq_len)
         self.host_len = [0] * batch  # upper bound of seq_len known on the host (capacity checks)
+        self.row_sampling: Optional[torch.Tensor] = None
         self.c = _capi.SmolBatch(
             tokens=self.tokens.data_ptr(), seq_len=self.seq_len.data_ptr(), block_table=self.block_table.data_ptr(),
             max_pages=self.max_pages, finished=self.finished.data_ptr(), seq_id=self.seq_id.data_ptr(),
             step=self.step.data_ptr(), out_codes=self.out_codes.data_ptr(), max_frames=max(max_frames, 1))
+
+    def set_row_sampling(self, table: Optional[torch.Tensor]) -> None:
+        """Per-sequence sampling parameters: ``table`` from ``RQTransformer.row_sampling`` (one record per sequence), read by
+        every later decode call; None returns every sequence to the call's ``SmolSampling``.  The batch keeps the tensor
+        alive; its contents may be rewritten in place between calls."""
+        if table is not None:
+            rec = C.sizeof(_capi.SmolRowSampling)
+            if (table.dtype != torch.uint8 or tuple(table.shape) != (self.batch, rec) or table.device != self.model.device
+                    or not table.is_contiguous()):
+                raise ValueError(f"row sampling table must be a contiguous uint8 [{self.batch}, {rec}] tensor on {self.model.device}")
+        self.row_sampling = table
+        self.c.row_sampling = table.data_ptr() if table is not None else None
 
     def release(self) -> None:
         if self.pages:
@@ -308,6 +321,14 @@ class RQTransformer:
         return _capi.SmolSampling(temp=float(temp), fast_temp=float(fast_temp or 0.0), top_k=int(top_k), top_p=float(top_p),
                                   min_p=float(min_p or 0.0), seed=int(seed), audio_only=int(audio_only),
                                   ignore_stop=int(ignore_stop))
+
+    def row_sampling(self, settings: Sequence["GenerationSettings"]) -> torch.Tensor:
+        """Device table [B, 32] uint8 of ``SmolRowSampling`` records, one per ``GenerationSettings`` (same min-p rule as a
+        call's ``SmolSampling``), for ``DecodeBatch.set_row_sampling`` / ``SmolBatch.row_sampling``.  Validated on the host:
+        ``ValueError`` for a negative or non-finite temperature, top_k < 0, top_p outside (0, 1], min_p outside [0, 1)."""
+        from .generate import row_sampling_table
+
+        return row_sampling_table(settings).to(self.device)
 
     def set_option(self, name: str, value: int) -> None:
         _capi.check(self.lib.smol_set_option(self._h, name.encode(), int(value)))

@@ -11,7 +11,8 @@ thing the reference fetches from the network for this step.
 utterances are admitted into free slots and retired at frame-chunk boundaries, the stop rule and the frame counters live
 on the device (``SmolBatch.finished`` / ``step``), and KV pages are handed out per utterance and recycled on retirement.
 The decode arithmetic does not depend on which sequences share a launch (tested bit for bit), and sampling is keyed by
-(utterance id, frame), so an utterance decodes to the same codes whatever the scheduler did around it.
+(utterance id, frame), so an utterance decodes to the same codes whatever the scheduler did around it.  Every request may
+carry its own ``GenerationSettings``: its sampling parameters go into a resident per-slot table (``SmolBatch.row_sampling``).
 """
 from __future__ import annotations
 
@@ -23,7 +24,7 @@ from typing import Deque, Dict, Iterator, List, Optional, Sequence, Tuple
 import torch
 
 from . import _capi
-from .generate import GenerationSettings, _sampling
+from .generate import GenerationSettings, _sampling, row_sampling_table
 from .model import RQTransformer
 
 
@@ -117,6 +118,7 @@ class _Request:
     uid: int
     prompt: torch.Tensor     # [R, S] int32 (host)
     budget: int              # frames this utterance may emit (max_new_tokens + 1, as the reference loop)
+    sampling: torch.Tensor   # [1, 32] uint8 (host): its SmolRowSampling record
 
 
 @dataclass
@@ -138,7 +140,9 @@ class ContinuousBatcher:
     * every ``chunk`` frames the host reads ``finished`` and ``step`` (5 bytes per slot), retires rows whose stop rule fired or
       whose frame budget is spent, copies their codes and returns their pages to the pool.
 
-    ``submit`` returns the utterance id that also seeds the sampler (``seq_id``), so results do not depend on arrival order.
+    ``submit`` returns the utterance id that also seeds the sampler (``seq_id``), so results do not depend on arrival order;
+    its ``settings`` (default: the batcher's) choose the utterance's temperatures, top-k / top-p / min-p, seed and frame budget.
+    The batcher's settings also fix the largest budget; ``audio_only`` / ``ignore_stop`` hold for every utterance.
     """
 
     def __init__(self, model: RQTransformer, settings: GenerationSettings, slots: int, max_prompt: int = 512,
@@ -162,6 +166,8 @@ class ContinuousBatcher:
         self.step = torch.zeros(slots, dtype=torch.int32, device=dev)
         self._out_rows = self.max_frames + chunk
         self.out_codes = torch.zeros(slots, self._out_rows, R, dtype=torch.int32, device=dev)
+        self.row_sampling = model.row_sampling([settings] * slots)   # [slots, 32]: rewritten for a slot at its admission
+        self._default_sampling = row_sampling_table([settings])
         self.c = self._view(0)
         self.sampling = _sampling(model, settings, audio_only, ignore_stop=ignore_stop)
         self._queue: Deque[_Request] = collections.deque()
@@ -177,7 +183,8 @@ class ContinuousBatcher:
             tokens=self.tokens.data_ptr() + 4 * b0 * R, seq_len=self.seq_len.data_ptr() + 4 * b0,
             block_table=self.block_table.data_ptr() + 4 * b0 * self.max_pages, max_pages=self.max_pages,
             finished=self.finished.data_ptr() + b0, seq_id=self.seq_id.data_ptr() + 4 * b0, step=self.step.data_ptr() + 4 * b0,
-            out_codes=self.out_codes.data_ptr() + 4 * b0 * self._out_rows * R, max_frames=self._out_rows)
+            out_codes=self.out_codes.data_ptr() + 4 * b0 * self._out_rows * R, max_frames=self._out_rows,
+            row_sampling=self.row_sampling.data_ptr() + self.row_sampling.shape[1] * b0)
 
     def close(self) -> None:
         for s in self._active:
@@ -195,19 +202,25 @@ class ContinuousBatcher:
             pass
 
     # ---- public surface ----
-    def submit(self, prompt: torch.Tensor, max_new_tokens: Optional[int] = None, uid: Optional[int] = None) -> int:
-        """Queue one utterance (token grid ``[1+N', S]`` or ``[1, 1+N', S]``); returns its id."""
+    def submit(self, prompt: torch.Tensor, max_new_tokens: Optional[int] = None, uid: Optional[int] = None,
+               settings: Optional[GenerationSettings] = None) -> int:
+        """Queue one utterance (token grid ``[1+N', S]`` or ``[1, 1+N', S]``); returns its id.  ``settings`` (None: the
+        batcher's) sample this utterance; its frame budget is ``max_new_tokens``, else ``settings.max_new_tokens``, plus one,
+        capped by the batcher's."""
         p = prompt if prompt.ndim == 2 else prompt[0]
         R = self.model.config.n_rows
         if p.shape[0] != R:
             raise ValueError(f"prompt has {p.shape[0]} rows, model expects {R}")
+        sampling = self._default_sampling if settings is None else row_sampling_table([settings])
+        if max_new_tokens is None and settings is not None:
+            max_new_tokens = settings.max_new_tokens
         budget = self.max_frames if max_new_tokens is None else min(max_new_tokens + 1, self.max_frames)
         if p.shape[1] < 2 or p.shape[1] + budget + self.chunk > self.max_positions:
             raise ValueError(f"prompt of {p.shape[1]} columns does not fit the batcher (max_prompt / max_new_tokens)")
         if uid is None:
             uid = self._next_uid
         self._next_uid = max(self._next_uid, uid) + 1
-        self._queue.append(_Request(uid, p.to(torch.int32).cpu().contiguous(), budget))
+        self._queue.append(_Request(uid, p.to(torch.int32).cpu().contiguous(), budget, sampling))
         return uid
 
     @property
@@ -248,6 +261,7 @@ class ContinuousBatcher:
         self.step[idx] = 0
         self.finished[idx] = 0
         self.seq_id[idx] = torch.tensor([r.uid for _, r in new], dtype=torch.int32, device=dev)
+        self.row_sampling[idx] = torch.cat([r.sampling for _, r in new]).to(dev)
         # prefill the new rows, one call per contiguous run of slots (rows = the run only: every other sequence is untouched)
         i = 0
         R = self.model.config.n_rows

@@ -12,6 +12,7 @@ reference, and so do they here -- ``__call__`` uses a codec stream with the upsa
 """
 from __future__ import annotations
 
+import dataclasses
 from typing import Iterator, List, Optional, Sequence
 
 import numpy as np
@@ -148,23 +149,40 @@ class SmolTTS:
                 stats["frames"], stats["audio_frames"] = n_frames, n_audio
 
     # ---- many utterances at once (new) ----
-    def synthesize_batch(self, inputs: Sequence[str], voices: Optional[Sequence[str]] = None, fixed_frames: Optional[int] = None) -> List[np.ndarray]:
+    def _batcher(self, n_inputs: int, settings: Optional[Sequence[GenerationSettings]], slots: int, chunk: int, max_prompt: int):
+        """A ContinuousBatcher for ``serve`` / ``serve_stream`` and each input's settings (None: this object's).  With a
+        settings list the batcher's frame budget is the largest of the list, so that no input's own budget is cut."""
+        from .serving import ContinuousBatcher
+
+        if settings is None:
+            return ContinuousBatcher(self.lm, self.settings, slots=slots, max_prompt=max_prompt, chunk=chunk), [None] * n_inputs
+        settings = list(settings)
+        if len(settings) != n_inputs:
+            raise ValueError(f"{len(settings)} settings for {n_inputs} inputs")
+        base = dataclasses.replace(self.settings, max_new_tokens=max(s.max_new_tokens for s in settings))
+        return ContinuousBatcher(self.lm, base, slots=slots, max_prompt=max_prompt, chunk=chunk), settings
+
+    def synthesize_batch(self, inputs: Sequence[str], voices: Optional[Sequence[str]] = None, fixed_frames: Optional[int] = None,
+                         settings: Optional[Sequence[GenerationSettings]] = None) -> List[np.ndarray]:
+        """``settings``: one ``GenerationSettings`` per input (sampling parameters, seed and frame budget), or None for this
+        object's settings."""
         voices = list(voices) if voices is not None else ["heart"] * len(inputs)
         prompts = [self._get_prompt(t, v)[0] for t, v in zip(inputs, voices)]
-        codes = generate_batch(self.lm, prompts, self.settings, fixed_frames=fixed_frames)   # list of [N, T_b]
+        codes = generate_batch(self.lm, prompts, self.settings if settings is None else list(settings),
+                               fixed_frames=fixed_frames)   # list of [N, T_b]
         return self.decode_codes(codes)
 
     def serve(self, inputs: Sequence[str], voices: Optional[Sequence[str]] = None, slots: int = 8, chunk: int = 16,
-              max_prompt: int = 512) -> Iterator[tuple]:
+              max_prompt: int = 512, settings: Optional[Sequence[GenerationSettings]] = None) -> Iterator[tuple]:
         """Continuous batching with audio out (replaces the one-blocking-call-per-request loop of server/tts_core.py:28-47):
         the utterances share ``slots`` rows of one resident decode batch (``ContinuousBatcher``); whatever retires at a chunk
-        boundary goes through the codec together, as one batch of streams.  Yields ``(index, pcm)`` in retirement order."""
-        from .serving import ContinuousBatcher
-
+        boundary goes through the codec together, as one batch of streams.  Yields ``(index, pcm)`` in retirement order.
+        ``settings``: one ``GenerationSettings`` per input, as in ``synthesize_batch``."""
         voices = list(voices) if voices is not None else ["heart"] * len(inputs)
-        cb = ContinuousBatcher(self.lm, self.settings, slots=slots, max_prompt=max_prompt, chunk=chunk)
+        cb, per_input = self._batcher(len(inputs), settings, slots, chunk, max_prompt)
         try:
-            uid_to_index = {cb.submit(self._get_prompt(t, v)[0]): i for i, (t, v) in enumerate(zip(inputs, voices))}
+            uid_to_index = {cb.submit(self._get_prompt(t, v)[0], settings=per_input[i]): i
+                            for i, (t, v) in enumerate(zip(inputs, voices))}
             while cb.pending or cb.running:
                 done = cb.step_chunk()
                 for g0 in range(0, len(done), self.codec_full.max_streams):
@@ -175,20 +193,19 @@ class SmolTTS:
             cb.close()
 
     def serve_stream(self, inputs: Sequence[str], voices: Optional[Sequence[str]] = None, slots: int = 8, chunk: int = 16,
-                     max_prompt: int = 512) -> Iterator[tuple]:
+                     max_prompt: int = 512, settings: Optional[Sequence[GenerationSettings]] = None) -> Iterator[tuple]:
         """``serve`` with audio as it is generated: every utterance in a decode slot owns a codec stream, and after each chunk
         of ``chunk`` frames the new frames of all running utterances go through the codec together.  Yields ``(index, pcm of
         the chunk, done)``; the chunks of an utterance concatenate to what ``serve`` / ``synthesize_batch`` return for it."""
-        from .serving import ContinuousBatcher
-
         codec = self.codec_full
         if slots > codec.max_streams:
             raise ValueError(f"serve_stream: {slots} slots, the codec was built for {codec.max_streams} streams")
         voices = list(voices) if voices is not None else ["heart"] * len(inputs)
-        cb = ContinuousBatcher(self.lm, self.settings, slots=slots, max_prompt=max_prompt, chunk=chunk)
+        cb, per_input = self._batcher(len(inputs), settings, slots, chunk, max_prompt)
         caches: dict = {}
         try:
-            uid_to_index = {cb.submit(self._get_prompt(t, v)[0]): i for i, (t, v) in enumerate(zip(inputs, voices))}
+            uid_to_index = {cb.submit(self._get_prompt(t, v)[0], settings=per_input[i]): i
+                            for i, (t, v) in enumerate(zip(inputs, voices))}
             while cb.pending or cb.running:
                 items = cb.step_chunk_stream()
                 live = [(uid, codes) for uid, codes, _ in items if codes.shape[-1] > 0]
