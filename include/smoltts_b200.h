@@ -207,8 +207,7 @@ int smol_set_frame_clock(SmolModel* m, uint64_t* d_frame_ns, int32_t capacity);
 /* Options: "mode" 2 (default) = data-flow persistent kernel (flag-carrying activation words, TMA
  * producer warp; whole frames at batch 1, larger batches fall back to mode 0),
  * 0 = persistent cooperative kernel with a grid barrier per phase, 1 = one launch per phase, a frame
- * captured in a CUDA graph;  "n_ctas" = grid size (default: one CTA per SM);  "ll_flags" = A/B switches of the
- * data-flow kernel used by tools/ll_ncu.py (0 = the shipped configuration);
+ * captured in a CUDA graph;  "n_ctas" = grid size (default: one CTA per SM);
  * "tc_min_batch" (default 9: the measured crossover) = rows (sequences of a decode call, sequences x prompt positions of a prefill iteration)
  * from which the tcgen05 variant runs, 0 = never;  "prefill_tile" = cap on the prompt positions per prefill iteration
  * (0 = as many as fit: 128 rows on the tensor-core variant, 8 on the CUDA-core variants).

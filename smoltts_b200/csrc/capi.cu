@@ -29,7 +29,7 @@ cudaError_t store_codes_launch(int32_t* frame_tokens, const int32_t* codes, int 
 cudaError_t silu_lut_launch(uint16_t* lut, cudaStream_t stream);
 // data-flow kernel (ll2_kernel.cu)
 namespace ll2 { using SmemPlan = LL2SmemPlan; }
-bool ll2_plan(const DevModel& M, int holdoff, int flags, ll2::SmemPlan* sp, size_t* smem);
+bool ll2_plan(const DevModel& M, int holdoff, ll2::SmemPlan* sp, size_t* smem);
 cudaError_t ll2_configure(size_t smem);
 cudaError_t ll2_max_ctas(size_t smem, int* per_sm);
 int ll2_mlp_cluster(const DevModel& M, size_t smem, int n_slots, int* n_clusters);
@@ -62,7 +62,6 @@ struct SmolModel {
     int tc_attn_split = 0;  // option: cached positions per split of the batch attention (0 = the kernel's default)
     int tc_min_batch = 9;  // rows (sequences, or prompt positions of a prefill tile) from which the tcgen05 variant runs:
                            // measured crossover (150m, us per frame): bs 8: 2276 CUDA-core vs 2566 tensor-core; bs 12: 3642 vs 2577
-    int ll_flags = 0;  // data-flow kernel: A/B switches and hold-off override (tools/ll_ncu.py)
     // data-flow kernel
     int ll2_state = 0;         // 0 unknown, 1 ready, -1 does not fit this model
     int ll2_holdoff = 400;     // option "ll_holdoff": cycles between the end of a phase and the first poll of the next
@@ -72,9 +71,6 @@ struct SmolModel {
     int ll2_cluster = 0;       // CTAs per cluster of the fused MLP (0: no cluster size fits this model / GPU)
     int ll2_clusters = 0;      // clusters of the fused grid
     int ll2_last_fused = 0;    // the last data-flow launch ran the fused MLP
-    int ll2_psum_split = 1;    // option "ll_psum_split": the fused MLP's output is staged by each cluster together (1) or by
-                               // every CTA alone (0: each polls all 7 x dim partial-sum words)
-    int ll2_last_split = 0;    // the last data-flow launch staged the fused MLP's output cluster-split
     smol::ll2::SmemPlan ll2_sp;
     size_t ll2_smem = 0;
     bool packed_ready = false; // tensor-core GEMV layout of the bound weights (rebuilt after a weight / workspace bind)
@@ -118,17 +114,15 @@ struct WsLayout {
     size_t ll, ll_epoch, ll2_score, ll2_tok, ll2_cand, ll2_psum, packed, total;
 };
 
-static int ll_batch_of(const SmolConfig& c) { (void)c; return smol::kLL2MaxTeams; }  // word regions for up to 8 teams
-
 // Word offsets of every phase's LL region for `bl` sequences x kLLRep replicas; returns the total words.
 static size_t ll_regions(const SmolConfig& c, int depth, int bl, uint32_t* off, uint16_t* len) {
     const int n_prog = smol::phases_per_frame(c.n_layer, c.n_fast_layer, depth);
     size_t words = 0;
     for (int p = 0; p < n_prog; ++p) {
         const smol::Phase ph = smol::decode_phase(p, c.n_layer, c.n_fast_layer);
-        const int n = ph.fast ? smol::ll_phase_words(ph.kind, 1, c.fast_dim, c.fast_n_head, c.fast_n_local_heads,
+        const int n = ph.fast ? smol::ll_phase_words(ph.kind, c.fast_dim, c.fast_n_head, c.fast_n_local_heads,
                                                      c.fast_intermediate_size, c.codebook_size)
-                              : smol::ll_phase_words(ph.kind, 0, c.dim, c.n_head, c.n_local_heads, c.intermediate_size,
+                              : smol::ll_phase_words(ph.kind, c.dim, c.n_head, c.n_local_heads, c.intermediate_size,
                                                      c.vocab_size);
         if (off) off[p] = (uint32_t)words;
         if (len) len[p] = (uint16_t)n;
@@ -182,7 +176,7 @@ static WsLayout ws_layout(const SmolConfig& c, int depth) {
     L.partial = take(B * c.n_head * smol::kMaxSplits * smol::kPartialStride * 4);
     L.split_count = take(B * c.n_local_heads * 4);
     L.barrier = take(256);
-    const int bl = ll_batch_of(c);
+    const int bl = smol::kLL2MaxTeams;   // word regions for up to 8 teams
     L.ll = take(ll_regions(c, depth, bl, nullptr, nullptr) * 8);
     L.ll_epoch = take(256);
     L.ll2_score = take((size_t)bl * 2 * c.n_head * ll2_score_len(c) * 8);
@@ -243,12 +237,7 @@ int smol_create(const SmolConfig* cfg, SmolModel** out) {
     const int n_prog = smol::phases_per_frame(d.n_layer, d.n_flayer, d.depth);
     if (n_prog > smol::kMaxProg) { delete m; return bad("frame program longer than 512 phases"); }
     for (int p = 0; p < n_prog; ++p) d.prog[p] = smol::pack_phase(smol::decode_phase(p, d.n_layer, d.n_flayer));
-    d.ll_batch = ll_batch_of(c);
-    ll_regions(c, depth, d.ll_batch, d.ll_off, d.ll_len);
-    {
-        const int first = 5 * d.n_layer + 2, per = 4 * d.n_flayer + 2;
-        d.ll_step_words = depth > 1 ? d.ll_off[first + per] - d.ll_off[first] : 0;
-    }
+    ll_regions(c, depth, smol::kLL2MaxTeams, d.ll_off, d.ll_len);
     *out = m;
     return SMOL_OK;
 }
@@ -477,7 +466,7 @@ static int ensure_packed(SmolModel* m) {
 static int ensure_ll2(SmolModel* m) {
     if (m->ll2_state != 0) return SMOL_OK;
     m->ll2_sp = smol::ll2::SmemPlan();
-    if (!smol::ll2_plan(m->dm, m->ll2_holdoff, m->ll_flags, &m->ll2_sp, &m->ll2_smem) || m->n_ctas > smol::kLLMaxCtas) { m->ll2_state = -1; return SMOL_OK; }
+    if (!smol::ll2_plan(m->dm, m->ll2_holdoff, &m->ll2_sp, &m->ll2_smem) || m->n_ctas > smol::kLLMaxCtas) { m->ll2_state = -1; return SMOL_OK; }
     CU(smol::ll2_configure(m->ll2_smem));
     int per_sm = 0;
     CU(smol::ll2_max_ctas(m->ll2_smem, &per_sm));
@@ -559,11 +548,8 @@ static int enqueue(SmolModel* m, CallArgs A, cudaStream_t stream, bool whole_ite
             if (A.n_iter == 0) return SMOL_OK;
             A.team_ctas = A.batch == 1 ? ll2_solo_ctas(m) : m->n_ctas / A.batch;
             A.mlp_cluster = A.batch == 1 ? ll2_fused_cluster(m, &A.team_ctas) : 0;
-            A.psum_split = A.mlp_cluster > 0 ? m->ll2_psum_split : 0;
             m->ll2_last_fused = A.mlp_cluster > 0 ? 1 : 0;
-            m->ll2_last_split = A.psum_split;
             m->ll2_sp.holdoff = m->ll2_holdoff;
-            m->ll2_sp.flags = m->ll_flags;
             CU(smol::ll2_launch(m->dm, A, m->ll2_sp, m->ll2_smem, A.team_ctas * A.batch, stream));
             m->launches += 1;
             return SMOL_OK;
@@ -835,20 +821,12 @@ int smol_set_option(SmolModel* m, const char* name, int64_t value) {
         m->frame_key_valid = false;  // a cached frame graph was captured for the other kernel variant
         return SMOL_OK;
     }
-    if (!std::strcmp(name, "ll_flags")) {
-        m->ll_flags = (int)value;
-        return SMOL_OK;
-    }
     if (!std::strcmp(name, "ll_holdoff")) {
         m->ll2_holdoff = value > 0 ? (int)value : 0;
         return SMOL_OK;
     }
     if (!std::strcmp(name, "ll_fused_mlp")) {
         m->ll2_fused_mlp = value != 0 ? 1 : 0;
-        return SMOL_OK;
-    }
-    if (!std::strcmp(name, "ll_psum_split")) {
-        m->ll2_psum_split = value != 0 ? 1 : 0;
         return SMOL_OK;
     }
     if (!std::strcmp(name, "ll_max_batch")) {
@@ -885,8 +863,6 @@ int64_t smol_get_option(const SmolModel* m, const char* name) {
     if (!std::strcmp(name, "ll_mlp_cluster")) return (int64_t)m->ll2_cluster;
     if (!std::strcmp(name, "ll_mlp_clusters")) return (int64_t)m->ll2_clusters;
     if (!std::strcmp(name, "ll_last_fused")) return (int64_t)m->ll2_last_fused;
-    if (!std::strcmp(name, "ll_psum_split")) return (int64_t)m->ll2_psum_split;
-    if (!std::strcmp(name, "ll_last_split")) return (int64_t)m->ll2_last_split;
     return -1;
 }
 

@@ -43,7 +43,6 @@ struct LL2SmemPlan {   // second-generation data-flow kernel: byte offsets into 
     int xbuf, res_x, res_h, part, desc, fq, fkv, scratch, act, ring;   // act: the fused MLP's K-slice of act (DSMEM)
     int n_slots;
     int holdoff;       // cycles between the end of a phase and the first poll of the next
-    int flags;         // experiment switches
 };
 
 struct DevLayer {
@@ -120,8 +119,6 @@ struct DevModel {
     // consumers poll ("LL" protocol: the flag travels with the data, no barrier, no fence)
     unsigned long long* ll;          // phase p, sequence b, replica r: ll + ll_off[p] + (b * kLLRep + r) * ll_len[p]
     uint32_t* ll_epoch;              // [0] phases executed by earlier launches (epochs never repeat)
-    int ll_batch;
-    uint32_t ll_step_words;          // words between the regions of the same phase of two consecutive depth steps
     uint32_t ll_off[kMaxProg];
     uint16_t ll_len[kMaxProg];
 
@@ -136,7 +133,7 @@ struct DevModel {
 };
 
 // Words (8 bytes, two bf16 + epoch) one sequence publishes in a phase; multiples of 16 words (128 B).
-__host__ __device__ inline int ll_phase_words(int kind, int fast, int dim, int n_head, int n_kv, int inter, int n_out) {
+__host__ __device__ inline int ll_phase_words(int kind, int dim, int n_head, int n_kv, int inter, int n_out) {
     int n = 0;
     switch (kind) {
         case 0: n = (n_head + 2 * n_kv) * 64 / 2; break;  // PH_QKV
@@ -147,7 +144,6 @@ __host__ __device__ inline int ll_phase_words(int kind, int fast, int dim, int n
         case 5: n = n_out / 2; break;                    // PH_HEAD
         default: n = 0; break;
     }
-    (void)fast;
     return (n + 15) / 16 * 16;
 }
 
@@ -173,7 +169,6 @@ struct CallArgs {
     int tc_split;     // tensor-core variant: cached positions per attention split (0 = default)
     int team_ctas;    // second-generation data-flow kernel: CTAs per sequence (one team each); grid = batch * team_ctas
     int mlp_cluster;  // data-flow kernel, batch 1: CTAs per thread-block cluster of the fused gated MLP (0 = unfused)
-    int psum_split;   // fused MLP: the CTAs of a cluster share the staging of the partial sums (ll2_kernel.cu: gather_psum_split)
     const int32_t* prompt;      // prefill: [B][n_rows][s_max]
     const int32_t* prompt_len;  // prefill: [B]
     int s_max;

@@ -34,6 +34,8 @@
 // assembly + stop rule G:143-171.
 
 #include <algorithm>
+#include <cstddef>
+#include <cstring>
 
 #include "common.cuh"
 #include "dev_model.h"
@@ -50,7 +52,6 @@ namespace ll2 {
 constexpr int kNW = kLL2Warps;
 constexpr int kCons = kNW * 32;
 constexpr int kMaxSlots = 8;
-constexpr int kDescWords = 16;
 constexpr int kGather = (768 + kCons - 1) / kCons;   // 16-byte polls (2 words) per thread and vector: covers K = 3072 (1536 words)
 constexpr int kNormPer = (192 + kCons - 1) / kCons;  // 4-element chunks a thread normalises (K <= 768)
 constexpr int kSampPer = (2560 + kCons - 1) / kCons; // logits per thread in the sampler
@@ -216,21 +217,69 @@ struct Team {
 };
 
 // ---- descriptors -----------------------------------------------------------------------------------
-//   word  0-1  src      LL source region (this team, this CTA's replica) | fast_embeddings row base
-//         2-3  normw    RMSNorm weight
-//         4-5  out      LL region this phase publishes to (this team, replica 0)
-//         6-7  aux      QKV: RoPE table | HEAD: fp32 logits dump
-//         8-9  wptr     packed weights: first 8-row group of this CTA
-//        10    e_back | src_kind << 8 | nrep << 12 | res_sel << 20 | gather << 21 | psum << 22 (input = a fused MLP's
-//              partial sums: 1 every CTA polls all of them, gather_psum; 2 the cluster splits them, gather_psum_split)
-//        11    K | n_items << 16
-//        12    kind | fast << 4 | layer << 8 | depth_pos << 16
-//        13    first item of this CTA
-//        14    fused MLP (W13 and W2 phases): lo | hi << 8 | n_units << 16 -- the K-slice [lo, hi) (k-blocks of w2) of this
-//              CTA's cluster and the W2 row tiles this CTA carries (i0, i0 + S, ..); 0 = not fused / no work
-//              psum == 2 (the phase after a W2 phase): j0 | n_quads << 16 -- the quads of the input vector this CTA stages
-//        15    len_out (words per replica of the output region) | n_src_words << 16
-//
+// What a phase's input vector is, and so which staging fills xbuf with it.  The inputs from IN_WORDS on are LL words
+// (polled after the hold-off).
+enum PhaseInput : uint8_t {
+    IN_NONE = 0,          // a CTA without tiles that stages nothing
+    IN_TOKEN_EMBEDDING,   // slow layer 0: embedding of the pending column (stage_embedding, with the frame boundary)
+    IN_CODE_EMBEDDING,    // depth step > 0, fast layer 0: embedding of the previous depth code (stage_embedding)
+    IN_WORDS,             // the previous phase's output words (gather_words)
+    IN_DEPTH_ATTENTION,   // fast WO: attention over the frame's depth positions from the QKV words (fast_attention)
+    IN_PSUM,              // a fused MLP's fp32 partial sums, every CTA polls all of them (gather_psum)
+    IN_PSUM_SPLIT,        // the same, split over the CTAs of the slice cluster (gather_psum_split)
+};
+
+// One phase as this CTA runs it, built once per launch (build_desc) into dynamic shared memory.  The head is what the TMA
+// producer, the phase dispatch and the fused w2 replay read (two 16-byte loads); the tail holds the rest of a weight
+// phase's operands (two more).
+struct PhaseDesc {
+    // ---- head
+    const uint16_t* wptr;      // packed weights: first tile of this CTA
+    unsigned long long* out;   // LL region this phase publishes to (this team, replica 0) | fused W2: its partial sums
+    uint8_t kind, fast, layer, depth_pos;   // the phase (Phase)
+    uint16_t K, n_items;       // reduction length; tiles of this CTA
+    struct {                   // fused MLP (W13 and W2 phases): the K-slice [lo, hi) (k-blocks of w2) of this CTA's cluster
+        uint8_t lo, hi;        // and the W2 row tiles this CTA carries (i0, i0 + S, ..); n_units = 0: not fused / no work
+        uint16_t n_units;
+    } mlp;
+    uint16_t i0;               // first item of this CTA
+    uint16_t len_out;          // words per replica of the output region
+    // ---- tail
+    union {
+        const unsigned long long* words;   // IN_WORDS, IN_DEPTH_ATTENTION, IN_PSUM*: the source region (this CTA's replica)
+        const uint16_t* emb;               // IN_CODE_EMBEDDING: the depth step's fast_embeddings rows
+    } src;
+    const uint16_t* normw;     // RMSNorm weight
+    union {
+        const uint16_t* rope;  // QKV: RoPE table
+        float* logits;         // HEAD: fp32 logits dump
+    } aux;
+    struct {                   // IN_PSUM_SPLIT: the quads [j0, j0 + n) of the input vector this CTA stages
+        uint16_t j0, n;
+    } quads;
+    uint8_t e_back;            // phases back to the one that published the input
+    uint8_t nrep;              // replicas of the output region
+    PhaseInput input;
+    uint8_t res_h;             // residual buffer the phase stages into / reads: 0 res_x, 1 res_h
+};
+static_assert(sizeof(PhaseDesc) == 64, "PhaseDesc: four 16-byte loads");
+static_assert(offsetof(PhaseDesc, src) == 32, "PhaseDesc: the head is the first two 16-byte loads");
+
+__device__ __forceinline__ void store_desc(uint32_t a, const PhaseDesc& d) {
+    uint4 v[4];
+    memcpy(v, &d, sizeof(d));
+#pragma unroll
+    for (int i = 0; i < 4; ++i) sts_v4(a + 16u * i, v[i]);
+}
+__device__ __forceinline__ void load_desc_head(uint32_t a, PhaseDesc& d) {
+    const uint4 v[2] = {lds_v4(a), lds_v4(a + 16u)};
+    memcpy(&d, v, 32);
+}
+__device__ __forceinline__ void load_desc_tail(uint32_t a, PhaseDesc& d) {
+    const uint4 v[2] = {lds_v4(a + 32u), lds_v4(a + 48u)};
+    memcpy(reinterpret_cast<unsigned char*>(&d) + 32, v, 32);
+}
+
 // Fused gated MLP (batch 1, A.mlp_cluster = S > 0; grid = clusters of S CTAs).  The 7 consumer warps split a w2 tile's
 // K = inter into the ranges [kb w / 7, kb (w + 1) / 7), and a w2 row is the sum, in warp order, of one acc / acd MMA chain
 // per range.  Cluster c < 7 owns range c: its CTAs compute the act values of the range (the w13 tiles of it, unchanged),
@@ -283,22 +332,24 @@ __device__ __forceinline__ unsigned long long* psum_region(const DevModel& M, in
     return M.ll2_psum + ((size_t)w2 * kLLRep + rep) * kNW * M.dim;
 }
 
-__device__ __forceinline__ void build_desc(const DevModel& M, const Team& tm, int S, int split, int p, uint32_t dsc) {
+__device__ __forceinline__ void build_desc(const DevModel& M, const Team& tm, int S, int p, uint32_t dsc) {
     const int rep = tm.cta % kLLRep;
     const Phase ph = unpack_phase(M.prog[p]);
     const bool fast = ph.fast != 0;
     const int kind = ph.kind;
     const int n_slow = 5 * M.n_layer;
-    uint32_t w[kDescWords];
-#pragma unroll
-    for (int i = 0; i < kDescWords; ++i) w[i] = 0u;
-    int src_kind = 3, nrep = kLLRep, n_items = 0, i0 = 0, K = 0, gather = 0, n_src = 0, e_back = 1, psum = 0;
+    PhaseDesc d = {};
+    d.kind = (uint8_t)kind; d.fast = (uint8_t)ph.fast; d.layer = (uint8_t)ph.layer; d.depth_pos = (uint8_t)ph.depth_pos;
+    d.len_out = (uint16_t)(S > 0 && kind == PH_W2 ? kNW * M.dim : M.ll_len[p]);
+    d.e_back = 1;
+    d.nrep = kLLRep;
+    d.res_h = (kind == PH_QKV || kind == PH_WO) ? 0 : 1;
     if (kind != PH_ATTN && kind != PH_SAMPLE) {
-        K = phase_k(M, ph);
+        const int K = phase_k(M, ph);
         // work item = one MMA tile of 16 row slots: 16 rows of the matrix, or 8 rows of w1 over the same 8 rows of w3
         const int items = phase_rows(M, ph) / (kind == PH_W13 ? 8 : 16);
-        i0 = (items * tm.cta) / tm.n;
-        n_items = (items * (tm.cta + 1)) / tm.n - i0;
+        int i0 = (items * tm.cta) / tm.n;
+        int n_items = (items * (tm.cta + 1)) / tm.n - i0;
         if (S > 0 && (kind == PH_W13 || kind == PH_W2)) {
             const int slice = tm.cta / S, r = tm.cta - slice * S;
             const int kb2 = (fast ? M.finter : M.inter) / 32, rt = (fast ? M.fdim : M.dim) / 16;
@@ -311,66 +362,52 @@ __device__ __forceinline__ void build_desc(const DevModel& M, const Team& tm, in
                 i0 = r;
                 n_items = 0;
             }
-            w[14] = nu > 0 ? (uint32_t)lo | ((uint32_t)hi << 8) | ((uint32_t)nu << 16) : 0u;
+            if (nu > 0) { d.mlp.lo = (uint8_t)lo; d.mlp.hi = (uint8_t)hi; d.mlp.n_units = (uint16_t)nu; }
         }
+        d.K = (uint16_t)K; d.n_items = (uint16_t)n_items; d.i0 = (uint16_t)i0;
         int p_src = p - 1;
-        unsigned long long src = 0ull;
+        d.input = IN_WORDS;
         if (kind == PH_QKV && ph.layer == 0) {
-            if (!fast) src_kind = 0;
+            if (!fast) d.input = IN_TOKEN_EMBEDDING;
             else if (ph.depth_pos == 0) p_src = n_slow - 1;  // the slow transformer's pre-norm hidden state (P:259, M:191)
             else {
-                src_kind = 2;  // embedding of the previous depth code (G:136-140)
+                d.input = IN_CODE_EMBEDDING;  // embedding of the previous depth code (G:136-140)
                 const int off = M.depthwise_wte ? (M.dup0 ? ph.depth_pos - 1 : ph.depth_pos) * M.codebook_size : 0;
-                src = (unsigned long long)(M.fast_embeddings + (size_t)off * M.fdim);
+                d.src.emb = M.fast_embeddings + (size_t)off * M.fdim;
             }
         }
-        if (src_kind == 3) {
-            src = (unsigned long long)ll_region(M, tm.team, p_src, rep);
-            n_src = (kind == PH_WO && fast) ? (M.fn_head + 2 * M.fn_kv) * kHeadDim / 2 : K / 2;
-            if (S > 0 && unpack_phase(M.prog[p_src]).kind == PH_W2) {   // 7 fp32 partials per element
-                psum = 1;
-                n_src = kNW * K;
-                src = (unsigned long long)psum_region(M, p_src, rep);
+        if (d.input == IN_WORDS) {
+            d.src.words = ll_region(M, tm.team, p_src, rep);
+            if (kind == PH_WO && fast) d.input = IN_DEPTH_ATTENTION;
+            else if (S > 0 && unpack_phase(M.prog[p_src]).kind == PH_W2) {   // 7 fp32 partials per element
+                d.input = IN_PSUM;
+                d.src.words = psum_region(M, p_src, rep);
                 // Split staging (gather_psum_split) where its early DSMEM stores are safe: in the phase right after the
                 // W2 phase (not the depth-0 QKV, which follows HEAD + SAMPLE) and in a slice cluster (not the idle one)
                 const int slice = tm.cta / S, r = tm.cta - slice * S, q = K / 4;
-                if (split && p_src == p - 1 && slice < kNW && 2 * ((q + S - 1) / S) <= kCons) {
-                    psum = 2;
+                if (p_src == p - 1 && slice < kNW && 2 * ((q + S - 1) / S) <= kCons) {
+                    d.input = IN_PSUM_SPLIT;
                     const int j0 = (q * r) / S, j1 = (q * (r + 1)) / S;
-                    w[14] = (uint32_t)j0 | ((uint32_t)(j1 - j0) << 16);
+                    d.quads.j0 = (uint16_t)j0; d.quads.n = (uint16_t)(j1 - j0);
                 }
             }
         }
-        e_back = p - p_src;
-        const DevLayer& L = fast ? M.fast_layers[ph.layer] : M.layers[ph.layer];
-        const uint16_t* nw = kind == PH_QKV ? L.attention_norm : kind == PH_W13 ? L.ffn_norm : kind == PH_HEAD ? (fast ? M.fast_norm : M.norm) : nullptr;
-        const unsigned long long out = (unsigned long long)(S > 0 && kind == PH_W2 ? psum_region(M, p, 0) : ll_region(M, tm.team, p, 0));
-        unsigned long long aux = 0ull;
-        if (kind == PH_QKV) aux = (unsigned long long)(fast ? M.fast_rope + (size_t)ph.depth_pos * kHeadDim : M.rope);
-        if (kind == PH_HEAD) {
-            aux = (unsigned long long)(fast ? M.depth_logits + ((size_t)tm.team * M.depth + ph.depth_pos) * M.codebook_size
-                                            : M.token_logits + (size_t)tm.team * M.vocab);
-            nrep = 1;  // logits words are read by the team's sampler CTA only (greedy rows use the candidate words)
-        }
-        const unsigned long long wp = (unsigned long long)(phase_weights(M, ph) + (size_t)i0 * 16 * K);   // 16 K elements per tile
         // normed phases stage the residual stream for everybody (the wo / w2 epilogues need their rows of it); a split
         // staging needs every CTA of the cluster, tiles or not
-        gather = (kind == PH_QKV || kind == PH_W13 || psum == 2) ? 1 : (n_items > 0 ? 1 : 0);
-        w[0] = (uint32_t)src; w[1] = (uint32_t)(src >> 32);
-        w[2] = (uint32_t)(unsigned long long)nw; w[3] = (uint32_t)((unsigned long long)nw >> 32);
-        w[4] = (uint32_t)out; w[5] = (uint32_t)(out >> 32);
-        w[6] = (uint32_t)aux; w[7] = (uint32_t)(aux >> 32);
-        w[8] = (uint32_t)wp; w[9] = (uint32_t)(wp >> 32);
+        if (n_items == 0 && kind != PH_QKV && kind != PH_W13 && d.input != IN_PSUM_SPLIT) d.input = IN_NONE;
+        d.e_back = (uint8_t)(p - p_src);
+        const DevLayer& L = fast ? M.fast_layers[ph.layer] : M.layers[ph.layer];
+        d.normw = kind == PH_QKV ? L.attention_norm : kind == PH_W13 ? L.ffn_norm : kind == PH_HEAD ? (fast ? M.fast_norm : M.norm) : nullptr;
+        d.out = S > 0 && kind == PH_W2 ? psum_region(M, p, 0) : ll_region(M, tm.team, p, 0);
+        if (kind == PH_QKV) d.aux.rope = fast ? M.fast_rope + (size_t)ph.depth_pos * kHeadDim : M.rope;
+        if (kind == PH_HEAD) {
+            d.aux.logits = fast ? M.depth_logits + ((size_t)tm.team * M.depth + ph.depth_pos) * M.codebook_size
+                                : M.token_logits + (size_t)tm.team * M.vocab;
+            d.nrep = 1;  // logits words are read by the team's sampler CTA only (greedy rows use the candidate words)
+        }
+        d.wptr = phase_weights(M, ph) + (size_t)i0 * 16 * K;   // 16 K elements per tile
     }
-    const int res_sel = (kind == PH_QKV || kind == PH_WO) ? 0 : 1;
-    w[10] = (uint32_t)e_back | ((uint32_t)src_kind << 8) | ((uint32_t)nrep << 12) | ((uint32_t)res_sel << 20) | ((uint32_t)gather << 21) |
-            ((uint32_t)psum << 22);
-    w[11] = (uint32_t)K | ((uint32_t)n_items << 16);
-    w[12] = (uint32_t)kind | ((uint32_t)(fast ? 1 : 0) << 4) | ((uint32_t)ph.layer << 8) | ((uint32_t)ph.depth_pos << 16);
-    w[13] = (uint32_t)i0;
-    w[15] = (uint32_t)(S > 0 && kind == PH_W2 ? kNW * M.dim : M.ll_len[p]) | ((uint32_t)n_src << 16);
-#pragma unroll
-    for (int i = 0; i < kDescWords / 4; ++i) sts_v4(dsc + 16u * i, make_uint4(w[4 * i], w[4 * i + 1], w[4 * i + 2], w[4 * i + 3]));
+    store_desc(dsc, d);
 }
 // ring stages of a tile: K in chunks of kLL2ChunkKb k-blocks
 __device__ __forceinline__ int phase_chunks(int K) { return (K / 32 + kLL2ChunkKb - 1) / kLL2ChunkKb; }
@@ -386,21 +423,20 @@ __device__ __noinline__ void producer(const CallArgs& A, const SmemPlan& SP, uin
     uint32_t stage = 0, slot = 0, par = 0;   // stages are produced strictly in order: slot / parity run along
     for (int it = 0; it < A.n_iter; ++it) {
         for (int p = 0; p < A.phase_end; ++p) {
-            const uint32_t dsc = sm0 + (uint32_t)SP.desc + (uint32_t)p * (kDescWords * 4u);
-            const uint4 d2 = lds_v4(dsc + 32u), d3 = lds_v4(dsc + 48u);
-            const int kind = (int)(d3.x & 15u);
-            const int n_items = (int)(d2.w >> 16), K = (int)(d2.w & 0xffffu);
-            const bool units = kind == PH_W2 && d3.z != 0u;   // fused MLP: the K-slice of each of this CTA's w2 row tiles
+            PhaseDesc d;
+            load_desc_head(sm0 + (uint32_t)SP.desc + (uint32_t)(p * sizeof(PhaseDesc)), d);
+            const int kind = d.kind;
+            const int n_items = d.n_items, K = d.K;
+            const bool units = kind == PH_W2 && d.mlp.n_units != 0;   // fused MLP: the K-slice of each of this CTA's w2 row tiles
             if (kind == PH_ATTN || kind == PH_SAMPLE || (n_items == 0 && !units)) continue;
-            const bool fast = (d3.x >> 4) & 1u;
-            const unsigned char* wp = reinterpret_cast<const unsigned char*>((unsigned long long)d2.x | ((unsigned long long)d2.y << 32));
+            const unsigned char* wp = reinterpret_cast<const unsigned char*>(d.wptr);
             // the slow transformer's weights are read once per frame: evict first; the depth transformer's are re-read
             // by every depth step: keep them in L2
-            const uint64_t pol = (fast && kind != PH_HEAD) ? pol_keep : pol_stream;
+            const uint64_t pol = (d.fast && kind != PH_HEAD) ? pol_keep : pol_stream;
             const int tiles = n_items, chunks = phase_chunks(K), kb = K / 32;
             const size_t tile_bytes = (size_t)K * 32;
             if (units) {   // one stage per (row tile, slice): k-blocks lo .. hi - 1 of tiles i0, i0 + S, ..
-                const int lo = (int)(d3.z & 255u), hi = (int)((d3.z >> 8) & 255u), nu = (int)(d3.z >> 16);
+                const int lo = d.mlp.lo, hi = d.mlp.hi, nu = d.mlp.n_units;
                 const uint32_t bytes = (uint32_t)((hi - lo) * 1024);
                 for (int u = 0; u < nu; ++u) {
                     if (stage >= ns) mbar_wait(empty0 + 8u * slot, par ^ 1u);
@@ -611,7 +647,7 @@ __device__ __noinline__ float gather_psum(const unsigned long long* src, int K, 
     return ss;
 }
 
-// The same staging shared by the S CTAs of a slice cluster (psum == 2): the CTA of cluster rank r polls only the quads
+// The same staging shared by the S CTAs of a slice cluster (IN_PSUM_SPLIT): the CTA of cluster rank r polls only the quads
 // [j0, j0 + nq) = [q r / S, q (r + 1) / S) of the vector (q = K / 4; thread 2 j + h: elements 4 (j0 + j) + 2 h, + 1, all 7
 // partials in flight together), computes them exactly as gather_psum does and sends each quad (8 bytes, st.async) to its
 // place in dst (and dst2) of every CTA of the cluster, itself included.  Everybody then waits on s_psumbar (K * 2 bytes
@@ -627,11 +663,11 @@ __device__ __noinline__ float gather_psum(const unsigned long long* src, int K, 
 //    next MLP's partials, which need this CTA's act values of that MLP, sent after the wait below.  So one barrier phase
 //    per staging, with the parity carried by the caller.
 __device__ __noinline__ float gather_psum_split(const unsigned long long* src, int K, uint32_t e_src, uint32_t dst, uint32_t dst2,
-                                                uint32_t resh, uint32_t quads, int S, uint32_t parity) {
+                                                uint32_t resh, int j0, int n_quads, int S, uint32_t parity) {
     const int tid = threadIdx.x, lane = tid & 31;
     const uint32_t bar = smem_u32(&s_psumbar);
     if (tid == 0) mbar_expect_tx(bar, (uint32_t)K * (dst2 ? 4u : 2u));
-    const int j0 = (int)(quads & 0xffffu), n2 = 2 * (int)(quads >> 16);
+    const int n2 = 2 * n_quads;
     if ((tid & ~31) < n2) {   // the warps that hold a quad (n2 is even: both halves of a quad are in one warp)
         const bool mine = tid < n2;
         const int e = 4 * j0 + 2 * tid;
@@ -684,12 +720,12 @@ __device__ __noinline__ float gather_psum_split(const unsigned long long* src, i
 
 // The two inputs that are not LL regions: the token embedding of the pending column (slow layer 0, P:205-221; the frame
 // boundary is taken here) and the embedding of the previous depth code (G:136-140).  Returns the thread's sum of squares.
-__device__ __noinline__ float stage_embedding(const DevModel& M, const CallArgs& A, const Team tm, int src_kind, int it, int p, uint32_t epoch,
+__device__ __noinline__ float stage_embedding(const DevModel& M, const CallArgs& A, const Team tm, int input, int it, int p, uint32_t epoch,
                                               int per_iter, int depth_pos, int K, const uint16_t* emb_base, uint32_t xb, uint32_t res) {
     const int tid = threadIdx.x;
     float ss = 0.f;
     uint4 v = make_uint4(0u, 0u, 0u, 0u);
-    if (src_kind == 0) {   // (the frame boundary was taken by the caller)
+    if (input == IN_TOKEN_EMBEDDING) {   // (the frame boundary was taken by the caller)
         if (tid < K / 8) v = embed_chunk(M, tid);
     } else {
         const int r = depth_pos;  // row of depth code depth_pos - 1
@@ -1283,6 +1319,46 @@ __device__ __forceinline__ void tile_pass_long(int kb, int chunks, int warp, int
     }
 }
 
+// Fused MLP, w2 part (after the W13 phase's tile passes, with the W2 phase's descriptor `w2`): once the slice's act values
+// have arrived from every CTA of the cluster, one warp per row tile replays warp `slice`'s MMA chain of the unfused K sweep
+// (k-blocks lo .. hi - 1, one ring stage) and publishes the tile's fp32 partials with the W2 phase's epoch.
+__device__ __forceinline__ void fused_w2(const PhaseDesc& w2, int S, int slice, int D, uint32_t epoch, int warp, int lane,
+                                         uint32_t full0, uint32_t empty0, uint32_t ring, uint32_t ns, uint32_t act,
+                                         uint32_t& cslot, uint32_t& cpar, uint32_t& act_par) {
+    const int nu = w2.mlp.n_units, nkb = w2.mlp.hi - w2.mlp.lo, c = lane & 3;
+    mbar_wait(smem_u32(&s_actbar), act_par);   // the slice's act values from every CTA of the cluster
+    act_par ^= 1u;
+#pragma unroll 1
+    for (int u = warp; u < nu; u += kNW) {
+        uint32_t sl = cslot + (uint32_t)u, pr = cpar;
+        while (sl >= ns) { sl -= ns; pr ^= 1u; }
+        mbar_wait(full0 + 8u * sl, pr);
+        const uint32_t ab = ring + sl * (uint32_t)kLL2SlotBytes + (uint32_t)lane * 16u, xb = act + (uint32_t)c * 16u;
+        float acc[4] = {0.f, 0.f, 0.f, 0.f}, acd[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll 1
+        for (int j = 0; j < nkb; ++j) {
+            const uint4 bx = lds_v4(xb + (uint32_t)j * 64u);
+            const uint4 a0 = lds_v4(ab + (uint32_t)j * 1024u), a1 = lds_v4(ab + (uint32_t)j * 1024u + 512u);
+            mma_bf16_16816(acc, a0.x, a0.y, a0.z, a0.w, bx.x, bx.y);
+            mma_bf16_16816(acd, a1.x, a1.y, a1.z, a1.w, bx.z, bx.w);
+        }
+        __syncwarp();
+        if (lane == 0) mbar_arrive_n(empty0 + 8u * sl, (uint32_t)kNW);   // the stage's only consumer
+        // partials of row slots g (acc[0] + acd[0]) and g + 8 (acc[2] + acd[2]), held by the lanes with c == 0:
+        // lane l publishes row slot l & 15 to replicas l >> 4, + 2, + 4, + 6
+        const float q0 = __fadd_rn(acc[0], acd[0]), q1 = __fadd_rn(acc[2], acd[2]);
+        const int rs = lane & 15;
+        const float qa = __shfl_sync(0xffffffffu, q0, (rs & 7) * 4), qb = __shfl_sync(0xffffffffu, q1, (rs & 7) * 4);
+        const uint32_t pv = __float_as_uint(rs < 8 ? qa : qb);
+        unsigned long long* o = w2.out + (size_t)(lane >> 4) * w2.len_out + slice * D + (w2.i0 + u * S) * 16 + rs;   // i0 = first row tile
+#pragma unroll
+        for (int i = 0; i < kLLRep / 2; ++i, o += 2 * (size_t)w2.len_out) st_relaxed_v2(o, pv, epoch);
+    }
+    uint32_t sl = cslot + (uint32_t)nu;
+    while (sl >= ns) { sl -= ns; cpar ^= 1u; }
+    cslot = sl;
+}
+
 template <bool kTrace>
 __global__ void __launch_bounds__(kLL2Threads, 1)
 smol_ll2_kernel(const __grid_constant__ DevModel M, const __grid_constant__ CallArgs A, const __grid_constant__ SmemPlan SP) {
@@ -1323,7 +1399,7 @@ smol_ll2_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Call
             s_best = 0u;
         }
         if (tid < M.n_rows) { s_tok[tid] = ldcg_i32(sq.tokens + tid); s_nw[tid] = 0; }
-        for (int p = tid; p < per_iter; p += kLL2Threads) build_desc(M, tm, A.mlp_cluster, A.psum_split, p, DSC0 + (uint32_t)p * (kDescWords * 4u));
+        for (int p = tid; p < per_iter; p += kLL2Threads) build_desc(M, tm, A.mlp_cluster, p, DSC0 + (uint32_t)(p * sizeof(PhaseDesc)));
         for (int i = tid; i < kBtabCache && i < A.b.max_pages; i += kLL2Threads) s_btab[i] = ldcg_i32(sq.btab + i);
     }
     __syncthreads();
@@ -1359,15 +1435,16 @@ smol_ll2_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Call
         int step = 1;
 #pragma unroll 1
         for (int p = 0; p < per_iter; p += step) {
-            const uint32_t dsc = DSC0 + (uint32_t)p * (kDescWords * 4u);
+            const uint32_t dsc = DSC0 + (uint32_t)(p * sizeof(PhaseDesc));
             const uint32_t epoch = s_epoch0 + (uint32_t)(it * per_iter + p) + 1u;
-            const uint4 d2 = lds_v4(dsc + 32u), d3 = lds_v4(dsc + 48u);
-            const int kind = (int)(d3.x & 15u);
+            PhaseDesc d;
+            load_desc_head(dsc, d);
+            const int kind = d.kind;
             // fused MLP: a W13 phase is always followed by its W2 phase, whose work it does -- the consumer warps skip that
-            // phase (no descriptor, no barrier; t_end stays the W13 phase's end)
+            // phase (no barrier; t_end stays the W13 phase's end)
             step = (A.mlp_cluster > 0 && kind == PH_W13) ? 2 : 1;
-            const bool fast = (d3.x >> 4) & 1u;
-            const int layer = (int)((d3.x >> 8) & 255u), depth_pos = (int)((d3.x >> 16) & 255u);
+            const bool fast = d.fast != 0;
+            const int layer = d.layer, depth_pos = d.depth_pos;
             LL2_TRACE(0);
             if (kind == PH_ATTN) {
                 phase_attn(M, A, tm, layer, p, epoch, SCR, SP.holdoff);
@@ -1382,30 +1459,20 @@ smol_ll2_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Call
                 continue;
             }
             // ================= a phase that streams weights =================
-            const uint4 d0 = lds_v4(dsc), d1 = lds_v4(dsc + 16u);
-            const int K = (int)(d2.w & 0xffffu), n_items = (int)(d2.w >> 16);
+            load_desc_tail(dsc, d);
+            const int K = d.K, n_items = d.n_items, i0 = d.i0;
             const int kb = K >> 5;
-            const int src_kind = (int)((d2.z >> 8) & 15u), nrep = (int)((d2.z >> 12) & 63u);
-            const bool do_gather = (d2.z >> 21) & 1u;
-            const uint32_t psum = (d2.z >> 22) & 3u;   // input: a fused MLP's partial sums (1: gather_psum, 2: gather_psum_split)
-            const uint32_t e_src = epoch - (d2.z & 255u);
-            const uint32_t res = ((d2.z >> 20) & 1u) ? RESH : RESX;
+            const uint32_t e_src = epoch - (uint32_t)d.e_back;
+            const uint32_t res = d.res_h ? RESH : RESX;
             const bool normed = kind == PH_QKV || kind == PH_W13 || kind == PH_HEAD;
-            const unsigned long long* src = reinterpret_cast<const unsigned long long*>((unsigned long long)d0.x | ((unsigned long long)d0.y << 32));
-            const uint16_t* normw = reinterpret_cast<const uint16_t*>((unsigned long long)d0.z | ((unsigned long long)d0.w << 32));
-            unsigned long long* out = reinterpret_cast<unsigned long long*>((unsigned long long)d1.x | ((unsigned long long)d1.y << 32));
-            const unsigned long long aux = (unsigned long long)d1.z | ((unsigned long long)d1.w << 32);
-            const int len_out = (int)(d3.w & 0xffffu), n_src = (int)(d3.w >> 16);
-            const int i0 = (int)d3.y;
-            const uint32_t mlp = kind == PH_W13 ? d3.z : 0u;   // fused MLP: lo | hi << 8 | n_units << 16 (0: unfused)
-            const int mlp_lo = (int)(mlp & 255u), mlp_hi = (int)((mlp >> 8) & 255u);
-            if (mlp != 0u && tid == 0) mbar_expect_tx(smem_u32(&s_actbar), (uint32_t)(mlp_hi - mlp_lo) * 64u);  // the slice's act, bf16
+            const bool mlp = kind == PH_W13 && d.mlp.n_units != 0;   // fused MLP (0 units: unfused, or the idle cluster)
+            if (mlp && tid == 0) mbar_expect_tx(smem_u32(&s_actbar), (uint32_t)(d.mlp.hi - d.mlp.lo) * 64u);  // the slice's act, bf16
 
             const int Hq = fast ? M.fn_head : M.n_head, Hkv = fast ? M.fn_kv : M.n_kv;
             const int q_rows = Hq * kHeadDim, k_end = (Hq + Hkv) * kHeadDim;
             // slow layer 0 of a later frame: adopt the previous frame's ids and advance the position first (the RoPE row
             // prefetched below is the NEW position's)
-            if (src_kind == 0 && it > 0) frame_boundary(M, A, tm, epoch - (uint32_t)per_iter);
+            if (d.input == IN_TOKEN_EMBEDDING && it > 0) frame_boundary(M, A, tm, epoch - (uint32_t)per_iter);
             // Operands that do not depend on the input are loaded NOW (volatile: the compiler must not sink them below the
             // wait): the norm weights of the 4 elements this thread will normalise, and -- in the warp that will reduce the
             // phase's first tile -- the RoPE pair of its row.
@@ -1413,13 +1480,13 @@ smol_ll2_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Call
 #pragma unroll
             for (int q = 0; q < kNormPer; ++q) {
                 nw2[q] = make_uint2(0u, 0u);
-                if (normed && tid + q * kCons < K / 4) nw2[q] = ldnc_v2(normw + 4 * (tid + q * kCons));
+                if (normed && tid + q * kCons < K / 4) nw2[q] = ldnc_v2(d.normw + 4 * (tid + q * kCons));
             }
             uint32_t rope0 = 0u;
             if (kind == PH_QKV && n_items > 0 && warp == (int)(tile_ctr % kNW) && lane < 16) {
                 const int n = i0 * 16 + lane;
                 if (n < k_end) {
-                    const uint16_t* table = reinterpret_cast<const uint16_t*>(aux) + (fast ? 0 : (size_t)min(s_pos, M.max_seq_len - 1) * kHeadDim);
+                    const uint16_t* table = d.aux.rope + (fast ? 0 : (size_t)min(s_pos, M.max_seq_len - 1) * kHeadDim);
                     rope0 = ldnc_u32(table + (n & (kHeadDim - 2)));
                 }
             }
@@ -1427,16 +1494,20 @@ smol_ll2_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Call
 
             // ---- the phase's input vector -> xbuf -----------------------------------------------------------
             float ss = 0.f;
-            if (src_kind != 3) {   // token embedding (slow layer 0) / embedding of the previous depth code: once per frame / depth step
-                ss = stage_embedding(M, A, tm, src_kind, it, p, epoch, per_iter, depth_pos, K, reinterpret_cast<const uint16_t*>(src), XB, res);
-            } else if (do_gather) {
-                if (SP.holdoff > 0) { while (clock32_now() - t_end < (uint32_t)SP.holdoff) {} }
-                if (kind == PH_WO && fast) fast_attention(M, layer, depth_pos, src, e_src, FQ, FKV, XB);
-                else if (psum == 2u) {
-                    ss = gather_psum_split(src, K, e_src, XB, (normed && kind != PH_HEAD) ? res : 0u, RESH, d3.z, A.mlp_cluster, psum_par);
+            if (d.input >= IN_WORDS && SP.holdoff > 0) { while (clock32_now() - t_end < (uint32_t)SP.holdoff) {} }
+            const uint32_t res2 = (normed && kind != PH_HEAD) ? res : 0u;   // normed phases stage the residual stream too
+            switch (d.input) {
+                case IN_TOKEN_EMBEDDING: case IN_CODE_EMBEDDING:   // once per frame / depth step
+                    ss = stage_embedding(M, A, tm, d.input, it, p, epoch, per_iter, depth_pos, K, d.src.emb, XB, res);
+                    break;
+                case IN_WORDS: ss = gather_words(d.src.words, K / 2, e_src, XB, res2); break;
+                case IN_DEPTH_ATTENTION: fast_attention(M, layer, depth_pos, d.src.words, e_src, FQ, FKV, XB); break;
+                case IN_PSUM: ss = gather_psum(d.src.words, K, e_src, XB, res2, RESH); break;
+                case IN_PSUM_SPLIT:
+                    ss = gather_psum_split(d.src.words, K, e_src, XB, res2, RESH, d.quads.j0, d.quads.n, A.mlp_cluster, psum_par);
                     psum_par ^= 1u;
-                } else if (psum == 1u) ss = gather_psum(src, K, e_src, XB, (normed && kind != PH_HEAD) ? res : 0u, RESH);
-                else ss = gather_words(src, n_src, e_src, XB, (normed && kind != PH_HEAD) ? res : 0u);
+                    break;
+                default: break;   // IN_NONE
             }
             LL2_TRACE(1);
             if (normed) {
@@ -1528,7 +1599,7 @@ smol_ll2_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Call
                             if (valid && n < k_end) {  // q and k rows: interleaved-pair RoPE with the bf16 table (P:616-640)
                                 uint32_t cs = rope0;
                                 if (t > 0) {
-                                    const uint16_t* table = reinterpret_cast<const uint16_t*>(aux) + (fast ? 0 : (size_t)min(s_pos, M.max_seq_len - 1) * kHeadDim);
+                                    const uint16_t* table = d.aux.rope + (fast ? 0 : (size_t)min(s_pos, M.max_seq_len - 1) * kHeadDim);
                                     cs = ldnc_u32(table + (n & (kHeadDim - 2)));
                                 }
                                 const float co = bf_lo(cs), si = bf_hi(cs);
@@ -1543,7 +1614,7 @@ smol_ll2_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Call
                             }
                         } else if (kind == PH_HEAD) {
                             if (valid) {
-                                reinterpret_cast<float*>(aux)[n] = val;
+                                d.aux.logits[n] = val;
                                 atomicMax(&s_best, cand_pack(val, n));
                             }
                         }
@@ -1552,24 +1623,24 @@ smol_ll2_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Call
                     const float nxt = __shfl_down_sync(0xffffffffu, val, 1);
                     const uint32_t word = pack_bf16(val, nxt);
                     if (kind == PH_QKV && !fast && valid && !(lane & 1) && n >= q_rows) kv_append(M, A, tm.team, layer, n, word);
-                    if (mlp != 0u) {
+                    if (mlp) {
                         // fused MLP: the tile's 8 act values (16 bytes) into every CTA of the cluster, lane r -> rank r
                         const uint32_t a0 = __shfl_sync(0xffffffffu, word, 0), a1 = __shfl_sync(0xffffffffu, word, 2);
                         const uint32_t a2 = __shfl_sync(0xffffffffu, word, 4), a3 = __shfl_sync(0xffffffffu, word, 6);
                         if (lane < A.mlp_cluster) {
-                            const uint32_t dst = ACT + (uint32_t)(((i0 + t) * 8 - mlp_lo * 32) * 2);
+                            const uint32_t dst = ACT + (uint32_t)(((i0 + t) * 8 - d.mlp.lo * 32) * 2);
                             st_async_v4(mapa(dst, (uint32_t)lane), a0, a1, a2, a3, mapa(smem_u32(&s_actbar), (uint32_t)lane));
                         }
                     } else {
 #pragma unroll
                         for (int rnd = 0; rnd < 2; ++rnd) {
                             const int idx = lane + 32 * rnd;
-                            const int wi = nrep == 1 ? idx : idx >> 3, rp = nrep == 1 ? 0 : idx & 7;
+                            const int wi = d.nrep == 1 ? idx : idx >> 3, rp = d.nrep == 1 ? 0 : idx & 7;
                             const int sl = 2 * (wi & 7);
                             const uint32_t wv = __shfl_sync(0xffffffffu, word, sl);
                             const int wn = __shfl_sync(0xffffffffu, n, sl);
                             const int wok = __shfl_sync(0xffffffffu, valid ? 1 : 0, sl);
-                            if (wi < 8 && wok && (nrep > 1 || rnd == 0)) st_relaxed_v2(out + (size_t)rp * len_out + (wn >> 1), wv, epoch);
+                            if (wi < 8 && wok && (d.nrep > 1 || rnd == 0)) st_relaxed_v2(d.out + (size_t)rp * d.len_out + (wn >> 1), wv, epoch);
                         }
                     }
                 }
@@ -1577,44 +1648,11 @@ smol_ll2_kernel(const __grid_constant__ DevModel M, const __grid_constant__ Call
                 pass_ctr += 1u;
                 t0 += nt;
             }
-            if (mlp != 0u) {
-                // ---- fused MLP, w2 part: one warp per row tile replays warp `slice`'s MMA chain of the unfused K sweep ------
-                const int nu = (int)(mlp >> 16), nkb = mlp_hi - mlp_lo, S = A.mlp_cluster, slice = tm.cta / S;
-                const uint32_t dw = dsc + (uint32_t)(kDescWords * 4);   // the W2 phase's descriptor: region, row tile i0
-                const uint4 w1 = lds_v4(dw + 16u), w3 = lds_v4(dw + 48u);
-                unsigned long long* out2 = reinterpret_cast<unsigned long long*>((unsigned long long)w1.x | ((unsigned long long)w1.y << 32));
-                const int len2 = (int)(w3.w & 0xffffu), D = (fast ? M.fdim : M.dim);
-                mbar_wait(smem_u32(&s_actbar), mlp_par);   // the slice's act values from every CTA of the cluster
-                mlp_par ^= 1u;
-#pragma unroll 1
-                for (int u = warp; u < nu; u += kNW) {
-                    uint32_t sl = cslot + (uint32_t)u, pr = cpar;
-                    while (sl >= NSLOTS) { sl -= NSLOTS; pr ^= 1u; }
-                    mbar_wait(full0 + 8u * sl, pr);
-                    const uint32_t ab = RING + sl * (uint32_t)kLL2SlotBytes + (uint32_t)lane * 16u, xb = ACT + (uint32_t)c * 16u;
-                    float acc[4] = {0.f, 0.f, 0.f, 0.f}, acd[4] = {0.f, 0.f, 0.f, 0.f};
-#pragma unroll 1
-                    for (int j = 0; j < nkb; ++j) {
-                        const uint4 bx = lds_v4(xb + (uint32_t)j * 64u);
-                        const uint4 a0 = lds_v4(ab + (uint32_t)j * 1024u), a1 = lds_v4(ab + (uint32_t)j * 1024u + 512u);
-                        mma_bf16_16816(acc, a0.x, a0.y, a0.z, a0.w, bx.x, bx.y);
-                        mma_bf16_16816(acd, a1.x, a1.y, a1.z, a1.w, bx.z, bx.w);
-                    }
-                    __syncwarp();
-                    if (lane == 0) mbar_arrive_n(empty0 + 8u * sl, (uint32_t)kNW);   // the stage's only consumer
-                    // partials of row slots g (acc[0] + acd[0]) and g + 8 (acc[2] + acd[2]), held by the lanes with c == 0:
-                    // lane l publishes row slot l & 15 to replicas l >> 4, + 2, + 4, + 6
-                    const float q0 = __fadd_rn(acc[0], acd[0]), q1 = __fadd_rn(acc[2], acd[2]);
-                    const int rs = lane & 15;
-                    const float qa = __shfl_sync(0xffffffffu, q0, (rs & 7) * 4), qb = __shfl_sync(0xffffffffu, q1, (rs & 7) * 4);
-                    const uint32_t pv = __float_as_uint(rs < 8 ? qa : qb);
-                    unsigned long long* o = out2 + slice * D + ((int)w3.y + u * S) * 16 + rs;   // w3.y = first row tile
-#pragma unroll
-                    for (int i = 0; i < kLLRep / 2; ++i) st_relaxed_v2(o + (size_t)((lane >> 4) + 2 * i) * len2, pv, epoch + 1u);
-                }
-                uint32_t sl = cslot + (uint32_t)nu;
-                while (sl >= NSLOTS) { sl -= NSLOTS; cpar ^= 1u; }
-                cslot = sl;
+            if (mlp) {   // the W2 phase's row tiles, from its descriptor's head
+                PhaseDesc w2;
+                load_desc_head(dsc + (uint32_t)sizeof(PhaseDesc), w2);
+                fused_w2(w2, A.mlp_cluster, tm.cta / A.mlp_cluster, fast ? M.fdim : M.dim, epoch + 1u, warp, lane, full0, empty0, RING,
+                         NSLOTS, ACT, cslot, cpar, mlp_par);
             }
             if (kind == PH_HEAD && M.force == nullptr && (fast ? s_rs.fast_temp : s_rs.temp) == 0.0f) {
                 // greedy row: the CTA's best (logit, index) goes out as one word per replica
@@ -1670,7 +1708,7 @@ struct LL2Plan {
 };
 
 // Shared-memory plan; smem == 0: this model does not fit the kernel.
-bool ll2_plan(const DevModel& M, int holdoff, int flags, ll2::SmemPlan* sp, size_t* smem) {
+bool ll2_plan(const DevModel& M, int holdoff, ll2::SmemPlan* sp, size_t* smem) {
     auto up = [](size_t v) { return (v + 127) / 128 * 128; };
     if (M.depth > kLL2Depth || M.n_rows > kMaxRows) return false;
     if (M.dim != M.fdim) return false;
@@ -1687,7 +1725,7 @@ bool ll2_plan(const DevModel& M, int holdoff, int flags, ll2::SmemPlan* sp, size
     sp->res_x = take((size_t)M.dim * 2);
     sp->res_h = take((size_t)M.dim * 2);
     sp->part = take((size_t)2 * 4 * ll2::kNW * 16 * 4);
-    sp->desc = take((size_t)phases_per_frame(M.n_layer, M.n_flayer, M.depth) * ll2::kDescWords * 4);
+    sp->desc = take((size_t)phases_per_frame(M.n_layer, M.n_flayer, M.depth) * sizeof(ll2::PhaseDesc));
     sp->fq = take((size_t)M.fdim * 2);
     sp->fkv = take((size_t)M.n_flayer * kLL2Depth * 2 * M.fn_kv * kHeadDim * 2);
     const int nl = M.vocab > M.codebook_size ? M.vocab : M.codebook_size;
@@ -1705,7 +1743,6 @@ bool ll2_plan(const DevModel& M, int holdoff, int flags, ll2::SmemPlan* sp, size
     if (n_slots > ll2::kMaxSlots) n_slots = ll2::kMaxSlots;
     sp->n_slots = n_slots;
     sp->holdoff = holdoff;
-    sp->flags = flags;
     *smem = off + (size_t)n_slots * kLL2SlotBytes;
     return true;
 }

@@ -21,7 +21,7 @@ ncu --metrics gpu__time_duration.sum,dram__bytes_read.sum,dram__bytes_write.sum 
 timeout 300 python tools/phase_profile.py --batch 256 --frames 16 --prompt-bytes 64 > $O/${T}_phase_bs256.log 2>&1
 timeout 300 python tools/phase_profile.py --batch 256 --frames 16 --prompt-bytes 400 > $O/${T}_phase_bs256_L420.log 2>&1
 timeout 300 python tools/phase_profile.py --batch 64 --frames 16 --sampled > $O/${T}_phase_bs64_sampled.log 2>&1
-timeout 400 python tools/ll2_probe.py --skip-check --holdoffs 400 --staggers 0 > $O/${T}_probe.log 2>&1
+timeout 400 python tools/ll2_probe.py --skip-check --holdoffs 400 > $O/${T}_probe.log 2>&1
 timeout 400 python tools/ll2_probe.py --skip-check --skip-timing --teams > $O/${T}_teams.log 2>&1
 # Mimi streaming decoder (the step after the path): step times, launch lists, DRAM bytes of a step, ncu of the row / tile kernels,
 # streaming and serving through both engines

@@ -103,14 +103,11 @@ def timing(args):
         return e0.elapsed_time(e1) * 1e3 / n
 
     for h in [int(h) for h in args.holdoffs.split(",")]:
-        for st in [int(x) for x in args.staggers.split(",")]:
-            model.set_option("ll_holdoff", h)
-            model.set_option("ll_flags", st)
-            run(8)
-            us = [run(args.frames) for _ in range(3)]
-            codes = int(batch.out_codes.sum().item())
-            print(f"holdoff={h:5d} stagger={st:4d} cycles: {min(us):8.1f} us/frame (runs {', '.join(f'{u:.1f}' for u in us)}) check={codes}")
-    model.set_option("ll_flags", args.trace_stagger)
+        model.set_option("ll_holdoff", h)
+        run(8)
+        us = [run(args.frames) for _ in range(3)]
+        codes = int(batch.out_codes.sum().item())
+        print(f"holdoff={h:5d} cycles: {min(us):8.1f} us/frame (runs {', '.join(f'{u:.1f}' for u in us)}) check={codes}")
     model.set_option("ll_holdoff", args.trace_holdoff)
     for n in [int(x) for x in args.n_ctas.split(",") if x]:
         model.set_option("n_ctas", n)
@@ -118,17 +115,15 @@ def timing(args):
         us = [run(args.frames) for _ in range(2)]
         print(f"n_ctas={n:4d}: {min(us):8.1f} us/frame")
     model.set_option("n_ctas", 0)
-    # the fused gated MLP (clusters, DSMEM) with split / per-CTA staging of its partial sums, against the unfused program
-    for fused, split in ((1, 1), (1, 0), (0, 1), (1, 1)):
+    # the fused gated MLP (clusters, DSMEM) against the unfused program
+    for fused in (1, 0, 1):
         model.set_option("ll_fused_mlp", fused)
-        model.set_option("ll_psum_split", split)
         run(8)
         us = [run(args.frames) for _ in range(2)]
-        print(f"ll_fused_mlp={fused} ll_psum_split={split} (ran fused: {model.get_option('ll_last_fused')}, split: "
-              f"{model.get_option('ll_last_split')}, cluster {model.get_option('ll_mlp_cluster')} x {model.get_option('ll_mlp_clusters')}, "
+        print(f"ll_fused_mlp={fused} (ran fused: {model.get_option('ll_last_fused')}, "
+              f"cluster {model.get_option('ll_mlp_cluster')} x {model.get_option('ll_mlp_clusters')}, "
               f"grid {model.get_option('ll_mlp_cluster') * model.get_option('ll_mlp_clusters')}): {min(us):8.1f} us/frame")
     model.set_option("ll_fused_mlp", args.trace_fused)
-    model.set_option("ll_psum_split", args.trace_split)
     # cycle trace at the default hold-off
     model.set_option("ll_holdoff", args.trace_holdoff)
     run(8)
@@ -244,10 +239,7 @@ def main():
     ap.add_argument("--prompt-bytes", type=int, default=200)
     ap.add_argument("--holdoffs", default="0,200,400,600,800")
     ap.add_argument("--trace-holdoff", type=int, default=400)
-    ap.add_argument("--staggers", default="0,250,350")
-    ap.add_argument("--trace-stagger", type=int, default=0)
     ap.add_argument("--trace-fused", type=int, default=1, help="ll_fused_mlp of the cycle / skew trace")
-    ap.add_argument("--trace-split", type=int, default=1, help="ll_psum_split of the cycle / skew trace")
     ap.add_argument("--n-ctas", default="", help="comma list of grid sizes to time")
     ap.add_argument("--skip-check", action="store_true")
     ap.add_argument("--skip-timing", action="store_true")

@@ -23,7 +23,6 @@ def main():
     ap.add_argument("--prompt-bytes", type=int, default=200)
     ap.add_argument("--mode", type=int, default=2)
     ap.add_argument("--n-ctas", type=int, default=0)
-    ap.add_argument("--flags", type=int, nargs="*", default=[0], help="values of the engine option \"ll_flags\" to A/B (a spare switch word the data-flow kernel receives in its shared-memory plan; the shipped kernel ignores it)")
     a = ap.parse_args()
     cfg = named_config(a.model)
     need = a.prompt_bytes + 12 + 2 * a.frames + 16
@@ -39,19 +38,16 @@ def main():
     model.prefill(batch, padded, lens)          # launch 0
     tokens0, len0 = batch.tokens.clone(), batch.seq_len.clone()
     host_len0 = list(batch.host_len)
-    for rnd in range(2 if len(a.flags) > 1 else 1):
-        for fl in a.flags:
-            model.set_option("ll_flags", fl)
-            batch.tokens.copy_(tokens0); batch.seq_len.copy_(len0); batch.step.zero_(); batch.host_len = list(host_len0)
-            model.decode_frames(batch, s, a.frames)     # launch 1 (warm)
-            torch.cuda.synchronize()
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record()
-            model.decode_frames(batch, s, a.frames)     # launch 2 (captured)
-            e1.record()
-            torch.cuda.synchronize()
-            print(f"{a.model} mode={a.mode} flags={fl}: {e0.elapsed_time(e1) * 1e3 / a.frames:.1f} us/frame over {a.frames} frames; "
-                  f"codes checksum {int(batch.out_codes.sum().item())}")
+    batch.tokens.copy_(tokens0); batch.seq_len.copy_(len0); batch.step.zero_(); batch.host_len = list(host_len0)
+    model.decode_frames(batch, s, a.frames)     # launch 1 (warm)
+    torch.cuda.synchronize()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    model.decode_frames(batch, s, a.frames)     # launch 2 (captured)
+    e1.record()
+    torch.cuda.synchronize()
+    print(f"{a.model} mode={a.mode}: {e0.elapsed_time(e1) * 1e3 / a.frames:.1f} us/frame over {a.frames} frames; "
+          f"codes checksum {int(batch.out_codes.sum().item())}")
 
 
 if __name__ == "__main__":
