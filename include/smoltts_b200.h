@@ -218,8 +218,21 @@ int64_t smol_get_option(const SmolModel* m, const char* name);
 /* Introspection for parity tests and benchmarks. name: "x" (slow stream [B,D] bf16), "h" [B,D] bf16,
  * "xf" (fast stream [B,Df] bf16), "q" [B,H*64] bf16, "attn" [B,D] bf16, "act" [B,F] bf16, "fkv"
  * [B,Lf,2,depth,Hkv*64] bf16, "token_logits" [B,V] f32, "depth_logits" [B,Nf,C] f32,
- * "frame_tokens" [B,R] i32. Returns NULL if unknown. */
+ * "frame_tokens" [B,R] i32.  Word regions of the data-flow kernel (mode 2): every word is 8 bytes {uint32 payload,
+ * uint32 epoch}, payload first; epoch 0 = never written, and every phase a launch runs gets an epoch no earlier launch used:
+ *   "ll"        phase p, sequence b, replica r (of 8): words ll + off[p] + (b * 8 + r) * len[p] (smol_ll_region), regions
+ *               for 8 sequences; a payload is two bf16 values, the lower element in the low half (QKV: q | k | v after
+ *               RoPE, ATTN: attention output, WO: h, W13: act, W2: layer output, HEAD: logits; SAMPLE phases have none);
+ *   "ll_epoch"  uint32 [0] = phases run by all earlier launches: phase p of the last frame of a launch carried
+ *               epoch ll_epoch - phase_count + p + 1 (read after the launch);
+ *   "ll2_score" fp32 q.k / 8 attention scores of the slow layers [8 sequences][layer % 2][n_head][len] words,
+ *               len = max_seq_len rounded up to 512;
+ *   "ll2_psum"  fp32 partial sums of the batch-1 fused MLP [W2 phase][8 replicas][7 K-slices][dim] words, W2 phases
+ *               numbered slow layers first, then depth position x fast layer.
+ * Returns NULL if unknown. */
 void* smol_debug_buffer(SmolModel* m, const char* name);
+/* Word offset and length (words per sequence and replica) of phase `phase`'s region in the "ll" debug buffer. */
+int smol_ll_region(const SmolModel* m, int32_t phase, uint32_t* word_offset, uint32_t* words);
 /* Kernel launches issued for one frame in the current mode (mode 0: one launch covers all the
  * frames of a call). */
 int32_t smol_launches_per_frame(const SmolModel* m);

@@ -144,6 +144,7 @@ PROTOTYPES = {
     "smol_set_option": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int64]),
     "smol_get_option": (C.c_int64, [C.c_void_p, C.c_char_p]),
     "smol_debug_buffer": (C.c_void_p, [C.c_void_p, C.c_char_p]),
+    "smol_ll_region": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
     "smol_launches_per_frame": (C.c_int32, [C.c_void_p]),
     "smol_launch_count": (C.c_int64, [C.c_void_p]),
     # include/smoltts_b200_mimi.h

@@ -879,7 +879,19 @@ void* smol_debug_buffer(SmolModel* m, const char* name) {
     if (!std::strcmp(name, "token_logits")) return d.token_logits;
     if (!std::strcmp(name, "depth_logits")) return d.depth_logits;
     if (!std::strcmp(name, "frame_tokens")) return d.frame_tokens;
+    if (!std::strcmp(name, "ll")) return d.ll;
+    if (!std::strcmp(name, "ll_epoch")) return d.ll_epoch;
+    if (!std::strcmp(name, "ll2_score")) return d.ll2_score;
+    if (!std::strcmp(name, "ll2_psum")) return d.ll2_psum;
     return nullptr;
+}
+
+int smol_ll_region(const SmolModel* m, int32_t phase, uint32_t* word_offset, uint32_t* words) {
+    if (!m || !word_offset || !words) return fail(SMOL_ERR_INVALID, "smol_ll_region: null argument");
+    if (phase < 0 || phase >= smol_phase_count(m)) return fail(SMOL_ERR_INVALID, "smol_ll_region: phase outside the frame's program");
+    *word_offset = m->dm.ll_off[phase];
+    *words = m->dm.ll_len[phase];
+    return SMOL_OK;
 }
 
 int32_t smol_launches_per_frame(const SmolModel* m) {

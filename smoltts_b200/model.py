@@ -60,6 +60,16 @@ class TokenConfig:
                    semantic_end_id=TOK_SEMANTIC0 + config.codebook_size - 1)
 
 
+LL_REPLICAS = 8      # replicas of every word region (dev_model.h: kLLRep)
+LL_PSUM_SLICES = 7   # K-slices of the fused MLP's partial sums (dev_model.h: kLL2Warps)
+
+
+def ll_bf16(payload: torch.Tensor) -> torch.Tensor:
+    """Payloads of bf16 words (int32 [n]) -> their 2n bf16 values, the low half of each word first (pack_bf16; both the
+    device and the host are little-endian)."""
+    return payload.contiguous().view(torch.bfloat16)
+
+
 def precompute_freqs_cis(seq_len: int, n_elem: int, base: float) -> torch.Tensor:
     """[seq_len, n_elem/2, 2] (cos, sin) rounded to bf16 -- same op sequence as the reference
     (modeling/model/rq_transformer.py:616-624) so the table is bit-identical."""
@@ -452,6 +462,54 @@ class RQTransformer:
         nbytes = n * torch.empty((), dtype=dtype).element_size()
         start = self._ws_ptr - self._workspace.data_ptr() + off
         return self._workspace[start:start + nbytes].view(dtype).view(*shape)[:B]
+
+    # ---- word regions of the data-flow kernel (include/smoltts_b200.h: smol_debug_buffer "ll", "ll2_score", ..)
+    def _words(self, name: str, word_offset: int, n_words: int) -> Tuple[torch.Tensor, torch.Tensor]:
+        """(payload, epoch) int32 views [n_words] of 8-byte words of the named buffer, starting at word `word_offset`."""
+        ptr = self.lib.smol_debug_buffer(self._h, name.encode())
+        if not ptr:
+            raise KeyError(name)
+        start = ptr - self._workspace.data_ptr() + 8 * word_offset
+        w = self._workspace[start:start + 8 * n_words].view(torch.int32).view(n_words, 2)
+        return w[:, 0], w[:, 1]
+
+    def ll_region(self, phase: int) -> Tuple[int, int]:
+        """(word offset, words per sequence and replica) of phase `phase`'s region."""
+        off, n = C.c_uint32(), C.c_uint32()
+        _capi.check(self.lib.smol_ll_region(self._h, int(phase), C.byref(off), C.byref(n)))
+        return int(off.value), int(n.value)
+
+    def ll_words(self, phase: int, team: int = 0, rep: int = 0) -> Tuple[torch.Tensor, torch.Tensor]:
+        """(payload, epoch) int32 views [len] of phase `phase`'s words: sequence (team) `team`, replica `rep`."""
+        off, n = self.ll_region(phase)
+        return self._words("ll", off + (team * LL_REPLICAS + rep) * n, n)
+
+    def ll_epoch(self) -> int:
+        """Phases run by every data-flow launch so far: phase p of a launch's last frame carried ll_epoch() - phase_count + p + 1."""
+        return int(self._words("ll_epoch", 0, 1)[0].item())
+
+    def ll_scores(self, team: int, layer: int) -> Tuple[torch.Tensor, torch.Tensor]:
+        """(fp32 q.k / 8 scores, epoch) [n_head, score_len] of slow layer `layer` (its parity's buffer: the last two layers
+        of a frame are kept)."""
+        H = self.config.n_head
+        n = (self.max_seq_len + 511) // 512 * 512   # capi.cu: ll2_score_len
+        pay, ep = self._words("ll2_score", (team * 2 + layer % 2) * H * n, H * n)
+        return pay.view(torch.float32).view(H, n), ep.view(H, n)
+
+    def ll_psums(self, phase: int, rep: int = 0) -> Tuple[torch.Tensor, torch.Tensor]:
+        """(fp32 partial sums, epoch) [7 K-slices, dim] of the fused MLP's W2 phase `phase` (batch 1), replica `rep`."""
+        cfg = self.config
+        n_slow, per = 5 * cfg.n_layer, 4 * cfg.n_fast_layer + 2
+        depth_pos, r = divmod(phase - n_slow - 2, per)   # fast phases: depth position, phase inside the depth step
+        if 0 <= phase < n_slow and phase % 5 == 4:
+            w2 = phase // 5
+        elif phase >= n_slow + 2 and r < 4 * cfg.n_fast_layer and r % 4 == 3:
+            w2 = cfg.n_layer + depth_pos * cfg.n_fast_layer + r // 4
+        else:
+            raise ValueError(f"phase {phase} is not a W2 phase")
+        n = LL_PSUM_SLICES * cfg.dim
+        pay, ep = self._words("ll2_psum", (w2 * LL_REPLICAS + rep) * n, n)
+        return pay.view(torch.float32).view(LL_PSUM_SLICES, cfg.dim), ep.view(LL_PSUM_SLICES, cfg.dim)
 
     def kv_view(self) -> torch.Tensor:
         """[n_pages, n_layer, 2, n_kv, page_size, 64] bf16 view of the paged pool."""

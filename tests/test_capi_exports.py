@@ -4,6 +4,8 @@ import ctypes
 import os
 import re
 
+import pytest
+
 from conftest import ROOT
 
 
@@ -60,6 +62,45 @@ def test_create_validates_shapes_without_a_gpu():
     assert lib.smol_create(ctypes.byref(make(fast_dim=512, fast_n_head=8)), ctypes.byref(h2)) == _capi.SMOL_ERR_UNSUPPORTED
     assert b"fast_project_in" in lib.smol_last_error()
     assert lib.smol_create(ctypes.byref(make(head_dim=128)), ctypes.byref(h2)) == _capi.SMOL_ERR_UNSUPPORTED
+
+
+@pytest.mark.parametrize("size,overrides", [("smoltts_byte_tiny", {}), ("smoltts_byte_70m", {}), ("smoltts_byte_150m", {}),
+                                            ("smoltts_byte_tiny", {"duplicate_code_0": False})])
+def test_ll_regions_follow_the_frame_program(size, overrides):
+    """smol_ll_region (host code: smol_create alone) against a restatement of ll_phase_words / decode_phase: one region per
+    phase, laid end to end for 8 sequences x 8 replicas, inside the workspace."""
+    from ll2_checks import decode_phase, phase_count, phase_words
+    from smoltts_b200 import _capi
+    from smoltts_b200.config import named_config
+
+    lib = _capi.load()
+    cfg = named_config(size, **overrides)
+    c = _capi.SmolConfig(
+        dim=cfg.dim, n_layer=cfg.n_layer, n_head=cfg.n_head, n_local_heads=cfg.n_local_heads, head_dim=64,
+        intermediate_size=cfg.intermediate_size, vocab_size=cfg.vocab_size, fast_dim=cfg.fast_dim, n_fast_layer=cfg.n_fast_layer,
+        fast_n_head=cfg.fast_n_head, fast_n_local_heads=cfg.fast_n_local_heads, fast_head_dim=64,
+        fast_intermediate_size=cfg.fast_intermediate_size, codebook_size=cfg.codebook_size, num_codebooks=cfg.num_codebooks,
+        duplicate_code_0=int(cfg.duplicate_code_0), depthwise_wte=int(cfg.depthwise_wte), depthwise_output=int(cfg.depthwise_output),
+        tie_word_embeddings=int(cfg.tie_word_embeddings), max_seq_len=512, max_batch=8, page_size=32, semantic_start_id=320,
+        semantic_end_id=320 + cfg.codebook_size - 1, im_end_id=270, mlx_embed_mask=0, norm_eps=cfg.norm_eps)
+    h = ctypes.c_void_p()
+    assert lib.smol_create(ctypes.byref(c), ctypes.byref(h)) == 0
+    try:
+        n = lib.smol_phase_count(h)
+        assert n == phase_count(cfg)
+        off, words = ctypes.c_uint32(), ctypes.c_uint32()
+        end = 0
+        for p in range(n):
+            assert lib.smol_ll_region(h, p, ctypes.byref(off), ctypes.byref(words)) == 0
+            kind = decode_phase(p, cfg.n_layer, cfg.n_fast_layer)[0]
+            assert words.value == phase_words(cfg, p), f"phase {p} (kind {kind}): {words.value} words"
+            assert off.value == end, f"phase {p}: region at word {off.value}, the previous one ends at {end}"
+            end += words.value * 8 * 8
+        assert end * 8 < lib.smol_workspace_bytes(h)
+        for bad in (-1, n):
+            assert lib.smol_ll_region(h, bad, ctypes.byref(off), ctypes.byref(words)) == _capi.SMOL_ERR_INVALID
+    finally:
+        lib.smol_destroy(h)
 
 
 def test_mimi_create_validates_shapes_without_a_gpu():
