@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define SMOL_ABI_VERSION 2
+#define SMOL_ABI_VERSION 3
 #define SMOL_MAX_LAYERS 64
 #define SMOL_MAX_FAST_LAYERS 16
 
@@ -177,9 +177,8 @@ int smol_sample(SmolModel* m, const SmolBatch* b, int32_t batch, const float* d_
  * sequence: slow step, slow sample, depth loop with sampling, frame assembly, stop rule. */
 int smol_decode_frame(SmolModel* m, const SmolBatch* b, int32_t batch, const SmolSampling* s, void* stream);
 
-/* The loop of generate_blocking (G:200-205) without host round trips.  mode 2 / 0: ONE persistent
- * launch walks n_frames frames;  mode 1: the frame's per-phase launches are captured in a CUDA
- * graph (re-captured when batch / sampling / state pointers change) and replayed n_frames times. */
+/* The loop of generate_blocking (G:200-205) without host round trips: ONE persistent launch walks
+ * n_frames frames (either mode).  It only enqueues, so a caller may capture it in its own CUDA graph. */
 int smol_decode_frames(SmolModel* m, const SmolBatch* b, int32_t batch, const SmolSampling* s,
                        int32_t n_frames, void* stream);
 
@@ -205,9 +204,9 @@ int smol_set_profile(SmolModel* m, uint64_t* d_phase_ns);
 int smol_set_frame_clock(SmolModel* m, uint64_t* d_frame_ns, int32_t capacity);
 
 /* Options: "mode" 2 (default) = data-flow persistent kernel (flag-carrying activation words, TMA
- * producer warp; whole frames at batch 1, larger batches fall back to mode 0),
- * 0 = persistent cooperative kernel with a grid barrier per phase, 1 = one launch per phase, a frame
- * captured in a CUDA graph;  "n_ctas" = grid size (default: one CTA per SM);
+ * producer warp; whole frames of up to "ll_max_batch" sequences, larger batches fall back to mode 0),
+ * 0 = persistent cooperative kernel with a grid barrier per phase (1, one launch per phase, was removed
+ * in ABI version 3 and is refused with SMOL_ERR_INVALID);  "n_ctas" = grid size (default: one CTA per SM);
  * "tc_min_batch" (default 9: the measured crossover) = rows (sequences of a decode call, sequences x prompt positions of a prefill iteration)
  * from which the tcgen05 variant runs, 0 = never;  "prefill_tile" = cap on the prompt positions per prefill iteration
  * (0 = as many as fit: 128 rows on the tensor-core variant, 8 on the CUDA-core variants).
@@ -233,9 +232,6 @@ int64_t smol_get_option(const SmolModel* m, const char* name);
 void* smol_debug_buffer(SmolModel* m, const char* name);
 /* Word offset and length (words per sequence and replica) of phase `phase`'s region in the "ll" debug buffer. */
 int smol_ll_region(const SmolModel* m, int32_t phase, uint32_t* word_offset, uint32_t* words);
-/* Kernel launches issued for one frame in the current mode (mode 0: one launch covers all the
- * frames of a call). */
-int32_t smol_launches_per_frame(const SmolModel* m);
 /* Total kernel launches issued by this model so far. */
 int64_t smol_launch_count(const SmolModel* m);
 

@@ -11,7 +11,7 @@ import os
 
 from . import build as _build
 
-SMOL_ABI_VERSION = 2
+SMOL_ABI_VERSION = 3
 SMOL_MAX_LAYERS = 64
 SMOL_MAX_FAST_LAYERS = 16
 
@@ -145,7 +145,6 @@ PROTOTYPES = {
     "smol_get_option": (C.c_int64, [C.c_void_p, C.c_char_p]),
     "smol_debug_buffer": (C.c_void_p, [C.c_void_p, C.c_char_p]),
     "smol_ll_region": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
-    "smol_launches_per_frame": (C.c_int32, [C.c_void_p]),
     "smol_launch_count": (C.c_int64, [C.c_void_p]),
     # include/smoltts_b200_mimi.h
     "smol_mimi_create": (C.c_int, [C.POINTER(SmolMimiConfig), C.POINTER(C.c_void_p)]),

@@ -1,7 +1,7 @@
 // C ABI of the B200 DualAR decode engine (include/smoltts_b200.h).  Host-side only: shape checks,
-// workspace carving, launch geometry and the two launch modes (persistent cooperative kernel /
-// per-phase launches replayed from a CUDA graph).  No torch types, no allocation after create,
-// no device synchronisation: every compute entry point only enqueues work on the caller's stream.
+// workspace carving, launch geometry and kernel selection (data-flow kernel / persistent cooperative
+// barrier kernel).  No torch types, no allocation after create, no device synchronisation: every
+// compute entry point only enqueues work on the caller's stream.
 
 #include <cuda_runtime.h>
 
@@ -42,13 +42,6 @@ using smol::DevModel;
 
 static_assert(sizeof(SmolRowSampling) == 32, "SmolRowSampling is 32 bytes (include/smoltts_b200.h)");
 
-struct GraphKey {
-    SmolBatch b;
-    SmolSampling s;
-    int batch;
-    const int32_t* force;
-};
-
 struct SmolModel {
     SmolConfig cfg;
     DevModel dm;
@@ -75,12 +68,6 @@ struct SmolModel {
     size_t ll2_smem = 0;
     bool packed_ready = false; // tensor-core GEMV layout of the bound weights (rebuilt after a weight / workspace bind)
     int64_t launches = 0;
-    // mode 1: cached CUDA graph of one frame
-    cudaGraphExec_t frame_graph = nullptr;
-    cudaStream_t capture_stream = nullptr;  // the caller's stream may be the legacy default stream, which cannot capture
-    GraphKey frame_key;
-    bool frame_key_valid = false;
-    int64_t frame_graph_launches = 0;
     bool tmaps_ready = false;  // tensor maps of the tcgen05 variant (rebuilt after a weight / workspace bind)
 };
 
@@ -242,12 +229,7 @@ int smol_create(const SmolConfig* cfg, SmolModel** out) {
     return SMOL_OK;
 }
 
-void smol_destroy(SmolModel* m) {
-    if (!m) return;
-    if (m->frame_graph) cudaGraphExecDestroy(m->frame_graph);
-    if (m->capture_stream) cudaStreamDestroy(m->capture_stream);
-    delete m;
-}
+void smol_destroy(SmolModel* m) { delete m; }
 
 int smol_bind_weights(SmolModel* m, const SmolWeights* w) {
     if (!m || !w) return fail(SMOL_ERR_INVALID, "smol_bind_weights: null argument");
@@ -282,7 +264,6 @@ int smol_bind_weights(SmolModel* m, const SmolWeights* w) {
         if (!bind_layer(w->fast_layers[l], d.fast_layers[l], "fast_layers[*]")) return SMOL_ERR_INVALID;
     m->weights_bound = true;
     m->tmaps_ready = false;
-    m->frame_key_valid = false;
     m->packed_ready = false;
     // tensor maps and the packed GEMV layout are built here, at setup time: compute calls stay asynchronous and capturable
     if (m->ws_bound) {
@@ -326,7 +307,6 @@ int smol_bind_workspace(SmolModel* m, void* d_workspace, size_t bytes) {
     CU(cudaMemset(base + L.split_count, 0, L.packed - L.split_count));
     CU(cudaMemset(base + L.frame_tokens, 0, L.partial - L.frame_tokens));
     m->ws_bound = true;
-    m->frame_key_valid = false;
     if (m->weights_bound) {
         const int rc = ensure_tmaps(m);
         return rc ? rc : ensure_packed(m);
@@ -345,7 +325,6 @@ int smol_kv_bind(SmolModel* m, void* d_kv_pool, int32_t n_pages) {
     m->dm.kv_pool = reinterpret_cast<uint16_t*>(d_kv_pool);
     m->dm.n_pages = n_pages;
     m->kv_bound = true;
-    m->frame_key_valid = false;
     return SMOL_OK;
 }
 
@@ -459,7 +438,6 @@ static int ensure_packed(SmolModel* m) {
     if (!ok) return fail(SMOL_ERR_CUDA, "packing the weights for the data-flow kernel failed");
     CU(cudaDeviceSynchronize());   // setup-time only
     m->packed_ready = true;
-    m->frame_key_valid = false;
     return SMOL_OK;
 }
 
@@ -529,19 +507,19 @@ static int check_batch(const SmolModel* m, const SmolBatch* b, int batch) {
     return SMOL_OK;
 }
 
-// Enqueue `n_iter` iterations of phases [begin, end).  mode 0: one cooperative launch.
-// mode 1: one launch per phase (optionally the caller wraps a frame in a graph).
-// whole_iters: the call runs complete frames / complete prefill positions (what the data-flow kernel carries).
 static bool use_tc(const SmolModel* m, int rows) {
     return m->tc_min_batch > 0 && rows >= m->tc_min_batch && tc_eligible(m->cfg);
 }
 
+// Enqueue `n_iter` iterations of phases [begin, end) as one launch: the data-flow kernel (mode 2, whole frames of at most
+// ll_max_batch sequences) or the cooperative barrier kernel.
+// whole_iters: the call runs complete frames / complete prefill positions (what the data-flow kernel carries).
 static int enqueue(SmolModel* m, CallArgs A, cudaStream_t stream, bool whole_iters = false) {
     const int bt = use_tc(m, A.batch) ? 0 : smol::decode_batch_tile(A.batch);
     int rc;
     A.repeat = m->repeat;
     A.tc_split = m->tc_attn_split;
-    if (m->mode == 2 && whole_iters && A.mode == 0 && A.batch <= m->ll2_max_batch && A.batch <= smol::kLL2MaxTeams &&
+    if (m->mode == 2 && whole_iters && !A.prefill && A.batch <= m->ll2_max_batch && A.batch <= smol::kLL2MaxTeams &&
         A.batch <= m->n_ctas) {
         if ((rc = ensure_ll2(m))) return rc;
         if (m->ll2_state == 1) {
@@ -557,55 +535,8 @@ static int enqueue(SmolModel* m, CallArgs A, cudaStream_t stream, bool whole_ite
     }
     rc = ensure_tile(m, bt);
     if (rc) return rc;
-    A.repeat = m->repeat;
-    if (m->mode != 1) {
-        A.cooperative = 1;
-        CU(smol::decode_launch(m->dm, A, bt, m->n_ctas, m->smem[bt], (int)m->xs_bytes[bt], stream));
-        m->launches += 1;
-        return SMOL_OK;
-    }
-    const int n_iter = A.n_iter, begin = A.phase_begin, end = A.phase_end;
-    const int finalize = A.finalize, advance = A.advance, base = A.iter_base;
-    A.cooperative = 0;
-    if (n_iter == 0 && finalize) {
-        A.n_iter = 0;
-        CU(smol::decode_launch(m->dm, A, bt, 1, m->smem[bt], (int)m->xs_bytes[bt], stream));
-        m->launches += 1;
-        return SMOL_OK;
-    }
-    for (int it = 0; it < n_iter; ++it) {
-        for (int p = begin; p < end; ++p) {
-            const bool last = (it == n_iter - 1) && (p == end - 1);
-            A.n_iter = 1;
-            A.iter_base = base + it * (A.tile_t > 1 ? A.tile_t : 1);
-            A.phase_begin = p;
-            A.phase_end = p + 1;
-            A.finalize = 0;
-            A.advance = 0;
-            A.tc_part = 0;
-            const smol::Phase ph = smol::unpack_phase(m->dm.prog[p]);
-            const bool weights = ph.kind != smol::PH_ATTN && ph.kind != smol::PH_SAMPLE;
-            if (bt == 0 && weights) {
-                // the grid barriers between a phase's pre-step, tiles and post-step become launch boundaries
-                const bool post = smol::tc_has_poststep(ph);
-                if (smol::tc_has_prestep(ph)) {
-                    A.tc_part = 1;
-                    CU(smol::decode_launch(m->dm, A, bt, m->n_ctas, m->smem[bt], (int)m->xs_bytes[bt], stream));
-                    m->launches += 1;
-                }
-                A.tc_part = 2;
-                if (post) {
-                    CU(smol::decode_launch(m->dm, A, bt, m->n_ctas, m->smem[bt], (int)m->xs_bytes[bt], stream));
-                    m->launches += 1;
-                    A.tc_part = 3;
-                }
-            }
-            A.finalize = last ? finalize : 0;
-            A.advance = (p == end - 1) ? advance : 0;
-            CU(smol::decode_launch(m->dm, A, bt, m->n_ctas, m->smem[bt], (int)m->xs_bytes[bt], stream));
-            m->launches += 1;
-        }
-    }
+    CU(smol::decode_launch(m->dm, A, bt, m->n_ctas, m->smem[bt], (int)m->xs_bytes[bt], stream));
+    m->launches += 1;
     return SMOL_OK;
 }
 
@@ -632,7 +563,7 @@ int smol_prefill(SmolModel* m, const SmolBatch* b, int32_t batch, const int32_t*
     if ((rc = check_batch(m, b, batch))) return rc;
     if (!d_prompt || !d_prompt_len || s_max < 1) return fail(SMOL_ERR_INVALID, "smol_prefill: bad prompt");
     CallArgs A = base_args(b, batch, nullptr);
-    A.mode = 1;
+    A.prefill = 1;
     // tile_t prompt positions per iteration share one pass over the weights (rows = batch * tile_t fit the workspace)
     // -- up to kPrefillRows rows (128-row tensor-core tiles); 8 positions on the CUDA-core variants
     const int rows_cap = ws_rows(m->cfg);
@@ -731,42 +662,8 @@ int smol_decode_frames(SmolModel* m, const SmolBatch* b, int32_t batch, const Sm
     CallArgs A = base_args(b, batch, s);
     A.phase_begin = 0;
     A.phase_end = smol::phases_per_frame(m->dm.n_layer, m->dm.n_flayer, m->dm.depth);
-    if (m->mode != 1) {
-        A.n_iter = n_frames;
-        return enqueue(m, A, stream, true);
-    }
-    // mode 1: one frame = phase_end launches, captured once per (batch, state pointers, sampling)
-    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-    CU(cudaStreamIsCapturing(stream, &cs));
-    if (cs != cudaStreamCaptureStatusNone) {  // the caller is capturing: just enqueue
-        A.n_iter = n_frames;
-        return enqueue(m, A, stream);
-    }
-    GraphKey key;
-    std::memset(&key, 0, sizeof(key));
-    key.b = *b; key.s = *s; key.batch = batch; key.force = m->dm.force;
-    if (!m->frame_key_valid || std::memcmp(&key, &m->frame_key, sizeof(key)) != 0) {
-        if (m->frame_graph) { cudaGraphExecDestroy(m->frame_graph); m->frame_graph = nullptr; }
-        cudaGraph_t g = nullptr;
-        if (!m->capture_stream) CU(cudaStreamCreateWithFlags(&m->capture_stream, cudaStreamNonBlocking));
-        CU(cudaStreamBeginCapture(m->capture_stream, cudaStreamCaptureModeThreadLocal));
-        A.n_iter = 1;
-        const int64_t before = m->launches;
-        rc = enqueue(m, A, m->capture_stream);
-        m->frame_graph_launches = m->launches - before;
-        m->launches = before;
-        cudaError_t e = cudaStreamEndCapture(m->capture_stream, &g);
-        if (rc) { if (g) cudaGraphDestroy(g); return rc; }
-        if (e != cudaSuccess) return cuda_fail(e, "cudaStreamEndCapture");
-        e = cudaGraphInstantiate(&m->frame_graph, g, 0);
-        cudaGraphDestroy(g);
-        if (e != cudaSuccess) return cuda_fail(e, "cudaGraphInstantiate");
-        m->frame_key = key;
-        m->frame_key_valid = true;
-    }
-    for (int f = 0; f < n_frames; ++f) CU(cudaGraphLaunch(m->frame_graph, stream));
-    m->launches += (int64_t)n_frames * m->frame_graph_launches;
-    return SMOL_OK;
+    A.n_iter = n_frames;
+    return enqueue(m, A, stream, true);
 }
 
 int smol_decode_frame(SmolModel* m, const SmolBatch* b, int32_t batch, const SmolSampling* s, void* stream) {
@@ -782,7 +679,6 @@ int smol_set_force(SmolModel* m, const int32_t* d_force) {
 int smol_set_profile(SmolModel* m, uint64_t* d_phase_ns) {
     if (!m) return fail(SMOL_ERR_INVALID, "null model");
     m->dm.prof = reinterpret_cast<unsigned long long*>(d_phase_ns);
-    m->frame_key_valid = false;
     return SMOL_OK;
 }
 
@@ -791,20 +687,19 @@ int smol_set_frame_clock(SmolModel* m, uint64_t* d_frame_ns, int32_t capacity) {
     if (d_frame_ns && capacity <= 0) return fail(SMOL_ERR_INVALID, "smol_set_frame_clock: capacity must be positive");
     m->dm.frame_ns = reinterpret_cast<unsigned long long*>(d_frame_ns);
     m->dm.frame_ns_cap = d_frame_ns ? capacity : 0;
-    m->frame_key_valid = false;
     return SMOL_OK;
 }
 
 int smol_set_option(SmolModel* m, const char* name, int64_t value) {
     if (!m || !name) return fail(SMOL_ERR_INVALID, "null argument");
     if (!std::strcmp(name, "mode")) {
-        if (value < 0 || value > 2) return fail(SMOL_ERR_INVALID, "mode must be 0, 1 or 2");
+        if (value == 1) return fail(SMOL_ERR_INVALID, "mode 1 (one launch per phase) was removed: use 0 or 2");
+        if (value != 0 && value != 2) return fail(SMOL_ERR_INVALID, "mode must be 0 or 2");
         m->mode = (int)value;
         return SMOL_OK;
     }
     if (!std::strcmp(name, "repeat")) {
         m->repeat = value > 0 ? (int)value : 0;
-        m->frame_key_valid = false;
         return SMOL_OK;
     }
     if (!std::strcmp(name, "prefill_tile")) {
@@ -813,12 +708,10 @@ int smol_set_option(SmolModel* m, const char* name, int64_t value) {
     }
     if (!std::strcmp(name, "tc_attn_split")) {
         m->tc_attn_split = value > 0 ? (int)value : 0;
-        m->frame_key_valid = false;
         return SMOL_OK;
     }
     if (!std::strcmp(name, "tc_min_batch")) {  // 0 disables the tensor-core variant
         m->tc_min_batch = value > 0 ? (int)value : 0;
-        m->frame_key_valid = false;  // a cached frame graph was captured for the other kernel variant
         return SMOL_OK;
     }
     if (!std::strcmp(name, "ll_holdoff")) {
@@ -838,7 +731,6 @@ int smol_set_option(SmolModel* m, const char* name, int64_t value) {
         if (value < 0) return fail(SMOL_ERR_INVALID, "n_ctas must be >= 0");
         m->n_ctas_override = (int)value;
         m->configured = false;
-        m->frame_key_valid = false;
         return SMOL_OK;
     }
     return fail(SMOL_ERR_INVALID, std::string("unknown option ") + name);
@@ -892,11 +784,6 @@ int smol_ll_region(const SmolModel* m, int32_t phase, uint32_t* word_offset, uin
     *word_offset = m->dm.ll_off[phase];
     *words = m->dm.ll_len[phase];
     return SMOL_OK;
-}
-
-int32_t smol_launches_per_frame(const SmolModel* m) {
-    if (!m) return 0;
-    return m->mode != 1 ? 1 : smol::phases_per_frame(m->dm.n_layer, m->dm.n_flayer, m->dm.depth);
 }
 
 int64_t smol_launch_count(const SmolModel* m) { return m ? m->launches : 0; }

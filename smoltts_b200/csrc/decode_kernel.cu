@@ -28,9 +28,6 @@
 // Rounding points follow the reference's eager bf16 forward exactly (bf16 after every Linear, each
 // RMSNorm stage, RoPE, SDPA, silu, the product and each residual add; fp32 inside), so only
 // summation order differs.
-//
-// The same kernel launched non-cooperatively runs exactly one phase (phase_end == phase_begin+1):
-// that is the "one kernel per op" mode used for CUDA-graph capture, per-phase profiling and tests.
 
 #include "common.cuh"
 #include "dev_model.h"
@@ -351,13 +348,13 @@ __device__ __forceinline__ int prefill_t(const CallArgs& A, const Ctx& c, int bg
     return A.iter_base + c.iter * (A.tile_t > 1 ? A.tile_t : 1) + row_off(A, bg);
 }
 __device__ __forceinline__ bool seq_active(const DevModel& M, const CallArgs& A, const Ctx& c, int bg) {
-    if (A.mode == 1) return prefill_t(A, c, bg) < ldcg_i32(A.prompt_len + row_seq(A, bg)) - 1;
+    if (A.prefill) return prefill_t(A, c, bg) < ldcg_i32(A.prompt_len + row_seq(A, bg)) - 1;
     return A.b.finished == nullptr || __ldcg(A.b.finished + bg) == 0;
 }
 
 // id of grid row r of sequence bg for the slow embedding
 __device__ __forceinline__ int input_token(const DevModel& M, const CallArgs& A, const Ctx& c, int bg, int r) {
-    if (A.mode == 1) {
+    if (A.prefill) {
         int t = prefill_t(A, c, bg);
         const int b = row_seq(A, bg);
         const int len = ldcg_i32(A.prompt_len + b);
@@ -880,7 +877,7 @@ __device__ void phase_sample(const DevModel& M, const CallArgs& A, const Ctx& c,
     }
 }
 
-// BT == 0: the tensor-core variant (tc_phases.cuh) -- 128-row tiles, batch attention, cooperative launches only.
+// BT == 0: the tensor-core variant (tc_phases.cuh) -- 128-row tiles, batch attention.
 template <int BT>
 __device__ __forceinline__ void run_phase(const DevModel& M, const CallArgs& A, const Ctx& c, const Phase& ph,
                                           uint32_t& parity, umma::Pipe& pipe, uint32_t& target, bool first_in_launch,
@@ -888,7 +885,7 @@ __device__ __forceinline__ void run_phase(const DevModel& M, const CallArgs& A, 
     if (BT == 0) {
         if (ph.kind == PH_ATTN) phase_attn_batch(M, A, c, ph);
         else if (ph.kind == PH_SAMPLE)
-            phase_sample(M, A, c, ph, A.cooperative && next_in_launch && !A.fast_from_xf && !(ph.fast && ph.depth_pos == M.depth - 1));
+            phase_sample(M, A, c, ph, next_in_launch && !A.fast_from_xf && !(ph.fast && ph.depth_pos == M.depth - 1));
         else phase_gemm_tc(M, A, c, ph, &g_tc_bars, pipe, target, first_in_launch, next_in_launch);
         return;
     }
@@ -925,14 +922,13 @@ smol_decode_kernel(const __grid_constant__ DevModel M, const __grid_constant__ C
     }
     __syncthreads();
 
-    uint32_t target = 0;
-    if (A.cooperative) target = ldcg_u32(M.barrier + 1);
+    uint32_t target = ldcg_u32(M.barrier + 1);
     uint32_t parity = 0;
     umma::Pipe pipe;
     pipe.chunk = 0; pipe.tile = 0;
     if (BT == 0) umma::setup(&g_tc_bars, pipe, (uint32_t)umma::kAcc, 2u);
-    const int per_iter = (A.mode == 1) ? phases_per_prefill_step(M.n_layer)
-                                       : phases_per_frame(M.n_layer, M.n_flayer, M.depth);
+    const int per_iter = A.prefill ? phases_per_prefill_step(M.n_layer)
+                                   : phases_per_frame(M.n_layer, M.n_flayer, M.depth);
     const bool prof_cta = (M.prof != nullptr) && c.cta == 0;  // CTA-uniform
     const bool prof = prof_cta && c.tid == 0;
     unsigned long long t0 = 0, t1 = 0;
@@ -952,9 +948,7 @@ smol_decode_kernel(const __grid_constant__ DevModel M, const __grid_constant__ C
                 __syncthreads();
                 if (prof) t1 = globaltimer_ns();
             }
-            // (tensor-core variant, one phase per launch: a phase may take up to three launches; bookkeeping runs in the last)
-            const bool final_part = A.tc_part == 0 || A.tc_part == (tc_has_poststep(ph) ? 3 : 2);
-            if (c.cta == 0 && p == per_iter - 1 && A.mode == 1 && final_part) {
+            if (c.cta == 0 && p == per_iter - 1 && A.prefill) {
                 // prefill bookkeeping: every sequence advances by the positions of this tile that lie inside its prompt
                 const int T = A.tile_t > 1 ? A.tile_t : 1;
                 for (int b = c.tid; b < A.real_batch; b += kThreads) {
@@ -963,12 +957,11 @@ smol_decode_kernel(const __grid_constant__ DevModel M, const __grid_constant__ C
                     if (n_act) A.b.seq_len[b] = ldcg_i32(A.b.seq_len + b) + n_act;
                 }
             }
-            if (c.cta == 0 && A.mode == 0 && A.advance && p == A.phase_end - 1) {
+            if (c.cta == 0 && !A.prefill && A.advance && p == A.phase_end - 1) {
                 for (int b = c.tid; b < A.batch; b += kThreads) A.b.seq_len[b] = ldcg_i32(A.b.seq_len + b) + 1;
             }
             const bool last = (it == A.n_iter - 1) && (p == A.phase_end - 1);
-            const bool sync = A.cooperative && !last;
-            if (sync) {
+            if (!last) {
                 if (BT == 0) fence_proxy_async_all();
                 grid_arrive(M.barrier, target, (uint32_t)c.n_ctas);
             }
@@ -981,7 +974,7 @@ smol_decode_kernel(const __grid_constant__ DevModel M, const __grid_constant__ C
                     st_it = nit; st_p = np;
                 }
             }
-            if (sync) {
+            if (!last) {
                 grid_wait(M.barrier, target);
                 if (BT == 0 && (c.tid == umma::kTmaProducerA || c.tid == umma::kTmaProducerB)) fence_proxy_async_all();   // the threads that issue TMA loads
             }
@@ -992,7 +985,7 @@ smol_decode_kernel(const __grid_constant__ DevModel M, const __grid_constant__ C
             }
         }
     }
-    if (A.mode == 1 && A.finalize && c.cta == 0) {
+    if (A.prefill && A.finalize && c.cta == 0) {
         // leave the last prompt column as the pending input of the first decode frame (G:66-73)
         for (int i = c.tid; i < A.real_batch * M.n_rows; i += kThreads) {
             const int b = i / M.n_rows, r = i - b * M.n_rows;
@@ -1000,7 +993,7 @@ smol_decode_kernel(const __grid_constant__ DevModel M, const __grid_constant__ C
             A.b.tokens[i] = ldcg_i32(A.prompt + ((size_t)b * M.n_rows + r) * A.s_max + (len - 1));
         }
     }
-    if (A.cooperative && c.cta == 0 && c.tid == 0) M.barrier[1] = target;
+    if (c.cta == 0 && c.tid == 0) M.barrier[1] = target;
     if (BT == 0) umma::teardown(&g_tc_bars);
 }
 
@@ -1125,9 +1118,7 @@ cudaError_t decode_max_ctas(int bt, size_t smem, int* per_sm) {
 cudaError_t decode_launch(const DevModel& M, const CallArgs& A, int bt, int n_ctas, size_t smem, int xs_bytes,
                           cudaStream_t stream) {
     void* args[3] = {(void*)&M, (void*)&A, (void*)&xs_bytes};
-    if (A.cooperative)
-        return cudaLaunchCooperativeKernel(decode_fn(bt), dim3(n_ctas), dim3(kThreads), args, smem, stream);
-    return cudaLaunchKernel(decode_fn(bt), dim3(n_ctas), dim3(kThreads), args, smem, stream);
+    return cudaLaunchCooperativeKernel(decode_fn(bt), dim3(n_ctas), dim3(kThreads), args, smem, stream);
 }
 
 }  // namespace smol

@@ -152,20 +152,17 @@ struct CallArgs {
     SmolBatch b;
     SmolSampling s;
     int batch;
-    int mode;         // 0 decode frames, 1 prefill steps
+    int prefill;      // 0 decode frames, 1 prefill steps
     int n_iter;       // frames (decode) or prompt positions (prefill) in this launch
     int iter_base;    // prefill: prompt position of iteration 0
     int finalize;     // prefill: this launch ends the prompt -> publish the last column as pending input
     int phase_begin;  // phases [begin, end) of every iteration
     int phase_end;
-    int cooperative;  // 1: grid barrier between phases; 0: exactly one phase per launch
     int advance;      // slow-only launches: bump seq_len after the last phase
     int fast_from_xf; // depth-step launches: layer 0 reads the caller-filled xf buffer
     int repeat;       // profiling only: run the body of every weight phase 1 + repeat times
     int tile_t;       // prefill: prompt positions handled per iteration (rows = real_batch * tile_t share the weight pass)
     int real_batch;   // prefill: sequences (rows / tile_t)
-    int tc_part;      // tensor-core variant, one phase per launch: 1 = only the phase's distributed pre-step, 2 = only its tiles,
-                      // 3 = only its post-step (0 = the whole phase: cooperative launches)
     int tc_split;     // tensor-core variant: cached positions per attention split (0 = default)
     int team_ctas;    // second-generation data-flow kernel: CTAs per sequence (one team each); grid = batch * team_ctas
     int mlp_cluster;  // data-flow kernel, batch 1: CTAs per thread-block cluster of the fused gated MLP (0 = unfused)
@@ -250,7 +247,6 @@ __host__ __device__ inline int tm_weight_slot(int weight_index, int box_rows) {
 }
 constexpr int kTensorMapBytes = 128;
 constexpr int kTcKSplit = 4;  // K slices of the wo / w2 tiles (their sum + residual + next RMSNorm is the phase's post-step)
-__host__ __device__ inline bool tc_has_poststep(const Phase& ph) { return ph.kind == PH_WO || ph.kind == PH_W2; }
 
 __host__ __device__ inline uint32_t pack_phase(const Phase& ph) {
     return (uint32_t)ph.kind | ((uint32_t)ph.fast << 4) | ((uint32_t)ph.layer << 8) | ((uint32_t)ph.depth_pos << 16);

@@ -167,9 +167,12 @@ __device__ void tc_fast_attention(const DevModel& M, const CallArgs& A, const Ct
         const uint4 ka1 = ok0 ? ldcg_v4(kb + (size_t)jl * kvw + part * 16 + 8) : zero4;
         const uint4 kb0 = ok1 ? ldcg_v4(kb + (size_t)(jl + 8) * kvw + part * 16) : zero4;
         const uint4 kb1 = ok1 ? ldcg_v4(kb + (size_t)(jl + 8) * kvw + part * 16 + 8) : zero4;
+        // V rows as 32-bit offsets from one per-lane base: a 64-bit address per position, each under its own j <= depth_pos
+        // predicate, makes this prologue ~20 % longer and spills predicates (the fast wo pre-step at bs=256: +9 %)
+        const uint32_t* vl = reinterpret_cast<const uint32_t*>(vb) + c.lane;   // V dims 2*lane, 2*lane+1 of position 0
         uint32_t vv[kMaxDepth];
 #pragma unroll
-        for (int j = 0; j < kMaxDepth; ++j) vv[j] = j <= depth_pos ? ldcg_u32(vb + (size_t)j * kvw + 2 * c.lane) : 0u;
+        for (int j = 0; j < kMaxDepth; ++j) vv[j] = j <= depth_pos ? __ldcg(vl + j * (kvw / 2)) : 0u;
         float qf[16];
         unpack8(q0, *reinterpret_cast<float(*)[8]>(qf));
         unpack8(q1, *reinterpret_cast<float(*)[8]>(qf + 8));
@@ -303,7 +306,7 @@ __device__ void phase_attn_batch(const DevModel& M, const CallArgs& A, const Ctx
         // cached positions that hold data: everything up to the group's last ACTIVE row (rows past the end of a prompt do
         // not append; their stale slots must not reach the PV product of the active rows as 0 x garbage)
         int Lload = Lg;
-        if (A.mode == 1) {
+        if (A.prefill) {
             const int act = ldcg_i32(A.prompt_len + bs) - 1 - (A.iter_base + c.iter * T);
             Lload = min(Lg, len0 + max(0, min(act, T)));
         }
@@ -518,8 +521,7 @@ __device__ void phase_attn_batch(const DevModel& M, const CallArgs& A, const Ctx
 }
 
 // One weight phase on the tensor cores.  `target` is the grid barrier's running count: most phases start with a
-// distributed pre-step (tc_norm_rows, or the depth attention before a fast wo) followed by an extra grid barrier;
-// one-phase-per-launch mode runs the pre-step and the tiles as two launches instead (A.tc_part).
+// distributed pre-step (tc_norm_rows, or the depth attention before a fast wo) followed by an extra grid barrier.
 __device__ void phase_gemm_tc(const DevModel& M, const CallArgs& A, const Ctx& c, const Phase& ph, umma::Bars* bars,
                               umma::Pipe& pipe, uint32_t& target, bool first_in_launch, bool next_in_launch) {
     const bool fast = ph.fast != 0;
@@ -542,34 +544,29 @@ __device__ void phase_gemm_tc(const DevModel& M, const CallArgs& A, const Ctx& c
     if (prof) ts = globaltimer_ns();
 
     // ---- distributed pre-step ----
-    // (a normed phase that follows a wo / w2 inside one cooperative launch finds M.xn written by that phase's post-step)
+    // (a normed phase that follows a wo / w2 inside one launch finds M.xn written by that phase's post-step)
     // (and the first QKV of a depth step finds its input written by the SAMPLE phase before it: phase_sample, tc_feed)
-    const bool fed_by_post = A.cooperative && !first_in_launch &&
+    const bool fed_by_post = !first_in_launch &&
                              (kind == PH_W13 || kind == PH_HEAD || (kind == PH_QKV && ph.layer > 0) ||
                               (kind == PH_QKV && fast && ph.layer == 0 && !A.fast_from_xf));
     if (tc_has_prestep(ph) && !fed_by_post) {
-        if (A.tc_part == 0 || A.tc_part == 1) {
-            if (kind == PH_WO) {
-                tc_fast_attention(M, A, c, ph.layer, ph.depth_pos);
-            } else {
-                int src_kind = 3;
-                const uint16_t* base = kind == PH_W13 ? M.h : stream;
-                uint16_t* spill = nullptr;
-                if (kind == PH_QKV && ph.layer == 0) {
-                    if (!fast) { src_kind = 0; spill = M.x; }
-                    else if (!A.fast_from_xf) { src_kind = ph.depth_pos == 0 ? 1 : 2; spill = M.xf; }
-                }
-                const uint16_t* norm_w = kind == PH_QKV ? L.attention_norm : kind == PH_W13 ? L.ffn_norm : (fast ? M.fast_norm : M.norm);
-                tc_norm_rows(M, A, c, ph, src_kind, base, spill, norm_w, D);
+        if (kind == PH_WO) {
+            tc_fast_attention(M, A, c, ph.layer, ph.depth_pos);
+        } else {
+            int src_kind = 3;
+            const uint16_t* base = kind == PH_W13 ? M.h : stream;
+            uint16_t* spill = nullptr;
+            if (kind == PH_QKV && ph.layer == 0) {
+                if (!fast) { src_kind = 0; spill = M.x; }
+                else if (!A.fast_from_xf) { src_kind = ph.depth_pos == 0 ? 1 : 2; spill = M.xf; }
             }
+            const uint16_t* norm_w = kind == PH_QKV ? L.attention_norm : kind == PH_W13 ? L.ffn_norm : (fast ? M.fast_norm : M.norm);
+            tc_norm_rows(M, A, c, ph, src_kind, base, spill, norm_w, D);
         }
-        if (A.cooperative) {
-            fence_proxy_async_all();
-            grid_arrive(M.barrier, target, (uint32_t)c.n_ctas);
-            grid_wait(M.barrier, target);
-            if (c.tid == umma::kTmaProducerA || c.tid == umma::kTmaProducerB) fence_proxy_async_all();   // the threads that issue TMA loads
-        }
-        if (A.tc_part == 1) return;
+        fence_proxy_async_all();
+        grid_arrive(M.barrier, target, (uint32_t)c.n_ctas);
+        grid_wait(M.barrier, target);
+        if (c.tid == umma::kTmaProducerA || c.tid == umma::kTmaProducerB) fence_proxy_async_all();   // the threads that issue TMA loads
     }
     if (prof) { const unsigned long long t = globaltimer_ns(); seg[0] += t - ts; ts = t; }
 
@@ -594,7 +591,7 @@ __device__ void phase_gemm_tc(const DevModel& M, const CallArgs& A, const Ctx& c
     int blk = 16;
     while (blk < blk_cap && m_tiles * ((n_out + blk - 1) / blk) * n_split > c.n_ctas) blk += 16;
     const int n_blocks = (n_out + blk - 1) / blk;
-    const int n_units = (A.tc_part == 0 || A.tc_part == 2) ? m_tiles * n_blocks * n_split : 0;
+    const int n_units = m_tiles * n_blocks * n_split;
 
     for (int u = c.cta; u < n_units; u += c.n_ctas) {
 #if SMOL_TC_UNIT_ORDER
@@ -696,13 +693,11 @@ __device__ void phase_gemm_tc(const DevModel& M, const CallArgs& A, const Ctx& c
     }
 
     // ---- post-step of the residual phases: wo: h = stream + wo(attn) (P:499); w2: stream = h + w2(act) (P:500) ----
-    if (has_post && A.tc_part != 2) {
-        if (A.cooperative) {
-            grid_arrive(M.barrier, target, (uint32_t)c.n_ctas);
-            grid_wait(M.barrier, target);
-        }
+    if (has_post) {
+        grid_arrive(M.barrier, target, (uint32_t)c.n_ctas);
+        grid_wait(M.barrier, target);
         const uint16_t* next_norm = nullptr;
-        if (A.cooperative && next_in_launch) {
+        if (next_in_launch) {
             const int n_net = fast ? M.n_flayer : M.n_layer;
             if (kind == PH_WO) next_norm = L.ffn_norm;
             else if (ph.layer + 1 < n_net) next_norm = (fast ? M.fast_layers[ph.layer + 1] : M.layers[ph.layer + 1]).attention_norm;

@@ -431,10 +431,6 @@ class RQTransformer:
     def launch_count(self) -> int:
         return int(self.lib.smol_launch_count(self._h))
 
-    @property
-    def launches_per_frame(self) -> int:
-        return int(self.lib.smol_launches_per_frame(self._h))
-
     def debug_buffer(self, name: str, batch: Optional[int] = None) -> torch.Tensor:
         """View of a workspace buffer (see include/smoltts_b200.h: smol_debug_buffer)."""
         cfg = self.config

@@ -57,6 +57,13 @@ def test_create_validates_shapes_without_a_gpu():
     b = _capi.SmolBatch()
     assert lib.smol_slow_step(h, ctypes.byref(b), 1, 1, None) == _capi.SMOL_ERR_UNBOUND
     assert b"bound" in lib.smol_last_error()
+    # "mode" takes 0 and 2; 1 (one launch per phase) was removed and is refused without changing the mode
+    assert lib.smol_set_option(h, b"mode", 1) == _capi.SMOL_ERR_INVALID
+    assert b"mode 1" in lib.smol_last_error() and b"removed" in lib.smol_last_error()
+    assert lib.smol_get_option(h, b"mode") == 2
+    for mode in (0, 2):
+        assert lib.smol_set_option(h, b"mode", mode) == 0
+        assert lib.smol_get_option(h, b"mode") == mode
     lib.smol_destroy(h)
     h2 = ctypes.c_void_p()
     assert lib.smol_create(ctypes.byref(make(fast_dim=512, fast_n_head=8)), ctypes.byref(h2)) == _capi.SMOL_ERR_UNSUPPORTED

@@ -156,10 +156,10 @@ def test_greedy_vs_literal_reference_goldens(size):
 
 
 def test_modes_and_batch_composition_are_bit_identical():
-    """mode 0 (one persistent kernel) == mode 1 (per-phase launches in a CUDA graph), and a sequence
-    decodes to the same ids alone, inside a batch of 3, and inside a batch of 11 (two batch tiles) -- on the GEMV variants
-    (the tcgen05 variant, which would take the batch of 11 and every prefill, is switched off here: it is bit-identical
-    with itself, tests/test_gpu_tc.py, not with the GEMV kernels)."""
+    """mode 0 == mode 2 whatever the number of frames per launch (chunks of 7, 20 and 9), and a sequence decodes to the
+    same ids alone, inside a batch of 3, and inside a batch of 11 (two batch tiles) -- on the GEMV variants of the barrier
+    kernel (the tcgen05 variant, which would take the batch of 11 and every prefill, is switched off here: it is
+    bit-identical with itself, tests/test_gpu_tc.py, not with the GEMV kernels)."""
     from smoltts_b200 import GenerationSettings, generate_batch
 
     cfg, sd, model, orc = model_and_oracle("smoltts_byte_tiny", max_batch=16)
@@ -181,7 +181,6 @@ def _modes_and_composition(model, prompts, gs):
     model.set_option("mode", 0)
     try:
         ref = generate_batch(model, prompts, gs, audio_only=False, fixed_frames=20, chunk=7)
-        model.set_option("mode", 1)
         alt = generate_batch(model, prompts, gs, audio_only=False, fixed_frames=20, chunk=20)
     finally:
         model.set_option("mode", 2)  # default: data-flow kernel up to 8 sequences, barrier kernel above
@@ -199,21 +198,20 @@ def _modes_and_composition(model, prompts, gs):
 
 
 @pytest.mark.parametrize("size,lens", [("smoltts_byte_tiny", [45]), ("smoltts_byte_70m", [70]), ("smoltts_byte_tiny", [33, 9, 58])])
-def test_prefill_tiles_and_modes_write_identical_kv(size, lens):
-    """Prefill on the CUDA-core barrier kernel (fewer than 9 rows) -- 8 / 3 / 1 prompt positions per iteration, one
-    cooperative launch or one launch per phase -- then two frames: bit-identical K/V, seq_len, pending tokens and codes,
-    also for ragged prompt lengths (rows of a tile past the end of a prompt are inert)."""
+def test_prefill_tiles_write_identical_kv(size, lens):
+    """Prefill on the CUDA-core barrier kernel (fewer than 9 rows) -- 8 / 3 / 1 prompt positions per iteration -- then two
+    frames: bit-identical K/V, seq_len, pending tokens and codes, also for ragged prompt lengths (rows of a tile past the end
+    of a prompt are inert)."""
     from smoltts_b200.generate import pack_prompts
 
     cfg, sd, model, orc = model_and_oracle(size)
     B = len(lens)
     prompts = [prompt_grid(byte_prompt(n, seed=110 + b), cfg) for b, n in enumerate(lens)]
-    variants = [(0, 8 // B), (0, 1), (1, 8 // B)] + ([(0, 3)] if B == 1 else [])
+    tiles = [8 // B, 1] + ([3] if B == 1 else [])
     got = []
     model.set_option("ll_max_batch", 0)       # the two frames on the barrier kernel too
     try:
-        for mode, tile in variants:
-            model.set_option("mode", mode)
+        for tile in tiles:
             model.set_option("prefill_tile", tile)
             padded, lens_t = pack_prompts(model, prompts)
             batch = model.new_batch(B, max_positions=128, max_frames=4)
@@ -227,14 +225,13 @@ def test_prefill_tiles_and_modes_write_identical_kv(size, lens):
             finally:
                 batch.release()
     finally:
-        model.set_option("mode", 2)
         model.set_option("prefill_tile", 0)
         model.set_option("ll_max_batch", 8)
     assert got[0][1].tolist() == [n + 12 - 1 + 2 for n in lens]
-    for (mode, tile), g in zip(variants[1:], got[1:]):
-        assert torch.equal(g[0].view(torch.int16), got[0][0].view(torch.int16)), f"KV differs (mode {mode}, tile {tile})"
+    for tile, g in zip(tiles[1:], got[1:]):
+        assert torch.equal(g[0].view(torch.int16), got[0][0].view(torch.int16)), f"KV differs (tile {tile})"
         for a, b in zip(g[1:], got[0][1:]):
-            assert torch.equal(a, b), f"state differs (mode {mode}, tile {tile})"
+            assert torch.equal(a, b), f"state differs (tile {tile})"
 
 
 @pytest.mark.parametrize("cfgset", [

@@ -4,8 +4,7 @@ Its dot products are summed by the tensor core, so it is not bit-identical to th
   * the oracle's greedy ids up to near-tie decisions (greedy-with-resync, same rule and TAU as tests/test_gpu_decode.py);
   * the CUDA-core variant's logits and cached K/V on the same inputs, within the spread the reference's own bf16
     executions show (rms 0.035 / 0.056 on token / codebook logits, DESIGN.md section 6);
-  * bit-identity with itself across launch modes (persistent kernel == per-phase CUDA graph), batch compositions and
-    prefill tile sizes.
+  * bit-identity with itself across batch compositions and prefill tile sizes.
 """
 import numpy as np
 import pytest
@@ -68,13 +67,8 @@ def test_tc_greedy_with_resync_vs_oracle(size):
     assert exact >= 0.915 * total, f"{exact}/{total} identical decisions: below the measured rate (150m: 804/864 = 0.93)"
 
 
-def _bits(t):
-    return t.view(torch.int32) if t.dtype == torch.float32 else t.view(torch.int16) if t.dtype == torch.bfloat16 else t
-
-
-def _prefill_and_frames(model, prompts, n_frames, tc_min_batch, mode=2, prefill_tile=0):
+def _prefill_and_frames(model, prompts, n_frames, tc_min_batch, prefill_tile=0):
     model.set_option("tc_min_batch", tc_min_batch)
-    model.set_option("mode", mode)
     model.set_option("prefill_tile", prefill_tile)
     B = len(prompts)
     padded, lens = pack_prompts(model, prompts)
@@ -92,13 +86,12 @@ def _prefill_and_frames(model, prompts, n_frames, tc_min_batch, mode=2, prefill_
                     seq_len=batch.seq_len.clone())
     finally:
         model.set_option("tc_min_batch", 9)
-        model.set_option("mode", 2)
         model.set_option("prefill_tile", 0)
         batch.release()
 
 
 @pytest.mark.parametrize("size", ["smoltts_byte_tiny", "smoltts_byte_150m"])
-def test_tc_close_to_cuda_core_variant_and_mode_invariant(size):
+def test_tc_close_to_cuda_core_variant(size):
     cfg, sd, model, orc = model_and_oracle(size, max_batch=32)
     B = 20
     prompts = [prompt_grid(byte_prompt(30 + b, seed=70 + b), cfg) for b in range(B)]
@@ -117,10 +110,6 @@ def test_tc_close_to_cuda_core_variant_and_mode_invariant(size):
         rms, mx = d.pow(2).mean().sqrt().item(), d.abs().max().item()
         print(f"{size}: {name} rms diff {rms:.4f} max {mx:.4f}")
         assert rms < (0.04 if name == "tl" else 0.06) and mx < 0.3   # the reference's own bf16-vs-fp32 rms: 0.035 / 0.056
-    # the per-phase CUDA-graph mode runs the same tiles (pre-step and tiles as two launches): bit-identical
-    g1 = _prefill_and_frames(model, prompts, 1, 9, mode=1)
-    for k in ("kv", "codes", "tl", "dl"):
-        assert torch.equal(_bits(tc[k]), _bits(g1[k])), f"{k}: persistent kernel vs per-phase graph"
     assert (tc["codes"] == cc["codes"]).float().mean().item() > 0.5   # a near-tie flip changes the rest of its frame
 
 

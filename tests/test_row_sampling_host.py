@@ -78,4 +78,4 @@ def test_ctypes_layouts_match_the_header(tmp_path):
     want = [ctypes.sizeof(R), R.top_k.offset, R.min_p.offset, R.seed.offset, ctypes.sizeof(B), B.max_frames.offset, B.row_sampling.offset]
     assert [int(v) for v in sizes.split()] == want
     assert want[0] == 32
-    assert int(version) == _capi.SMOL_ABI_VERSION == 2
+    assert int(version) == _capi.SMOL_ABI_VERSION == 3

@@ -21,7 +21,7 @@ def main():
     ap.add_argument("--model", default="smoltts_byte_150m")
     ap.add_argument("--frames", type=int, default=16)
     ap.add_argument("--prompt-bytes", type=int, default=200)
-    ap.add_argument("--mode", type=int, default=2)
+    ap.add_argument("--mode", type=int, default=2, choices=(0, 2), help="2: data-flow kernel (default), 0: barrier kernel")
     ap.add_argument("--n-ctas", type=int, default=0)
     a = ap.parse_args()
     cfg = named_config(a.model)
