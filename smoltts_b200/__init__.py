@@ -24,6 +24,7 @@ from .model import (  # noqa: F401
 from .serving import ContinuousBatcher, PromptEncoder, byte_level_tokenizer  # noqa: F401,E402
 from .shard import ShardedGenerator, generate_sharded  # noqa: F401,E402
 from .mimi import MimiCache, MimiConfig, MimiModel, load_mimi  # noqa: F401,E402
+from .resample import Resampler, design_filter  # noqa: F401,E402
 from .tts import SmolTTS  # noqa: F401,E402
 
 __version__ = "0.1.0"

@@ -115,6 +115,15 @@ class SmolMimiEncoderWeights(C.Structure):
         ("conv_out", SmolMimiConv), ("rope", C.c_void_p)]
 
 
+# ---- include/smoltts_b200_resample.h ----
+SMOL_RESAMPLE_MAX_RATIO = 320
+SMOL_RESAMPLE_MAX_CALL = 256
+
+
+class SmolResampleConfig(C.Structure):
+    _fields_ = [(n, C.c_int32) for n in ("rate_in", "rate_out", "max_streams")]
+
+
 # name -> (restype, argtypes); every symbol the headers declare
 PROTOTYPES = {
     "smol_abi_version": (C.c_int, []),
@@ -165,6 +174,15 @@ PROTOTYPES = {
     "smol_mimi_encode": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(C.c_int64), C.c_int32, C.c_void_p, C.c_void_p]),
     "smol_mimi_encoder_debug_buffer": (C.c_void_p, [C.c_void_p, C.c_char_p]),
     "smol_mimi_encoder_launches": (C.c_int32, [C.c_void_p]),
+    # include/smoltts_b200_resample.h
+    "smol_resampler_create": (C.c_int, [C.POINTER(SmolResampleConfig), C.POINTER(C.c_void_p)]),
+    "smol_resampler_destroy": (None, [C.c_void_p]),
+    "smol_resampler_taps": (C.c_int32, [C.c_void_p]),
+    "smol_resampler_workspace_bytes": (C.c_size_t, [C.c_void_p]),
+    "smol_resampler_bind": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "smol_resampler_reset": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.c_int32, C.c_void_p]),
+    "smol_resample": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(C.c_int64), C.POINTER(C.c_int32), C.c_int32, C.c_int32, C.c_void_p,
+                                C.POINTER(C.c_int64), C.c_void_p]),
 }
 
 _lib = None

@@ -18,9 +18,9 @@ CSRC = os.path.join(PKG, "csrc")
 LIB_DIR = os.path.join(PKG, "_lib")
 LIB_PATH = os.path.join(LIB_DIR, "libsmoltts_b200.so")
 STAMP = os.path.join(LIB_DIR, "build.stamp")
-SOURCES = ["decode_kernel.cu", "ll2_kernel.cu", "capi.cu", "mimi_kernels.cu", "mimi_encoder.cu"]
+SOURCES = ["decode_kernel.cu", "ll2_kernel.cu", "capi.cu", "mimi_kernels.cu", "mimi_encoder.cu", "resample.cu"]
 HEADERS = ["common.cuh", "mimi_common.cuh", "dev_model.h", "sampler.cuh", "umma.cuh", "tc_phases.cuh", "tmap_host.h", os.path.join("..", "..", "include", "smoltts_b200.h"),
-           os.path.join("..", "..", "include", "smoltts_b200_mimi.h")]
+           os.path.join("..", "..", "include", "smoltts_b200_mimi.h"), os.path.join("..", "..", "include", "smoltts_b200_resample.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

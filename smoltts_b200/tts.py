@@ -9,11 +9,14 @@ through the codec as one batch of B streams per step.
 Parity note: the reference's ``__call__`` decodes the whole code sequence with ``codec.decode`` (the upsampler sees the
 sequence) while its ``stream`` upsamples every frame alone (codec/mimi.py:73-104): the two give different audio in the
 reference, and so do they here -- ``__call__`` uses a codec stream with the upsampler's carry, ``stream`` one without.
+
+Rates (new): the codec works at 24 kHz mono.  ``SmolTTS(..., output_rate=r)`` converts every entry point's PCM to ``r`` on the
+GPU (``resample.Resampler``), and ``create_speaker`` takes reference audio at any supported rate, mono or multi-channel.
 """
 from __future__ import annotations
 
 import dataclasses
-from typing import Iterator, List, Optional, Sequence
+from typing import Dict, Iterator, List, Optional, Sequence
 
 import numpy as np
 import torch
@@ -21,22 +24,37 @@ import torch
 from .generate import GenerationSettings, SingleBatchGenerator, generate_batch, generate_blocking
 from .mimi import MimiModel
 from .model import RQTransformer
+from .resample import Resampler
 from .serving import PromptEncoder
 
+CODEC_RATE = 24_000   # Mimi's sampling rate
 VOICES = ["heart", "bella", "nova", "sky", "sarah", "michael", "fenrir", "liam", "emma", "isabella", "fable"]   # :127-143
 
 
 class SmolTTS:
     def __init__(self, lm: RQTransformer, prompt_encoder: PromptEncoder, codec_stream: MimiModel, codec_full: Optional[MimiModel] = None,
-                 settings: Optional[GenerationSettings] = None):
+                 settings: Optional[GenerationSettings] = None, output_rate: Optional[int] = None):
         """codec_stream: a MimiModel with the reference's decode_step rule (upsample_carry=False); codec_full: one with
-        upsample_carry=True for ``__call__`` / ``synthesize_batch`` (defaults to codec_stream if it already carries)."""
+        upsample_carry=True for ``__call__`` / ``synthesize_batch`` (defaults to codec_stream if it already carries).
+
+        output_rate: the sampling rate of the PCM every entry point returns.  None or 24 000 is the codec's own rate: nothing
+        is resampled and no resampler is built.  Any other rate (``max(up, down) <= 320`` against 24 kHz: 8, 11.025, 16,
+        22.05, 32, 44.1, 48, 88.2, 96, 176.4, 192 kHz ...) converts on the GPU: whole utterances in one launch per codec call (per 256 streams),
+        streams a frame at a time; ``stream``'s first chunk is shorter by the filter's look-ahead, and its last chunk is the
+        filter's tail."""
         self.lm = lm
         self.prompt_encoder = prompt_encoder
         self.codec = codec_stream
         self.codec_full = codec_full if codec_full is not None else codec_stream
         self.settings = settings or GenerationSettings()
-        self.sampling_rate = 24_000
+        self.sampling_rate = CODEC_RATE
+        self.resampler: Optional[Resampler] = None
+        if output_rate is not None and int(output_rate) != CODEC_RATE:
+            # a resampler stream runs beside each codec stream; whole utterances take free slots for the length of one call
+            streams = self.codec.max_streams + (self.codec_full.max_streams if self.codec_full is not self.codec else 0)
+            self.resampler = Resampler(CODEC_RATE, int(output_rate), max_streams=streams, device=self.codec.device)
+            self.sampling_rate = int(output_rate)
+        self._input_resamplers: Dict[int, Resampler] = {}
 
     # ---- prompt assembly (:123-151) ----
     def _get_prompt(self, input: str, voice: str, sysprompt: Optional[torch.Tensor] = None) -> torch.Tensor:
@@ -46,7 +64,10 @@ class SmolTTS:
     def create_speaker(self, samples: Sequence[dict], system_prompt: Optional[str] = None) -> torch.Tensor:
         """Voice-clone prefix (__init__.py:97-118) from ``{"text", "audio"}`` samples -- 1-D float PCM at 24 kHz, mono -- or
         ``{"text", "codes"}`` samples with ready-made Mimi codes.  The audio of all samples is encoded in one
-        ``MimiModel.encode`` call (the codec must have been built with ``encode_max_samples > 0``)."""
+        ``MimiModel.encode`` call (the codec must have been built with ``encode_max_samples > 0``).
+
+        A sample with ``"sampling_rate"`` may carry audio at that rate, 1-D ``[L]`` or ``[C, L]``: the channels are averaged on
+        the device and the clips of each rate resampled to 24 kHz together (one launch per 256 clips) before the encode."""
         samples = list(samples)
         with_audio = [i for i, s in enumerate(samples) if "audio" in s and "codes" not in s]
         if with_audio:
@@ -54,7 +75,24 @@ class SmolTTS:
             if codec is None:
                 raise ValueError("create_speaker: samples carry 'audio' but the codec has no encoder "
                                  "(build the MimiModel with encode_max_samples > 0, or pass 'codes')")
-            clips = [torch.as_tensor(samples[i]["audio"], dtype=torch.float32).reshape(-1) for i in with_audio]
+            clips, by_rate = [], {}
+            for k, i in enumerate(with_audio):
+                s = samples[i]
+                if "sampling_rate" not in s:
+                    clips.append(torch.as_tensor(s["audio"], dtype=torch.float32).reshape(-1))
+                    continue
+                a = torch.as_tensor(s["audio"]).to(device=codec.device, dtype=torch.float32)
+                if a.dim() not in (1, 2) or (a.dim() == 2 and a.shape[0] > a.shape[1]):
+                    raise ValueError(f"create_speaker: audio of shape {tuple(a.shape)}; expected [L] or [channels, L] "
+                                     "(channels first: transpose [L, channels] audio)")
+                clips.append(a.mean(dim=0) if a.dim() == 2 else a)
+                if int(s["sampling_rate"]) != CODEC_RATE:
+                    by_rate.setdefault(int(s["sampling_rate"]), []).append(k)
+            for rate, ks in by_rate.items():
+                if rate not in self._input_resamplers:
+                    self._input_resamplers[rate] = Resampler(rate, CODEC_RATE, max_streams=codec.encode_max_clips, device=codec.device)
+                for k, y in zip(ks, self._input_resamplers[rate].resample([clips[k] for k in ks])):
+                    clips[k] = y
             codes = codec.encode(clips)
             samples = [dict(s) for s in samples]
             for i, c in zip(with_audio, codes):
@@ -68,8 +106,10 @@ class SmolTTS:
         codes = generate_blocking(self.lm, prompt, self.settings)          # [1, N, T]
         if codes.shape[-1] == 0:
             return np.zeros(0, dtype=np.float32)
-        pcm = self.codec_full.decode(codes.to(torch.int64))
-        return pcm.flatten().cpu().numpy()
+        pcm = self.codec_full.decode(codes.to(torch.int64)).flatten()
+        if self.resampler is not None:
+            pcm = self.resampler.resample([pcm])[0]
+        return pcm.cpu().numpy()
 
     # ---- streaming (:85-95) ----
     def stream(self, input: str, voice: Optional[str] = "heart", overlap: bool = True, lm_ctas: int = 96,
@@ -79,14 +119,24 @@ class SmolTTS:
         keeps both engines busy: the decode step of frame t + 1 is launched BEFORE the host looks at frame t, and frame t's ids,
         its codec step and its PCM go through a side stream -- the data-flow kernel is told to take ``lm_ctas`` of the GPU's SMs (a
         bs=1 frame takes the same 600-612 us on 96 .. 148 CTAs, DESIGN.md section 4), the codec's kernels run on the others.
-        Throughput is then bound by the slower engine instead of the sum plus the host's time per frame.  Same chunks, bit for bit."""
+        Throughput is then bound by the slower engine instead of the sum plus the host's time per frame.  Same chunks, bit for bit.
+
+        With an ``output_rate``, each frame's PCM goes through a resampler stream right after its codec step (on the side stream
+        in overlap mode) and the filter's tail follows the last frame as one more chunk."""
         prompt = self._get_prompt(input, voice if voice is not None else "0")
         codec = self.codec
         cache = codec.make_cache()
+        rs = self.resampler
+        rstate = None
+
+        def pcm_out(pcm: torch.Tensor) -> np.ndarray:
+            return (pcm if rstate is None else rs.step([pcm], [rstate])[0]).cpu().numpy()
         n_frames = n_audio = 0
         old_ctas = None
         batch = None
         try:
+            if rs is not None:
+                rstate = rs.make_state()
             if not overlap:
                 for frame in SingleBatchGenerator(self.lm, prompt, self.settings):
                     n_frames += 1
@@ -95,7 +145,9 @@ class SmolTTS:
                     if cache.frames >= codec.max_frames:
                         break
                     n_audio += 1
-                    yield codec.decode_step(frame.audio_codes, cache).flatten().cpu().numpy()
+                    yield pcm_out(codec.decode_step(frame.audio_codes, cache).flatten())
+                if rstate is not None and n_audio:
+                    yield rs.finish([rstate])[0].cpu().numpy()
                 return
             from .generate import _sampling
 
@@ -132,15 +184,21 @@ class SmolTTS:
                     out = None
                     if lo <= slow <= hi and cache.frames < codec.max_frames:
                         codes = col[1:] if cfg.duplicate_code_0 else torch.cat([col[0:1] - lo, col[1:]])
-                        out = codec.decode_step(codes.view(1, -1, 1), cache).flatten().cpu().numpy()
+                        out = pcm_out(codec.decode_step(codes.view(1, -1, 1), cache).flatten())
                         n_audio += 1
                 if out is not None:
                     yield out
                 if slow == tc.im_end_id or (lo <= slow <= hi and out is None):
                     break
+            if rstate is not None and n_audio:
+                with torch.cuda.stream(side):
+                    tail = rs.finish([rstate])[0].cpu().numpy()
+                yield tail
         finally:
             torch.cuda.synchronize(codec.device)
             codec.release_cache(cache)
+            if rstate is not None:
+                rs.release_state(rstate)
             if batch is not None:
                 batch.release()
             if old_ctas is not None:
@@ -197,12 +255,13 @@ class SmolTTS:
         """``serve`` with audio as it is generated: every utterance in a decode slot owns a codec stream, and after each chunk
         of ``chunk`` frames the new frames of all running utterances go through the codec together.  Yields ``(index, pcm of
         the chunk, done)``; the chunks of an utterance concatenate to what ``serve`` / ``synthesize_batch`` return for it."""
-        codec = self.codec_full
+        codec, rs = self.codec_full, self.resampler
         if slots > codec.max_streams:
             raise ValueError(f"serve_stream: {slots} slots, the codec was built for {codec.max_streams} streams")
         voices = list(voices) if voices is not None else ["heart"] * len(inputs)
         cb, per_input = self._batcher(len(inputs), settings, slots, chunk, max_prompt)
         caches: dict = {}
+        rstates: dict = {}   # with an output_rate: one resampler stream per live utterance, next to its codec stream
         try:
             uid_to_index = {cb.submit(self._get_prompt(t, v)[0], settings=per_input[i]): i
                             for i, (t, v) in enumerate(zip(inputs, voices))}
@@ -212,19 +271,41 @@ class SmolTTS:
                 for uid, _ in live:
                     if uid not in caches:
                         caches[uid] = codec.make_cache()
-                pcms = dict(zip((u for u, _ in live), self.decode_codes([c for _, c in live], [caches[u] for u, _ in live]))) if live else {}
+                        if rs is not None:
+                            rstates[uid] = rs.make_state()
+                uids = [u for u, _ in live]
+                pcms = dict(zip(uids, self._decode_pcm([c for _, c in live], [caches[u] for u in uids]))) if live else {}
+                if rs is not None:
+                    pcms = dict(zip(uids, rs.step([pcms[u] for u in uids], [rstates[u] for u in uids])))
+                    ended = [uid for uid, _, done in items if done and uid in rstates]
+                    for uid, tail in zip(ended, rs.finish([rstates[u] for u in ended])):
+                        pcms[uid] = torch.cat([pcms[uid], tail]) if uid in pcms else tail
                 for uid, codes, done in items:
                     if done and uid in caches:
                         codec.release_cache(caches.pop(uid))
-                    yield uid_to_index[uid], pcms.get(uid, np.zeros(0, dtype=np.float32)), done
+                        if rs is not None:
+                            rs.release_state(rstates.pop(uid))
+                    yield uid_to_index[uid], pcms[uid].cpu().numpy() if uid in pcms else np.zeros(0, dtype=np.float32), done
         finally:
             for c in caches.values():
                 codec.release_cache(c)
+            for st in rstates.values():
+                rs.release_state(st)
             cb.close()
 
     def decode_codes(self, codes: Sequence[torch.Tensor], caches: Optional[Sequence] = None) -> List[np.ndarray]:
         """Ragged code sequences [N, T_b] -> PCM, all streams stepping together while they last (fresh codec streams, or the
-        given ones continued)."""
+        given ones continued).  With an ``output_rate`` the utterances (fresh streams only) are resampled together, in one
+        launch."""
+        if self.resampler is not None and caches is not None:
+            raise ValueError("decode_codes: continued codec streams come out at 24 kHz; serve_stream resamples them as streams")
+        outs = self._decode_pcm(codes, caches)
+        if self.resampler is not None and outs:
+            outs = self.resampler.resample(outs)
+        return [o.cpu().numpy() for o in outs]
+
+    def _decode_pcm(self, codes: Sequence[torch.Tensor], caches: Optional[Sequence] = None) -> List[torch.Tensor]:
+        """``decode_codes`` at the codec's rate, as device tensors."""
         codec = self.codec_full
         B = len(codes)
         if B > codec.max_streams:
@@ -254,4 +335,4 @@ class SmolTTS:
         if own:
             for c in caches:
                 codec.release_cache(c)
-        return [o.cpu().numpy() for o in outs]
+        return outs
